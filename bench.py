@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- detector scenes/s @40k points on N B200s (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full detector forward (PointNet++ backbone SA1-4 + FP1-2, Hough voting, vote
@@ -222,6 +222,22 @@ def make_detector(device):
 
 RESULT_KEYS = ("objectness_scores", "center", "size_scores", "size_residuals", "sem_cls_scores",
                "bbox_corner", "aggregated_vote_inds")
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: what the timed path computed in its last step, one <out_dir>/<name>.npy per array, so that two
+    builds can be compared output for output (the inputs depend only on the arguments).  float64 stays float64,
+    integers (indices) become float64, which holds them exactly; everything else is stored as float32."""
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iub" else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of one step take %d bytes, more than --dump-outputs stores" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class L2Flusher:
@@ -502,6 +518,7 @@ def run_ours(args):
     eager_warm = args.warmup if args.mode == "eager" else min(args.warmup, 12)
     per_step, wall, clocks = timed_loop(step_resident, eager_steps, eager_warm, flush, barrier,
                                         ClockSampler(local) if args.mode == "eager" else None)
+    last_step = {k: out_holder["o"][k] for k in RESULT_KEYS}
     launches_per_step = meter.launches // (eager_steps + eager_warm)
     dev_s = sum(per_step) / 1e3
     regions = None
@@ -517,12 +534,13 @@ def run_ours(args):
                                         ("pm_tiles_per_cta", args.pm_tiles_per_cta)) if v is not None}
         runner = GraphedDetector(model, resident[0], n_streams=N_STREAMS, result_keys=RESULT_KEYS, **tune)
 
-        def timed_graph(submit, steps, warmup, repeats, sampler=None):
+        def timed_graph(submit, steps, warmup, repeats, sampler=None, after_regions=None):
             """`repeats` timed regions of exactly `steps` submits each, every region bracketed by a barrier +
             synchronize on both sides and timed with CUDA events (start event forked into every stream, end
             event after joining them).  nvidia-smi needs ~0.2 s for its first sample, so the sampler runs from
             the first warm-up step on and, if it still has fewer than 4 samples when the regions are done, the
-            SAME workload keeps running untimed until it has (reported as extra untimed steps)."""
+            SAME workload keeps running untimed until it has (reported as extra untimed steps).
+            `after_regions` is called once the last region has finished, before any untimed step."""
             if sampler:
                 sampler.start()
             for i in range(warmup):
@@ -546,6 +564,8 @@ def run_ours(args):
                 barrier()
                 out.append(e0.elapsed_time(e1))
             wall_ = time.perf_counter() - t0
+            if after_regions:
+                after_regions()
             clk = None
             if sampler:
                 extra, t_end = 0, time.perf_counter() + 3.0
@@ -559,8 +579,13 @@ def run_ours(args):
                                  % (repeats, extra))
             return out, wall_, clk
 
+        def keep_last_step():
+            """Results of the last timed step, from its slot (the steps that follow reuse the slots)."""
+            out = runner.outputs[(runner._next - 1) % runner.n]
+            last_step.update({k: out[k].clone() for k in RESULT_KEYS})
+
         regions, wall, clocks = timed_graph(lambda i: runner.submit(resident[i % n_sets]),
-                                            args.steps, args.warmup, REPEATS, ClockSampler(local))
+                                            args.steps, args.warmup, REPEATS, ClockSampler(local), keep_last_step)
 
         def submit_e2e(i):
             slot = runner._next
@@ -746,6 +771,8 @@ def run_ours(args):
             "wall_s_timed_region": round(wall, 4),
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -817,6 +844,8 @@ def run_train(args, rank, world, local, device, dist, barrier):
 
     per_step, wall, clocks = timed_loop(lambda i: step(resident[i % n_sets], True), args.steps, args.warmup, flush,
                                         barrier, ClockSampler(local))
+    last_step = {"loss": static_loss.clone(),
+                 "gradients": torch.cat([p.grad.reshape(-1) for p in model.parameters() if p.grad is not None])}
     loss_holder = {}
 
     def step_e2e(i):
@@ -868,6 +897,8 @@ def run_train(args, rank, world, local, device, dist, barrier):
                 "gpu_launches": int(launches_per_step * args.steps), "gpu_launches_per_step": int(launches_per_step),
                 "roofline": None, "cpu_baseline": None, "clocks": clocks, "wall_s_timed_region": round(wall, 4)}
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -1021,8 +1052,10 @@ def run_reference(args):
         resident = [h.to(device) for h in host]
         flush = L2Flusher(device)
 
+        out_holder = {}
+
         def step(i):
-            forward_resident(model, resident[i % n_sets])
+            out_holder["o"] = forward_resident(model, resident[i % n_sets])
         per_step, wall, clocks = timed_loop(step, args.steps, args.warmup, flush, barrier, ClockSampler(local))
         t = torch.tensor([sum(per_step)], device=device, dtype=torch.float64)
         if dist is not None:
@@ -1046,6 +1079,8 @@ def run_reference(args):
                             "d2h_bytes_per_step": 0},
                     "clocks": clocks}
             print(json.dumps(line))
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {k: out_holder["o"][k] for k in RESULT_KEYS})
         if dist is not None:
             dist.destroy_process_group()
         return
@@ -1063,7 +1098,7 @@ def run_reference(args):
             model({"point_clouds": scene})
         t0 = time.perf_counter()
         for _ in range(steps):
-            model({"point_clouds": scene})
+            out = model({"point_clouds": scene})
         el = time.perf_counter() - t0
     val = steps / el
     line = {"impl": "reference", "metric": "detector scenes/s @40k pts", "value": round(val, 4),
@@ -1076,13 +1111,20 @@ def run_reference(args):
             "e2e": {"value": round(val, 4), "unit": "scenes/s", "h2d_bytes_per_step": 0,
                     "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: out[k] for k in RESULT_KEYS})
 
 
 def main():
     global N_STREAMS, CFG, N_POINTS
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="K, timed steps per measured region.  Graph mode (headline): %d regions of exactly K steps "
+                         "each, on device-resident and on host inputs; its secondary passes time min(K, 60) eager "
+                         "steps, min(K, 5) eager host-to-host steps and min(K, 5) steps of per-kernel events.  "
+                         "Eager mode and config 5: exactly K steps.  --impl reference: K steps on the reference's "
+                         "CUDA stack, min(K, 5) forwards on the CPU port" % REPEATS)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json workload")
@@ -1094,7 +1136,12 @@ def main():
     ap.add_argument("--pm-tiles-per-cta", type=int, default=None, help="tuning: pm_linear row tiles per CTA in the graphs")
     ap.add_argument("--mode", default="graph", choices=["graph", "eager"],
                     help="graph: CUDA-graph replay on %d streams (headline); eager: plain launches" % N_STREAMS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path computed in its last step (rank 0) as "
+                         "DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     N_STREAMS = max(1, args.streams)
     CFG = dict(CONFIGS[args.config], id=args.config)

@@ -21,6 +21,13 @@ import cases  # noqa: E402
 from oracle.build_ref import load_ref  # noqa: E402
 
 
+def compact(out):
+    """Outputs the tests compare bit for bit are stored as their `cases.sha` digest (dtype, shape and bytes); the
+    gradients, compared within a tolerance, are stored in full.  This keeps the file small."""
+    return {k: v if k.endswith(("/grad", "/sha")) or k.startswith("meta/") else np.array(cases.sha(v))
+            for k, v in out.items()}
+
+
 def main():
     ref = load_ref()
     dev = torch.device("cuda:0")
@@ -69,7 +76,7 @@ def main():
     dst = os.path.join(ROOT, "gpurun_out", "golden")
     os.makedirs(dst, exist_ok=True)
     path = os.path.join(dst, "ref_ops.npz")
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **compact(out))
     print("wrote", path, os.path.getsize(path), "bytes,", len(out), "arrays")
 
 

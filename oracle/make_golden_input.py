@@ -16,6 +16,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+import cases  # noqa: E402
 import cases_input  # noqa: E402
 
 REF = "/root/reference"
@@ -112,7 +113,8 @@ def main():
     out = {}
     for name in cases_input.CASES:
         for k, v in getitem(cases_input.case(name)).items():
-            out["%s/%s" % (name, k)] = v
+            # the point clouds (most of the file) are compared bit for bit: their digest is enough
+            out["%s/%s" % (name, k)] = np.array(cases.sha(v)) if k == "point_clouds" else v
     # np.percentile on its own: many sizes / duplicate patterns
     for i, z in enumerate(cases_input.percentile_inputs()):
         out["percentile/%d" % i] = np.float32(np.percentile(z, 0.99))

@@ -187,13 +187,15 @@ def test_bench_byte_and_flop_models_match_the_abi():
     assert bench.ALGO_FLOPS["spc_sa_fused_forward"](a) == bench.ALGO_FLOPS["spc_sa_fused_forward_ex"](a_ex)
 
 
-def test_bench_reference_arm_runs_without_a_gpu():
+def test_bench_reference_arm_runs_without_a_gpu(tmp_path):
     """`bench.py --impl reference` must always print one JSON line: here (no GPU, hence no reference CUDA extension)
-    it times the CPU oracle port on a bounded sample; the keys the driver reads are all present."""
+    it times the CPU oracle port on a bounded sample; the keys a reader of the line needs are all present, and
+    --dump-outputs writes the detections of the last timed step."""
     import json
+    import bench
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "1"], capture_output=True, text=True, timeout=300,
-                         env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+                          "--warmup", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True,
+                         timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["metric"] == "detector scenes/s @40k pts" and line["value"] > 0
@@ -201,6 +203,10 @@ def test_bench_reference_arm_runs_without_a_gpu():
     assert line["cpu_baseline"]["kind"] in ("port", "reference") and line["cpu_baseline"]["cores"] >= 0
     assert set(line["e2e"]) >= {"value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step"}
     assert "workload" in line["config"] and "model" not in line["config"]
+    dumped = {p.name: np.load(p) for p in tmp_path.iterdir()}
+    assert set(dumped) == {k + ".npy" for k in bench.RESULT_KEYS}
+    assert dumped["bbox_corner.npy"].shape == (1, 256, 8, 3)
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in dumped.values())
 
 
 def test_launch_options_are_thread_local_and_restored():

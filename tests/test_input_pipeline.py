@@ -8,6 +8,7 @@ import pytest
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import cases  # noqa: E402
 import cases_input  # noqa: E402
 from oracle import input_pipeline as oi  # noqa: E402
 from spacap3d_b200 import input_pipeline as ip  # noqa: E402
@@ -42,7 +43,7 @@ def test_oracle_equals_reference(name):
         assert fh == GOLD[name + "/floor_height"]
     pc = oi.prepare_point_cloud(c["verts"], choices, c["multiview"] if c["use_multiview"] else None, fh, aug,
                                 c["use_color"], c["use_normal"])
-    np.testing.assert_array_equal(pc, GOLD[name + "/point_clouds"])
+    assert cases.sha(pc) == str(GOLD[name + "/point_clouds"])
     votes, mask = oi.vote_labels(pc, c["inst"][choices], c["sem"][choices])
     np.testing.assert_array_equal(votes, GOLD[name + "/vote_label"])
     np.testing.assert_array_equal(mask, GOLD[name + "/vote_label_mask"])
@@ -97,7 +98,7 @@ def test_device_batch_equals_reference(name):
     pc = out["point_clouds"].cpu().numpy()
     # fp64 rotation products rounded to fp32: identical unless BLAS' dgemm and the kernel's fma chain round an fp64
     # intermediate differently AND that flips the fp32 rounding; never observed -> exact comparison
-    np.testing.assert_array_equal(pc[0], GOLD[name + "/point_clouds"])
+    assert cases.sha(pc[0]) == str(GOLD[name + "/point_clouds"])             # stored as a digest of the exact bytes
     np.testing.assert_array_equal(out["vote_label"][0].cpu().numpy(), GOLD[name + "/vote_label"])
     np.testing.assert_array_equal(out["vote_label_mask"][0].cpu().numpy(), GOLD[name + "/vote_label_mask"])
     np.testing.assert_allclose(out["target_bboxes"][0].cpu().numpy(), GOLD[name + "/target_bboxes"], rtol=1e-13,

@@ -21,7 +21,17 @@ Bars:
   * the vote FPS depends on feature values (vote_xyz = seed_xyz + predicted offset), so once
     vote_xyz differs in the last bits its picks may differ: end to end only the fraction of equal
     picks is reported; on the reference's votes the picks are bit-equal.
+
+Without the staged reference stack (its Python sources and checkpoints are not part of this repository), A is
+replaced by tests/golden/detector_ref.npz: digests of every output of C with seeded weights run on the REFERENCE's
+nine point ops (its CUDA extension, or the C oracle pinned to it) and a restatement of its host decode, computed
+without any kernel of this package (oracle/make_golden_detector.py).  The exact mode of C must match them bit for
+bit ("C_exact_vs_pinned"); the fast mode is then held to the bars above against those exact outputs
+("C_fast_vs_C_exact", run for the C_fast_vs_A cases), with the box decode compared with bench.reference_host_decode,
+this project's restatement of the reference's decode.  B, which needs the reference's models/*.py, skips.
 """
+import os
+
 import pytest
 import torch
 
@@ -35,26 +45,37 @@ TOL = 1e-2
 TOL_E2E_VOTES = 2e-2
 
 
-def _stack_or_skip():
+def _stack_available():
+    """True when the reference stack is staged; a staged stack whose extension does not load is an error, not a
+    reason to fall back to the pinned outputs."""
     from oracle import refstack
     if not refstack.available():
-        pytest.skip("baseline/_ref not staged (python oracle/stage_reference.py in the build container)")
-    try:
-        from oracle.build_ref import load_ref
-        load_ref()
-    except Exception as e:  # noqa: BLE001
-        pytest.skip("oracle/_ref not loadable: %r" % (e,))
+        return False
+    from oracle.build_ref import load_ref
+    load_ref()
+    return True
 
 
 @pytest.fixture(scope="module", params=[1, 7, 132], ids=["xyz_C1", "rgb_normal_C7", "multiview_C132"])
 def report(request):
-    _stack_or_skip()
+    import numpy as np
     import refparity
-    return refparity.collect(request.param, batch=8, n_points=40000)
+    if _stack_available():
+        return refparity.collect(request.param, batch=8, n_points=40000)
+    golden = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "detector_ref.npz"))
+    return refparity.collect_pinned(request.param, golden, batch=8, n_points=40000)
+
+
+def _tag(report, tag):
+    if tag in report:
+        return report[tag]
+    if tag == "C_fast_vs_A" and "C_fast_vs_C_exact" in report:       # no reference stack: see the module docstring
+        return report["C_fast_vs_C_exact"]
+    pytest.skip("%s needs the reference's models/*.py (baseline/_ref, not part of this repository)" % tag)
 
 
 def test_exact_mode_equals_reference_bit_for_bit(report):
-    r = report["B_exact_vs_A"]
+    r = report["B_exact_vs_A"] if "B_exact_vs_A" in report else report["C_exact_vs_pinned"]
     assert r["ball_query_tables_compared"] == 5
     bad = [k for k, v in r.items() if k.endswith("equal") and v is not True]
     assert not bad, bad
@@ -63,7 +84,7 @@ def test_exact_mode_equals_reference_bit_for_bit(report):
 @pytest.mark.parametrize("tag", ["B_fast_vs_A", "C_fast_vs_A"])
 def test_fast_mode_indices_bit_exact(report, tag):
     import refparity
-    r = report[tag]
+    r = _tag(report, tag)
     for k in refparity.INDEX_KEYS + refparity.XYZ_KEYS:
         assert r[k + ":equal"] is True, k
     for i in range(4):
@@ -74,7 +95,7 @@ def test_fast_mode_indices_bit_exact(report, tag):
 
 @pytest.mark.parametrize("tag", ["B_fast_vs_A", "C_fast_vs_A"])
 def test_fast_mode_features_elementwise(report, tag):
-    r = report[tag]
+    r = _tag(report, tag)
     for i in (1, 2, 3, 4):
         assert r["sa%d_features:nerr" % i] <= TOL, (i, r["sa%d_features:nerr" % i])
         assert r["stage|sa%d_features:nerr" % i] <= TOL, (i, r["stage|sa%d_features:nerr" % i])
@@ -92,7 +113,7 @@ def test_fast_mode_features_elementwise(report, tag):
 @pytest.mark.parametrize("tag", ["B_fast_vs_A", "C_fast_vs_A"])
 def test_box_decode_equals_get_3d_box_batch(report, tag):
     """SURVEY row N1: the on-device decode against the reference's host decode (proposal_module.py:81-104)."""
-    r = report[tag]
+    r = _tag(report, tag)
     assert r["proposal|bbox_corner_vs_get_3d_box_batch:equal"] is True, r["proposal|bbox_corner_vs_get_3d_box_batch:maxabs"]
     assert r["bbox_corner_vs_get_3d_box_batch:equal"] is True
 

@@ -1,5 +1,7 @@
 """Training mode (autograd through the unfused sm_100a kernels) against the reference's own CUDA
 extension driving the same modules: forward values, input gradients and every parameter gradient.
+Where that extension is not built (oracle/_ref), its nine entry points are served by the C oracle,
+which tests/test_oracle_golden.py pins to the extension's stored outputs.
 The reference's atomics make its gradients order-nondeterministic, hence rtol 1e-4 rather than
 bitwise; both sides run cuDNN with TF32 disabled (SURVEY F8)."""
 import numpy as np
@@ -29,9 +31,9 @@ def _run(model, xyz, feats):
 
 
 def test_train_step_matches_reference_extension(ref_ext):
-    if ref_ext is None:
-        pytest.skip("oracle/_ref/pointnet2_ref_ext.so not on this box")
     import bench
+    import refparity
+    provider = ref_ext if ref_ext is not None else refparity.OracleOnDevice(DEV)
     from spacap3d_b200.scenes import make_scene_xyz
     old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
     torch.backends.cudnn.allow_tf32 = False
@@ -46,7 +48,7 @@ def test_train_step_matches_reference_extension(ref_ext):
             xyz = torch.from_numpy(xyz_np).to(DEV).requires_grad_(True)
             feats = feats_np.to(DEV).requires_grad_(True)
             if use_ref:
-                with bench.swapped_ops(ref_ext, host_decode=False):
+                with bench.swapped_ops(provider, host_decode=False):
                     loss, up, inds = _run(model, xyz, feats)
                     loss.backward()
             else:
