@@ -307,15 +307,15 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
           hw[i] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
           lw[i] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
         }
-        if (c0 + 32 <= Nt) {
-          uint4 *yh = reinterpret_cast<uint4 *>(p.Y_hi + row * p.N + ch0);
+        // per 8-channel chunk: a slice of n_tile channels (a multiple of 16, so Nt is one too) can end halfway
+        // through a block of 32
+        uint4 *yh = reinterpret_cast<uint4 *>(p.Y_hi + row * p.N + ch0);
+        uint4 *yl = p.Y_lo ? reinterpret_cast<uint4 *>(p.Y_lo + row * p.N + ch0) : nullptr;
 #pragma unroll
-          for (int i = 0; i < 4; ++i) yh[i] = make_uint4(hw[4 * i], hw[4 * i + 1], hw[4 * i + 2], hw[4 * i + 3]);
-          if (p.Y_lo) {
-            uint4 *yl = reinterpret_cast<uint4 *>(p.Y_lo + row * p.N + ch0);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) yl[i] = make_uint4(lw[4 * i], lw[4 * i + 1], lw[4 * i + 2], lw[4 * i + 3]);
-          }
+        for (int i = 0; i < 4; ++i) {
+          if (c0 + 8 * i + 8 > Nt) continue;
+          yh[i] = make_uint4(hw[4 * i], hw[4 * i + 1], hw[4 * i + 2], hw[4 * i + 3]);
+          if (yl) yl[i] = make_uint4(lw[4 * i], lw[4 * i + 1], lw[4 * i + 2], lw[4 * i + 3]);
         }
       }
     } else {

@@ -27,6 +27,16 @@ LAYERS = {
     "sa3": (1024, 256, 512, 0.8, 16, [256, 128, 128, 256]),
     "sa4": (512, 256, 256, 1.2, 16, [256, 128, 128, 256]),
     "vote_agg": (1024, 256, 256, 0.3, 16, [256, 128, 128, 128]),
+    # the remaining compiled (C1, C2, C3, nsample) kernels of each form, so that every one runs against the fp32 sequence
+    "inline_wide_ns64": (4096, 4, 128, 0.3, 64, [4, 128, 128, 256]),
+    "inline_wide_c256_ns16": (2048, 2, 256, 0.4, 16, [2, 128, 128, 256]),
+    "inline_c128_ns64": (4096, 3, 128, 0.3, 64, [3, 128, 128, 128]),
+    "inline_c128_ns32": (4096, 1, 256, 0.3, 32, [1, 128, 128, 128]),
+    "projected_narrow_ns32": (4096, 16, 256, 0.3, 32, [16, 64, 64, 128]),
+    "projected_narrow_ns16": (4096, 24, 256, 0.3, 16, [24, 64, 64, 128]),
+    "projected_wide_ns64": (2048, 64, 256, 0.4, 64, [64, 128, 128, 256]),
+    "projected_c128_ns64": (2048, 32, 256, 0.4, 64, [32, 128, 128, 128]),
+    "projected_c128_ns32": (2048, 128, 512, 0.4, 32, [128, 128, 128, 128]),
 }
 
 
