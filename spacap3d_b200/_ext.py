@@ -281,7 +281,7 @@ def three_interpolate_grad(grad_out, idx, weight, m):
 
 
 def sa_fused_forward(xyz, new_xyz, idx, W0, b0, W1, b1, W2, b2, *, G=None, feat=None, radius=1.0,
-                     want_point_major=False, W0_host=None, b0_host=None):
+                     want_point_major=False):
     """Fused set-abstraction forward (eval): gather + layer 0 + two tcgen05 1x1 convs + max-pool.
     See spc_sa_fused_forward in include/spacap3d_ops.h.
       in-line form   : G is None, feat (B,Cf,n) or None, W0 (C1,3+Cf)
@@ -317,18 +317,12 @@ def sa_fused_forward(xyz, new_xyz, idx, W0, b0, W1, b1, W2, b2, *, G=None, feat=
             Cf = feat.shape[1]
             pfeat = feat.data_ptr()
         assert W0.shape == (C1, 3 + Cf)
-    pW0h = pb0h = None
-    if W0_host is not None and b0_host is not None:     # host copies of the folded layer-0 weights (constant-bank path)
-        for t, nm in ((W0_host, "W0_host"), (b0_host, "b0_host")):
-            if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
-                raise RuntimeError("%s must be a contiguous float CPU tensor" % nm)
-        assert W0_host.shape == W0.shape and b0_host.numel() == C1
-        pW0h, pb0h = W0_host.data_ptr(), b0_host.data_ptr()
     out = torch.empty((B, C3, npoint), dtype=torch.float32, device=xyz.device)
     out_pm = torch.empty((B, npoint, C3), dtype=HALF, device=xyz.device) if want_point_major else None
     with torch.cuda.device(xyz.device):
+        # the two None after b0 fill the W0_host / b0_host slots, which the library ignores
         _lib.call("spc_sa_fused_forward_ex", xyz.data_ptr(), new_xyz.data_ptr(), idx.data_ptr(),
-                  pG, pfeat, W0.data_ptr(), b0.data_ptr(), pW0h, pb0h, int(Cf), float(radius), W1.data_ptr(),
+                  pG, pfeat, W0.data_ptr(), b0.data_ptr(), None, None, int(Cf), float(radius), W1.data_ptr(),
                   b1.data_ptr(), W2.data_ptr(), b2.data_ptr(), B, n, npoint, nsample, C1, C2, C3,
                   out.data_ptr(), out_pm.data_ptr() if out_pm is not None else None, int(_options.sa_min_tiles),
                   _stream())

@@ -27,6 +27,7 @@
 #include <mutex>
 
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -51,35 +52,11 @@ __device__ __forceinline__ int fps_v_to_k(unsigned v, int Q, int T, int log2T) {
   return (int)(q * (unsigned)T + res);
 }
 
-// ---- PTX helpers: cluster address mapping, mbarrier, async DSMEM store --------------------------
-__device__ __forceinline__ uint32_t fps_s2u(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+// ---- PTX helpers: cluster address mapping, async DSMEM store -----------------------------------
 __device__ __forceinline__ uint32_t mapa_cluster(uint32_t local_addr, uint32_t cta_rank) {
   uint32_t r;
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(cta_rank));
   return r;
-}
-__device__ __forceinline__ void fps_mbar_init(uint64_t *bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(fps_s2u(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void fps_mbar_arm(uint64_t *bar, unsigned tx_bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(fps_s2u(bar)), "r"(tx_bytes)
-               : "memory");
-}
-// NB: plain (cta-scope) try_wait.  A cluster-scope acquire here compiles to an L1 invalidate
-// (CCTL.IVALL) on every poll; completion of a transaction barrier already makes the st.async
-// payload visible (same contract as a TMA load).
-__device__ __forceinline__ void fps_mbar_wait(uint64_t *bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "FPS_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra FPS_DONE;\n"
-      "bra FPS_WAIT;\n"
-      "FPS_DONE:\n"
-      "}\n" ::"r"(fps_s2u(bar)),
-      "r"(parity)
-      : "memory");
 }
 // 16-byte + 4-byte remote stores into a peer CTA's shared memory; each store signals its bytes
 // on the peer's mbarrier (complete_tx), so the receiver needs no fence and no cluster barrier
@@ -190,18 +167,18 @@ __global__ void __launch_bounds__(THREADS, (THREADS <= 256 ? 2 : 1)) fps_cluster
   uint32_t r_slot0 = 0, r_slot1 = 0, r_bar0 = 0, r_bar1 = 0;   // my slot / barrier in peer `lane`
   if (C > 1) {
     if (tid == 0) {
-      fps_mbar_init(&c_bar[0], 1);
-      fps_mbar_init(&c_bar[1], 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      fps_mbar_arm(&c_bar[0], tx_bytes);
-      fps_mbar_arm(&c_bar[1], tx_bytes);
+      mbarrier_init(&c_bar[0], 1);
+      mbarrier_init(&c_bar[1], 1);
+      fence_mbarrier_init();
+      mbarrier_arrive_expect_tx(&c_bar[0], tx_bytes);
+      mbarrier_arrive_expect_tx(&c_bar[1], tx_bytes);
     }
     cluster.sync();   // peers' barriers are initialised before anyone stores into them
     if (warp == 0 && lane < C) {
-      r_slot0 = mapa_cluster(fps_s2u(&c_cand[0][rank]), lane);
-      r_slot1 = mapa_cluster(fps_s2u(&c_cand[1][rank]), lane);
-      r_bar0 = mapa_cluster(fps_s2u(&c_bar[0]), lane);
-      r_bar1 = mapa_cluster(fps_s2u(&c_bar[1]), lane);
+      r_slot0 = mapa_cluster(s2u(&c_cand[0][rank]), lane);
+      r_slot1 = mapa_cluster(s2u(&c_cand[1][rank]), lane);
+      r_bar0 = mapa_cluster(s2u(&c_bar[0]), lane);
+      r_bar1 = mapa_cluster(s2u(&c_bar[1]), lane);
     }
   } else {
     __syncthreads();
@@ -253,8 +230,8 @@ __global__ void __launch_bounds__(THREADS, (THREADS <= 256 ? 2 : 1)) fps_cluster
         st_async_v4(rs, bmax, wk, wxb, wyb, rb);
         st_async_b32(rs + 16, __float_as_uint(wz), rb);
       }
-      fps_mbar_wait(&c_bar[buf], (unsigned)((j - 1) >> 1) & 1u);   // u-th use of this buffer
-      if (tid == 0) fps_mbar_arm(&c_bar[buf], tx_bytes);           // re-arm for round j+2
+      mbarrier_wait(&c_bar[buf], (unsigned)((j - 1) >> 1) & 1u);           // u-th use of this buffer
+      if (tid == 0) mbarrier_arrive_expect_tx(&c_bar[buf], tx_bytes);   // re-arm for round j+2
       e4 = make_uint4(0u, 0u, 0u, 0u);
       ez = 0.f;
       if (lane < C) {

@@ -18,48 +18,9 @@
 // atomic, and rows are flushed with plain coalesced stores (or global atomics when the
 // position range had to be split across CTAs to fill the machine).
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace spc {
-
-// ----------------------------------------------------------------------------------------------
-// mbarrier / bulk-copy helpers (PTX)
-// ----------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void fence_mbar_init() {
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_LOOP:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra WAIT_DONE;\n"
-      "bra WAIT_LOOP;\n"
-      "WAIT_DONE:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-// global -> shared bulk copy (TMA engine, 1-D): bytes % 16 == 0, both addresses 16-B aligned
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, unsigned bytes,
-                                         uint64_t *bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-          "r"(smem_u32(dst_smem)),
-      "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
 
 __device__ __forceinline__ void st_cs_v4(float *p, float a, float b, float c, float d) {
   asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d)
@@ -117,14 +78,14 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_kernel(
     const size_t bytes = (size_t)ct * N * sizeof(float);
     const bool bulk_ok = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) && (bytes % 16 == 0);
     if (bulk_ok) {
-      if (tid == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
+      if (tid == 0) { mbarrier_init(&bar, 1); fence_mbarrier_init(); }
       __syncthreads();
       if (tid == 0) {
         // expect_tx is limited to 2^20-1 bytes per call; our rows are <= 227 KB
-        mbar_expect_tx(&bar, (unsigned)bytes);
+        mbarrier_arrive_expect_tx(&bar, (unsigned)bytes);
         bulk_g2s(s_rows, src, (unsigned)bytes, &bar);
       }
-      mbar_wait(&bar, 0);
+      mbarrier_wait(&bar, 0);
     } else {
       for (size_t e = tid; e < (size_t)ct * N; e += GP_THREADS) s_rows[e] = __ldg(src + e);
       __syncthreads();
@@ -321,17 +282,7 @@ static GradPlan plan_group_grad(int C, int N, int S) {
   return g;
 }
 
-// counts[b][h][1 + idx[b,t]] += 1   (offsets row = Np ints per (b,h), slot 0 stays 0)
-__global__ void gg_hist_kernel(const int32_t *__restrict__ idx, int N, int S, int Sp, int H, int Np,
-                               int *__restrict__ offsets) {
-  const int b = blockIdx.y;
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= S) return;
-  const int i = __ldg(idx + (size_t)b * S + t);
-  if ((unsigned)i < (unsigned)N) atomicAdd(offsets + ((size_t)b * H + t / Sp) * Np + 1 + i, 1);
-}
-
-// in-place inclusive scan of offsets[b][h][1..N]  (one CTA per (b,h))
+// in-place inclusive scan of offsets[r][1..N]  (one CTA per offsets row r)
 __global__ void __launch_bounds__(1024) gg_scan_kernel(int N, int Np, int *__restrict__ offsets) {
   __shared__ int s_part[32];
   int *row = offsets + (size_t)blockIdx.x * Np + 1;
@@ -357,79 +308,28 @@ __global__ void __launch_bounds__(1024) gg_scan_kernel(int N, int Np, int *__res
   for (int e = e0; e < e1; ++e) { run += row[e]; row[e] = run; }
 }
 
-// Deterministic fill: a warp owns 32 consecutive points and scans every position of its partition in
-// ascending order, so each list comes out sorted by position without any atomics on the cursors.
-// The partition's indices are staged in shared memory once per CTA (8 warps = 256 points).
-constexpr int GG_FILL_WARPS = 8;
-__global__ void __launch_bounds__(GG_FILL_WARPS * 32) gg_fill_kernel(const int32_t *__restrict__ idx, int N, int S,
-                                                                      int Sp, int H, int Np,
-                                                                      const int *__restrict__ offsets,
-                                                                      uint16_t *__restrict__ order) {
-  extern __shared__ __align__(128) int s_idx[];     // [Sp]
-  __shared__ int s_cur[GG_FILL_WARPS][32];
-  __shared__ __align__(8) uint64_t bar;
-  const int b = blockIdx.z, h = blockIdx.y;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int p0 = h * Sp, len = min(S, p0 + Sp) - p0;
-  const int32_t *ix = idx + (size_t)b * S + p0;
-  const bool bulk_ok = ((reinterpret_cast<uintptr_t>(ix) & 15) == 0) && (len % 4 == 0);
-  if (bulk_ok) {
-    if (tid == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
-    __syncthreads();
-    if (tid == 0) {
-      mbar_expect_tx(&bar, (unsigned)(len * sizeof(int)));
-      bulk_g2s(s_idx, ix, (unsigned)(len * sizeof(int)), &bar);
-    }
-    mbar_wait(&bar, 0);
-  } else {
-    for (int e = tid; e < len; e += GG_FILL_WARPS * 32) s_idx[e] = __ldg(ix + e);
-    __syncthreads();
-  }
-  const int i0 = (blockIdx.x * GG_FILL_WARPS + warp) * 32;
-  if (i0 >= N) return;
-  const int *off = offsets + ((size_t)b * H + h) * Np;
-  s_cur[warp][lane] = (i0 + lane < N) ? off[i0 + lane] : 0;
-  __syncwarp();
-  uint16_t *ord = order + (size_t)b * S + p0;
-  for (int t0 = 0; t0 < len; t0 += 32) {
-    const int t = t0 + lane;
-    const int v = t < len ? s_idx[t] : -1;
-    const unsigned rel = (unsigned)(v - i0);
-    const bool hit = v >= 0 && rel < 32u && v < N;
-    if (!__any_sync(0xffffffffu, hit)) continue;
-    const unsigned peers = __match_any_sync(0xffffffffu, hit ? rel : 32u + (unsigned)lane);
-    int base = 0;
-    if (hit) base = s_cur[warp][rel];
-    __syncwarp();
-    if (hit) {
-      const unsigned before = peers & ((1u << lane) - 1u);
-      ord[base + __popc(before)] = (uint16_t)t;
-      if (before == 0u) s_cur[warp][rel] = base + __popc(peers);
-    }
-    __syncwarp();
-  }
-}
-
 // ----------------------------------------------------------------------------------------------
-// One-kernel list build (N <= 8192): histogram + scan + a TWO-LEVEL stable counting sort, one CTA per
-// (scene, partition).  The fill above lets every warp (32 points) scan all Sp positions -- N/32 x Sp/32
-// warp iterations, 43 us at the SA2 shape and a third of the whole backward.  Here
+// List build (N <= 8192): histogram + scan + a TWO-LEVEL stable counting sort in ONE kernel per (scene, partition).
 //   A. the positions are first bucketed by key >> 5 (<= 256 buckets): warp w walks its contiguous chunk of
 //      positions, counts per bucket (match.any, no atomics: a row of counters per warp), the counters are
 //      turned into start offsets (bucket b starts where the list of key 32b starts, then warp by warp), and
 //      a second walk in the same order scatters the positions => stable;
 //   B. one warp per bucket orders its (short) region by the low 5 key bits with per-key cursors, again in
-//      position order => every list ascending, exactly what gg_fill_kernel produces (tested bit for bit).
-// Work: 2 x Sp/32 + Sp/32 + N/32 warp iterations per partition instead of N/32 x Sp/32.
+//      position order => every list ascending, so group_points_grad_csr_kernel sums each list in a fixed order.
+// Work: 2 x Sp/32 + Sp/32 + N/32 warp iterations per partition.  A warp per 32 points scanning all Sp positions
+// (N/32 x Sp/32 warp iterations) took 43 us at the SA2 shape, a third of the whole backward.
 // ----------------------------------------------------------------------------------------------
 constexpr int GB_THREADS = 1024;
 constexpr int GB_MAX_N = 8192;
 
-static size_t gg_build_smem(int N, int Sp, int Np) {
+static constexpr size_t gg_build_smem(int N, int Sp, int Np) {
   const int nbk = (N + 31) >> 5;
   return (size_t)Sp * sizeof(int) + (size_t)Np * sizeof(int) + (size_t)32 * nbk * sizeof(int) +
          (size_t)Sp * sizeof(uint16_t) + 16;
 }
+// plan_group_grad keeps Sp <= GG_PART_MAX, so every N <= GB_MAX_N fits one CTA
+static_assert(gg_build_smem(GB_MAX_N, GG_PART_MAX, (GB_MAX_N + 1 + 3) / 4 * 4) <= 220 * 1024,
+              "gg_build_kernel's shared memory must fit at every N <= GB_MAX_N");
 
 __global__ void __launch_bounds__(GB_THREADS) gg_build_kernel(const int32_t *__restrict__ idx, int N, int S, int Sp,
                                                               int H, int Np, int *__restrict__ offsets,
@@ -449,10 +349,10 @@ __global__ void __launch_bounds__(GB_THREADS) gg_build_kernel(const int32_t *__r
   const int32_t *ix = idx + (size_t)b * S + p0;
   const bool bulk_ok = ((reinterpret_cast<uintptr_t>(ix) & 15) == 0) && (len % 4 == 0);
   if (bulk_ok) {
-    if (tid == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
+    if (tid == 0) { mbarrier_init(&bar, 1); fence_mbarrier_init(); }
     __syncthreads();
     if (tid == 0) {
-      mbar_expect_tx(&bar, (unsigned)(len * sizeof(int)));
+      mbarrier_arrive_expect_tx(&bar, (unsigned)(len * sizeof(int)));
       bulk_g2s(s_idx, ix, (unsigned)(len * sizeof(int)), &bar);
     }
   } else {
@@ -460,7 +360,7 @@ __global__ void __launch_bounds__(GB_THREADS) gg_build_kernel(const int32_t *__r
   }
   for (int e = tid; e < Np; e += GB_THREADS) s_off[e] = 0;
   for (int e = tid; e < 32 * NBK; e += GB_THREADS) s_cnt[e] = 0;
-  if (bulk_ok) mbar_wait(&bar, 0);
+  if (bulk_ok) mbarrier_wait(&bar, 0);
   __syncthreads();
   // ---- histogram and scan: s_off[i] = number of positions with key < i ---------------------------------
   for (int t = tid; t < len; t += GB_THREADS) {
@@ -579,19 +479,19 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
   const bool bulk_ok = ((reinterpret_cast<uintptr_t>(g) & 15) == 0) && (S % 8 == 0) && (len % 8 == 0) &&
                        ((reinterpret_cast<uintptr_t>(ord_g) & 15) == 0) && ((reinterpret_cast<uintptr_t>(off_g) & 15) == 0);
   if (bulk_ok) {
-    if (tid == 0) { mbar_init(&bar, 1); fence_mbar_init(); }
+    if (tid == 0) { mbarrier_init(&bar, 1); fence_mbarrier_init(); }
     __syncthreads();
     if (tid == 0) {
       unsigned bytes = (unsigned)(ct * len * sizeof(float));
       if (LISTS_SMEM) bytes += (unsigned)(len * sizeof(uint16_t) + Np * sizeof(int));
-      mbar_expect_tx(&bar, bytes);
+      mbarrier_arrive_expect_tx(&bar, bytes);
       if (LISTS_SMEM) {       // lists first: they are needed first and come from L2
         bulk_g2s(s_off, off_g, (unsigned)(Np * sizeof(int)), &bar);
         bulk_g2s(s_ord, ord_g, (unsigned)(len * sizeof(uint16_t)), &bar);
       }
       for (int r = 0; r < ct; ++r) bulk_g2s(s_rows + (size_t)r * Sp, g + (size_t)r * S, (unsigned)(len * sizeof(float)), &bar);
     }
-    mbar_wait(&bar, 0);
+    mbarrier_wait(&bar, 0);
   } else {
     for (int r = 0; r < ct; ++r)
       for (int e = tid; e < len; e += GG_THREADS) s_rows[(size_t)r * Sp + e] = __ldg(g + (size_t)r * S + e);
@@ -948,20 +848,10 @@ extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *id
   int *offsets = reinterpret_cast<int *>(workspace);
   const size_t off_bytes = (size_t)B * g.H * (size_t)g.Np * sizeof(int);
   uint16_t *order = reinterpret_cast<uint16_t *>(reinterpret_cast<char *>(workspace) + off_bytes);
+  // histogram + scan + two-level stable sort in one kernel per (scene, partition)
   const size_t build_smem = gg_build_smem(N, g.Sp, g.Np);
-  if (N <= GB_MAX_N && build_smem <= 220 * 1024) {
-    // histogram + scan + two-level stable sort in one kernel per (scene, partition)
-    SPC_CUDA(cudaFuncSetAttribute(gg_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)build_smem));
-    gg_build_kernel<<<dim3(g.H, B), GB_THREADS, build_smem, stream>>>(idx, N, S, g.Sp, g.H, g.Np, offsets, order);
-  } else {
-    SPC_CUDA(cudaMemsetAsync(offsets, 0, off_bytes, stream));
-    gg_hist_kernel<<<dim3(ceil_div(S, 256), B), 256, 0, stream>>>(idx, N, S, g.Sp, g.H, g.Np, offsets);
-    gg_scan_kernel<<<B * g.H, 1024, 0, stream>>>(N, g.Np, offsets);
-    const size_t fill_smem = (size_t)g.Sp * sizeof(int);
-    SPC_CUDA(cudaFuncSetAttribute(gg_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fill_smem));
-    gg_fill_kernel<<<dim3(ceil_div(N, 32 * GG_FILL_WARPS), g.H, B), GG_FILL_WARPS * 32, fill_smem, stream>>>(
-        idx, N, S, g.Sp, g.H, g.Np, offsets, order);
-  }
+  SPC_CUDA(cudaFuncSetAttribute(gg_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)build_smem));
+  gg_build_kernel<<<dim3(g.H, B), GB_THREADS, build_smem, stream>>>(idx, N, S, g.Sp, g.H, g.Np, offsets, order);
   SPC_LAUNCH_CHECK("group_points_grad list build");
   if (g.H > 1) SPC_CUDA(cudaMemsetAsync(grad_points, 0, (size_t)B * C * N * sizeof(float), stream));
 #define GG_CASE(ct)                                                                                              \

@@ -17,6 +17,7 @@
 // between steps, every product with a (float64) rotation matrix / mean colour / translation is evaluated in float64
 // and rounded to float32 on assignment.
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace spc {
 
@@ -198,9 +199,9 @@ __global__ void __launch_bounds__(PP_THREADS) prepare_points_kernel(PrepArgs a) 
   const unsigned bytes = (unsigned)nrows * C * 4u;
   if ((((uintptr_t)o | bytes) & 15) == 0) {
     if (t == 0) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(o),
-                   "r"((unsigned)__cvta_generic_to_shared(s_tile)), "r"(bytes) : "memory");
+      fence_proxy_async_smem();
+      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(o), "r"(s2u(s_tile)), "r"(bytes)
+                   : "memory");
       asm volatile("cp.async.bulk.commit_group;" ::: "memory");
       asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the tile must outlive the copy's reads
     }

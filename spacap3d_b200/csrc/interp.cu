@@ -7,6 +7,7 @@
 // three_interpolate keeps (idx, weight) of a point in registers and sweeps channels with
 // coalesced stores, the small feature rows being served by L1.
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace spc {
 
@@ -75,34 +76,20 @@ __global__ void __launch_bounds__(NN_THREADS) three_nn_kernel(const float *__res
 // ------------------------------------------------------------------------------------------------
 constexpr int TI_THREADS = 256;
 
-__device__ __forceinline__ uint32_t ti_s2u(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 // one bulk-TMA copy global -> shared (bytes % 16 == 0, 16-byte aligned) or a plain copy; all threads call it
 __device__ __forceinline__ void ti_stage(float *dst, const float *src, size_t count, uint64_t *bar, int tid, int nthr) {
   const size_t bytes = count * sizeof(float);
   if (((reinterpret_cast<uintptr_t>(src) & 15) == 0) && bytes % 16 == 0 && bytes < (1u << 20)) {
     if (tid == 0) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(ti_s2u(bar)));
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+      mbarrier_init(bar, 1);
+      fence_mbarrier_init();
     }
     __syncthreads();
     if (tid == 0) {
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(ti_s2u(bar)), "r"((unsigned)bytes)
-                   : "memory");
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-                       "r"(ti_s2u(dst)),
-                   "l"(src), "r"((unsigned)bytes), "r"(ti_s2u(bar))
-                   : "memory");
+      mbarrier_arrive_expect_tx(bar, (unsigned)bytes);
+      bulk_g2s(dst, src, (unsigned)bytes, bar);
     }
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "TI_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n"
-        "@p bra TI_DONE;\n"
-        "bra TI_WAIT;\n"
-        "TI_DONE:\n"
-        "}\n" ::"r"(ti_s2u(bar))
-        : "memory");
+    mbarrier_wait(bar, 0);
   } else {
     for (size_t e = tid; e < count; e += nthr) dst[e] = __ldg(src + e);
     __syncthreads();

@@ -12,7 +12,7 @@
 // and the product is formed from three MMAs (hi.hi + lo.hi + hi.lo, fp32 accumulation in TMEM): ~2^-22 relative,
 // i.e. fp32-grade, for 3x the tensor work of layers that are far too small to be tensor-bound.
 //
-// Execution: one CTA per (128-row tile, 128-channel slice of N; the voting tail takes whole rows), 6 warps: warp 0 = TMA producer (cp.async.bulk.tensor, 128-byte swizzle, K
+// Execution: one CTA per (128-row tile, 128-channel slice of N; the voting tail takes whole rows), 6 warps: warp 0 = TMA producer (2-D tensor loads, 128-byte swizzle, K
 // in chunks of 64), warp 1 = MMA issuer (one thread, tcgen05.mma kind::f16, M = 128, N = N), warps 2-5 = epilogue
 // (TMEM lane = row, so a thread owns a point: channel-major stores are coalesced across the warp and the voting
 // tail's per-point L2 norm is a register reduction).  Two- to three-stage mbarrier pipeline between producer and
@@ -23,97 +23,9 @@
 #include <mutex>
 
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace spc {
-
-// ---- PTX wrappers (same conventions as sa_fused.cu) ---------------------------------------------------------
-__device__ __forceinline__ uint32_t pl_s2u(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void pl_mbar_init(uint64_t *bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(pl_s2u(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void pl_mbar_arrive(uint64_t *bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(pl_s2u(bar)) : "memory");
-}
-__device__ __forceinline__ void pl_mbar_expect_tx(uint64_t *bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(pl_s2u(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void pl_mbar_wait(uint64_t *bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "PL_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra PL_DONE;\n"
-      "bra PL_WAIT;\n"
-      "PL_DONE:\n"
-      "}\n" ::"r"(pl_s2u(bar)),
-      "r"(parity)
-      : "memory");
-}
-// 2-D tiled TMA load: box (64 elements of K, `rows` rows) at (k0, row0) -> shared memory, completion on `bar`
-__device__ __forceinline__ void pl_tma_load(void *dst, const CUtensorMap *tm, int k0, int row0, uint64_t *bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::
-          "r"(pl_s2u(dst)),
-      "l"(reinterpret_cast<uint64_t>(tm)), "r"(k0), "r"(row0), "r"(pl_s2u(bar))
-      : "memory");
-}
-__device__ __forceinline__ void pl_tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void pl_tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void pl_tmem_alloc(uint32_t *dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(pl_s2u(dst_smem)), "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void pl_tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void pl_umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void pl_umma_commit(uint64_t *bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(pl_s2u(bar))
-               : "memory");
-}
-__device__ __forceinline__ void pl_tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]),
-        "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]),
-        "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]),
-        "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-// instruction descriptor: D = F32, A = B = F16, both K-major (see sa_fused.cu make_idesc_f16)
-__host__ __device__ constexpr uint32_t pl_idesc_f16(int M, int N) {
-  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// shared-memory descriptor, K-major, 128-byte swizzle: 8-row groups 1024 B apart (see sa_fused.cu)
-__device__ __forceinline__ uint64_t pl_smem_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
 
 constexpr int PL_ROWS = 128;         // rows per tile = UMMA M
 constexpr int PL_KC = 64;            // K elements per pipeline chunk = one 128-byte swizzle atom
@@ -137,20 +49,12 @@ struct PmLinearParams {
   float *vote_xyz;             // vote mode: (B, n, 3)
 };
 
-__device__ __forceinline__ void pl_split(float h, __half &hi, __half &lo) {
-  uint16_t a, b;
-  asm("cvt.rn.satfinite.f16.f32 %0, %1;" : "=h"(a) : "f"(h));
-  hi = __ushort_as_half(a);
-  asm("cvt.rn.satfinite.f16.f32 %0, %1;" : "=h"(b) : "f"(h - __half2float(hi)));
-  lo = __ushort_as_half(b);
-}
-
 __global__ void __launch_bounds__(PL_THREADS, 1)
 pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
                  const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
                  const PmLinearParams p) {
   extern __shared__ __align__(128) uint8_t pl_smem_raw[];
-  uint8_t *smem = pl_smem_raw + ((1024u - (pl_s2u(pl_smem_raw) & 1023u)) & 1023u);   // swizzle atoms: 1024-byte aligned
+  uint8_t *smem = pl_smem_raw + ((1024u - (s2u(pl_smem_raw) & 1023u)) & 1023u);   // swizzle atoms: 1024-byte aligned
   __shared__ __align__(8) uint64_t full[PL_MAX_STAGES], empty[PL_MAX_STAGES], acc_full[2], acc_empty[2];
   __shared__ uint32_t tmem_base_smem;
   __shared__ float s_bias[288];
@@ -187,15 +91,15 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
   const uint32_t tmem_cols = Nr > 256 ? 512u : (uint32_t)(NBUF * BUFC);
 
   if (tid == 0) {
-    for (int s = 0; s < p.stages; ++s) { pl_mbar_init(&full[s], 1); pl_mbar_init(&empty[s], 1); }
-    for (int u = 0; u < 2; ++u) { pl_mbar_init(&acc_full[u], 1); pl_mbar_init(&acc_empty[u], 128); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < p.stages; ++s) { mbarrier_init(&full[s], 1); mbarrier_init(&empty[s], 1); }
+    for (int u = 0; u < 2; ++u) { mbarrier_init(&acc_full[u], 1); mbarrier_init(&acc_empty[u], 128); }
+    fence_mbarrier_init();
   }
-  if (warp == 1) pl_tmem_alloc(&tmem_base_smem, tmem_cols);
+  if (warp == 1) tmem_alloc(&tmem_base_smem, tmem_cols);
   for (int e = tid; e < 288; e += PL_THREADS) s_bias[e] = e < Nt ? __ldg(p.bias + n_off + e) : 0.f;
-  pl_tc_fence_before();
+  tc_fence_before();
   __syncthreads();
-  pl_tc_fence_after();
+  tc_fence_after();
   const uint32_t tmem_base = tmem_base_smem;
 
   if (warp == 0) {
@@ -206,17 +110,17 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
         const int row0 = (tile0 + i) * PL_ROWS;
         for (int c = 0; c < KCH; ++c, ++g) {                  // g: chunk counter over all tiles (the stage ring goes on)
           const int s = g % p.stages;
-          if (g >= p.stages) pl_mbar_wait(&empty[s], (unsigned)((g / p.stages - 1) & 1));
+          if (g >= p.stages) mbarrier_wait(&empty[s], (unsigned)((g / p.stages - 1) & 1));
           uint8_t *st = stage0 + (size_t)s * STAGE_BYTES;
           const bool load_w = !p.resident || i == 0;
-          pl_mbar_expect_tx(&full[s], (unsigned)(A_STAGE + (load_w ? W_CHUNK : 0)));
-          pl_tma_load(st, &tmA_hi, c * PL_KC, row0, &full[s]);
-          if (p.has_lo) pl_tma_load(st + A_BYTES, &tmA_lo, c * PL_KC, row0, &full[s]);
+          mbarrier_arrive_expect_tx(&full[s], (unsigned)(A_STAGE + (load_w ? W_CHUNK : 0)));
+          tma_load_2d(st, &tmA_hi, c * PL_KC, row0, &full[s]);
+          if (p.has_lo) tma_load_2d(st + A_BYTES, &tmA_lo, c * PL_KC, row0, &full[s]);
           if (load_w) {
             uint8_t *b = p.resident ? smem + (size_t)c * W_CHUNK : st + A_STAGE;
             for (int r = 0; r < Nr; r += BR) {
-              pl_tma_load(b + (size_t)r * 128, &tmB_hi, c * PL_KC, n_off + r, &full[s]);
-              pl_tma_load(b + B_BYTES + (size_t)r * 128, &tmB_lo, c * PL_KC, n_off + r, &full[s]);
+              tma_load_2d(b + (size_t)r * 128, &tmB_hi, c * PL_KC, n_off + r, &full[s]);
+              tma_load_2d(b + B_BYTES + (size_t)r * 128, &tmB_lo, c * PL_KC, n_off + r, &full[s]);
             }
           }
         }
@@ -225,39 +129,40 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
   } else if (warp == 1) {
     // =============================== MMA ISSUER (one thread) =======================================
     if (lane == 0) {
-      const uint32_t idesc1 = pl_idesc_f16(PL_ROWS, N1), idesc2 = pl_idesc_f16(PL_ROWS, 16);
+      const uint32_t idesc1 = make_idesc_f16(PL_ROWS, N1), idesc2 = make_idesc_f16(PL_ROWS, 16);
       for (int i = 0, g = 0; i < ntile; ++i) {
       const int buf = i % NBUF;
       const uint32_t tacc = tmem_base + (uint32_t)(buf * BUFC);
       if (i >= NBUF) {                                        // the epilogue has drained this buffer (tile i - NBUF)
-        pl_mbar_wait(&acc_empty[buf], (unsigned)((i / NBUF - 1) & 1));
-        pl_tc_fence_after();
+        mbarrier_wait(&acc_empty[buf], (unsigned)((i / NBUF - 1) & 1));
+        tc_fence_after();
       }
       for (int c = 0; c < KCH; ++c, ++g) {
         const int s = g % p.stages;
-        pl_mbar_wait(&full[s], (unsigned)((g / p.stages) & 1));
-        pl_tc_fence_after();
-        const uint32_t aH = pl_s2u(stage0 + (size_t)s * STAGE_BYTES);
+        mbarrier_wait(&full[s], (unsigned)((g / p.stages) & 1));
+        tc_fence_after();
+        const uint32_t aH = s2u(stage0 + (size_t)s * STAGE_BYTES);
         const uint32_t aL = aH + A_BYTES;
-        const uint32_t bH = p.resident ? pl_s2u(smem + (size_t)c * W_CHUNK) : aH + A_STAGE;
+        const uint32_t bH = p.resident ? s2u(smem + (size_t)c * W_CHUNK) : aH + A_STAGE;
         const uint32_t bL = bH + B_BYTES;
 #pragma unroll
         for (int kk = 0; kk < PL_KC / 16; ++kk) {
           const uint32_t ko = kk * 32;                        // 16 fp16 = 32 bytes inside the 128-byte atom
           const uint32_t acc = (c > 0 || kk > 0) ? 1u : 0u;
-          pl_umma_f16(tacc, pl_smem_desc(aH + ko), pl_smem_desc(bH + ko), idesc1, acc);
-          pl_umma_f16(tacc, pl_smem_desc(aH + ko), pl_smem_desc(bL + ko), idesc1, 1u);
-          if (p.has_lo) pl_umma_f16(tacc, pl_smem_desc(aL + ko), pl_smem_desc(bH + ko), idesc1, 1u);
+          umma_f16(tacc, make_smem_desc_sw128(aH + ko), make_smem_desc_sw128(bH + ko), idesc1, acc);
+          umma_f16(tacc, make_smem_desc_sw128(aH + ko), make_smem_desc_sw128(bL + ko), idesc1, 1u);
+          if (p.has_lo) umma_f16(tacc, make_smem_desc_sw128(aL + ko), make_smem_desc_sw128(bH + ko), idesc1, 1u);
           if (N2) {
             const uint32_t off = (uint32_t)N1 * 128u;         // weight rows N1.. : 1024-byte aligned (N1 % 8 == 0)
-            pl_umma_f16(tacc + N1, pl_smem_desc(aH + ko), pl_smem_desc(bH + off + ko), idesc2, acc);
-            pl_umma_f16(tacc + N1, pl_smem_desc(aH + ko), pl_smem_desc(bL + off + ko), idesc2, 1u);
-            if (p.has_lo) pl_umma_f16(tacc + N1, pl_smem_desc(aL + ko), pl_smem_desc(bH + off + ko), idesc2, 1u);
+            umma_f16(tacc + N1, make_smem_desc_sw128(aH + ko), make_smem_desc_sw128(bH + off + ko), idesc2, acc);
+            umma_f16(tacc + N1, make_smem_desc_sw128(aH + ko), make_smem_desc_sw128(bL + off + ko), idesc2, 1u);
+            if (p.has_lo)
+              umma_f16(tacc + N1, make_smem_desc_sw128(aL + ko), make_smem_desc_sw128(bH + off + ko), idesc2, 1u);
           }
         }
-        pl_umma_commit(&empty[s]);                            // the stage may be refilled once these MMAs have read it
+        umma_commit(&empty[s]);                               // the stage may be refilled once these MMAs have read it
       }
-      pl_umma_commit(&acc_full[buf]);
+      umma_commit(&acc_full[buf]);
       }
     }
   } else {
@@ -268,8 +173,8 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
     const int buf = i % NBUF;
     const long long row = (long long)(tile0 + i) * PL_ROWS + r;
     const bool ok = row < p.M;
-    pl_mbar_wait(&acc_full[buf], (unsigned)((i / NBUF) & 1));
-    pl_tc_fence_after();
+    mbarrier_wait(&acc_full[buf], (unsigned)((i / NBUF) & 1));
+    tc_fence_after();
     const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * BUFC);
     const int b = ok ? (int)(row / p.n) : 0;
     const int j = ok ? (int)(row - (long long)b * p.n) : 0;
@@ -278,7 +183,7 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       const bool relu = p.mode == SPC_PM_HIDDEN || p.mode == SPC_PM_OUT_CM;
       for (int c0 = 0; c0 < Nr; c0 += 32) {
         float v[32];
-        pl_tmem_ld32(taddr + c0, v);
+        tmem_ld32(taddr + c0, v);
         if (!ok) continue;
 #pragma unroll
         for (int i = 0; i < 32; ++i) {
@@ -302,8 +207,8 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
           __half h0, l0, h1, l1;
-          pl_split(v[2 * i], h0, l0);
-          pl_split(v[2 * i + 1], h1, l1);
+          split_f16(v[2 * i], h0, l0);
+          split_f16(v[2 * i + 1], h1, l1);
           hw[i] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
           lw[i] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
         }
@@ -329,7 +234,7 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       float ss = 0.f;
       for (int c0 = 0; c0 < D; c0 += 32) {
         float v[32];
-        pl_tmem_ld32(taddr + c0, v);
+        tmem_ld32(taddr + c0, v);
         if (!ok) continue;
 #pragma unroll
         for (int i = 0; i < 32; ++i) {
@@ -339,7 +244,7 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       }
       {
         float v[32];
-        pl_tmem_ld32(taddr + D, v);                           // columns D .. D+2: the xyz offsets
+        tmem_ld32(taddr + D, v);                              // columns D .. D+2: the xyz offsets
         if (ok) {
           const float *sx = p.seed_xyz + row * 3;
           float *vx = p.vote_xyz + row * 3;
@@ -352,7 +257,7 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
       float *o = p.out + (size_t)b * D * p.n + j;
       for (int c0 = 0; c0 < D; c0 += 32) {
         float v[32];
-        pl_tmem_ld32(taddr + c0, v);
+        tmem_ld32(taddr + c0, v);
         if (!ok) continue;
         uint32_t hw[16], lw[16];
 #pragma unroll
@@ -363,8 +268,8 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
           __half h0, l0, h1, l1;
-          pl_split(v[2 * i], h0, l0);
-          pl_split(v[2 * i + 1], h1, l1);
+          split_f16(v[2 * i], h0, l0);
+          split_f16(v[2 * i + 1], h1, l1);
           hw[i] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
           lw[i] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
         }
@@ -378,14 +283,14 @@ pm_linear_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_consta
         }
       }
     }
-    pl_tc_fence_before();
-    pl_mbar_arrive(&acc_empty[buf]);
+    tc_fence_before();
+    mbarrier_arrive(&acc_empty[buf]);
     }
   }
   __syncthreads();
   if (warp == 1) {
-    pl_tc_fence_after();
-    pl_tmem_dealloc(tmem_base, tmem_cols);
+    tc_fence_after();
+    tmem_dealloc(tmem_base, tmem_cols);
   }
 }
 

@@ -1,130 +1,16 @@
-// sa_common.cuh -- PTX wrappers (mbarrier, tcgen05 alloc / mma / commit / ld / fences), the UMMA descriptors of the
-// 128-byte-swizzle K-major shared-memory layout and the launch parameters shared by the two fused set-abstraction
-// kernels: sa_fused.cu (projected layer 0, SA2-SA4 / vote aggregation) and sa_inline.cu (in-line layer 0, SA1).
+// sa_common.cuh -- offsets into the 128-byte-swizzle K-major shared-memory layout, weight staging, the pooled epilogue
+// and the launch parameters shared by the two fused set-abstraction kernels: sa_fused.cu (projected layer 0, SA2-SA4 /
+// vote aggregation) and sa_inline.cu (in-line layer 0, SA1).  The PTX wrappers they use are in ptx.cuh.
 #pragma once
 #include <cuda_fp16.h>
 
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace spc {
 
-// ---------------------------------------------------------------------------------------------
-// PTX wrappers: mbarrier, tcgen05 (alloc / mma / commit / ld / fences)
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t s2u(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbarrier_init(uint64_t *bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s2u(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbarrier_wait(uint64_t *bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "SA_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra SA_DONE;\n"
-      "bra SA_WAIT;\n"
-      "SA_DONE:\n"
-      "}\n" ::"r"(s2u(bar)),
-      "r"(parity)
-      : "memory");
-}
-// same, for the gather / epilogue warps, which share their SM sub-partitions with each other: try_wait with a
-// suspend-time hint parks the thread in hardware until the phase completes or the hint expires -- ~4 attempts per
-// wait in ncu, against a tight spin that stole 25-30 % of the issue slots (round 1) and a nanosleep back-off that
-// still spent ~15 % of the kernel's instructions on polling.
-__device__ __forceinline__ void mbarrier_wait_relaxed(uint64_t *bar, unsigned parity) {
-  // the retry loop stays inside the asm block: try_wait + one predicated branch per attempt (exported through selp
-  // into a C++ loop every attempt cost ~8 instructions: selp, setp, divergence bookkeeping)
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "SA_RWAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-      "@!p bra SA_RWAIT;\n"
-      "}\n" ::"r"(s2u(bar)),
-      "r"(parity), "r"(20000u)
-      : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_smem() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_before() {
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_after() {
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t *dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s2u(dst_smem)),
-               "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// D[tmem] (+)= A[smem] . B[smem]^T ; one thread issues for the CTA
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
-                                          uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on an mbarrier once every previously issued MMA of this thread has completed
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s2u(bar))
-               : "memory");
-}
-// 32 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]),
-        "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]),
-        "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]),
-        "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// UMMA instruction descriptor (cute::UMMA::InstrDescriptor): c_format (bits 4-5) = 1 (F32), a_format (7-9) =
-// b_format (10-12) = 0 (F16; 1 would be BF16), both operands K-major, N >> 3 at bit 17, M >> 4 at bit 24.
-// fp16 operands carry 11 significant bits (bf16: 8): the fused MLP lands ~8x closer to the fp32 reference for the
-// same tensor-pipe rate and shared-memory footprint.  Conversions saturate (cvt ... .satfinite) instead of
-// producing inf above 65504, a range the BN-folded activations of this network never approach.
-__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N) {
-  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-// UMMA shared-memory descriptor (cute::UMMA::SmemDescriptor bit layout: [0,14) start address >> 4,
-// [16,30) leading byte offset >> 4, [32,46) stride byte offset >> 4, [46,48) version = 1,
-// [61,64) layout type) for the 128-byte-swizzle K-major layout (type 2): a row is 128 contiguous
-// bytes (64 fp16), 8-row groups are 1024 B apart (SBO), the 16-byte chunk c of row r sits at chunk
-// position c ^ (r & 7) (Swizzle<3,4,3>); K beyond 64 elements continues in the next "K atom",
-// rows*128 bytes further.  The leading-byte-offset field is unused for swizzled K-major (= 1).
-__device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-// byte offset of the 16-byte chunk (row, kc) of a [rows x K] fp16 operand in that layout
+// byte offset of the 16-byte chunk (row, kc) of a [rows x K] fp16 operand in the layout of make_smem_desc_sw128
+// (ptx.cuh)
 __device__ __forceinline__ uint32_t sw128_off(int row, int kc, int rows) {
   return (uint32_t)((kc >> 3) * rows * 128 + row * 128 + (((kc & 7) ^ (row & 7)) << 4));
 }
@@ -140,12 +26,6 @@ __device__ __forceinline__ uint32_t pack_relu_f16x2(float lo, float hi) {
   asm("cvt.rn.satfinite.relu.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
 }
-__device__ __forceinline__ __half to_f16_sat(float v) {
-  uint16_t r;
-  asm("cvt.rn.satfinite.f16.f32 %0, %1;" : "=h"(r) : "f"(v));
-  return __ushort_as_half(r);
-}
-
 
 // ---------------------------------------------------------------------------------------------
 struct SaFusedParams {
@@ -177,10 +57,6 @@ constexpr int SA_MAX_K0 = 3 + 13;   // the in-line form supports up to 13 raw fe
 // scene of a tile (tiles never straddle scenes: npoint*nsample % 128 == 0 is checked at launch)
 __device__ __forceinline__ int sa_tile_scene(const SaFusedParams &p, int tile, int tiles_per_scene) {
   return p.tps_magic ? (int)__umulhi((unsigned)tile, p.tps_magic) : tile / tiles_per_scene;
-}
-
-__device__ __forceinline__ void mbarrier_arrive(uint64_t *bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s2u(bar)) : "memory");
 }
 
 // Row-major fp16 weights (ROWS, 8*KCH) -> the swizzled UMMA layout in shared memory; 8 x 16-byte loads in flight

@@ -181,7 +181,7 @@ __global__ void __launch_bounds__(SAP_THREADS, 1) sa_fused_pipe_kernel(const SaF
       mbarrier_init(&d2_full[s], 1);
       mbarrier_init(&d2_empty[s], 128);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   tc_fence_before();
   __syncthreads();
@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(SAP_THREADS, 1) sa_fused_pipe_kernel(const SaF
     sa_stage_weights<C3, C2 / 8, NT>(sW2, p.W2, t);
     for (int e = t; e < C2; e += NT) sB1[e] = __ldg(p.b1 + e);
     fence_proxy_async_smem();
-    asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");
+    named_bar_sync<1, NT>();
   }
   const uint32_t tmem_base = tmem_base_smem;
   const int tiles_per_scene = (p.np * NS) / SA_ROWS;

@@ -60,11 +60,6 @@ struct SaInlineSmem {
   static constexpr int TMEM_COLS = OCC == 2 ? 256 : 512;
 };
 
-// fp16 (hi, lo) split of a float: v ~= hi + lo with |v - hi - lo| <= 2^-22 |v| (+ the fp16 subnormal floor)
-__device__ __forceinline__ void sai_split(float v, __half &hi, __half &lo) {
-  hi = to_f16_sat(v);
-  lo = to_f16_sat(v - __half2float(hi));
-}
 template <int C1, int C2, int C3, int NS, int OCC>
 __global__ void __launch_bounds__(SAI_THREADS, OCC) sa_inline_kernel(const SaFusedParams p) {
   using L = SaInlineSmem<C1, C2, C3, OCC>;
@@ -104,7 +99,7 @@ __global__ void __launch_bounds__(SAI_THREADS, OCC) sa_inline_kernel(const SaFus
     mbarrier_init(&d1_empty, 128);
     mbarrier_init(&h2_full, 128);
     mbarrier_init(&h2_empty, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   tc_fence_before();
   __syncthreads();
@@ -129,11 +124,11 @@ __global__ void __launch_bounds__(SAI_THREADS, OCC) sa_inline_kernel(const SaFus
       } else {
         __half lo[4], hi;
 #pragma unroll
-        for (int u = 0; u < 4; ++u) sai_split(w[u], hi, lo[u]);
+        for (int u = 0; u < 4; ++u) split_f16(w[u], hi, lo[u]);
         o[0] = (uint32_t)__half_as_ushort(lo[0]) | ((uint32_t)__half_as_ushort(lo[1]) << 16);
         o[1] = (uint32_t)__half_as_ushort(lo[2]) | ((uint32_t)__half_as_ushort(lo[3]) << 16);
         __half bh = __float2half_rn(0.f), bl = bh;
-        if (g == 0) sai_split(__ldg(p.b0 + c), bh, bl);
+        if (g == 0) split_f16(__ldg(p.b0 + c), bh, bl);
         o[2] = (uint32_t)__half_as_ushort(bh) | ((uint32_t)__half_as_ushort(bl) << 16);
         o[3] = 0u;
       }
@@ -143,7 +138,7 @@ __global__ void __launch_bounds__(SAI_THREADS, OCC) sa_inline_kernel(const SaFus
     sa_stage_weights<C3, C2 / 8, NT>(sW2, p.W2, t);
     for (int e = t; e < C2; e += NT) sB1[e] = __ldg(p.b1 + e);
     fence_proxy_async_smem();
-    asm volatile("bar.sync 1, %0;" ::"n"(NT) : "memory");
+    named_bar_sync<1, NT>();
   }
   const uint32_t tmem_base = tmem_base_smem;
   const int tiles_per_scene = (p.np * NS) / SA_ROWS;

@@ -142,16 +142,6 @@ class _FoldedMLP:
         self.data = None
         self._w0f_t = None
         self._w0x = None
-        self._host0 = None
-
-    def host0(self, W0, b0):
-        """Host copies of the folded layer-0 weights (the fused kernel takes them by value through its
-        parameters when they are small).  One device->host copy per weight refresh, never inside a graph capture."""
-        if self._host0 is None:
-            if torch.cuda.is_current_stream_capturing():
-                return None, None
-            self._host0 = (W0.cpu().contiguous(), b0.cpu().contiguous())
-        return self._host0
 
     def w0f(self, W0):
         """((C1, Cf) fp16 hi, lo): feature columns of the folded conv0 for the projection layer (spc_pm_linear),
@@ -173,7 +163,7 @@ class _FoldedMLP:
         if key != self.key:
             self.key = key
             self.data = None
-            self._w0f_t = self._w0x = self._host0 = None
+            self._w0f_t = self._w0x = None
             blocks = list(mlp.children())
             if len(blocks) == 3:
                 folded = [_fold_conv_bn(b) for b in blocks]
@@ -372,9 +362,8 @@ class PointnetSAModuleVotes(nn.Module):
         try:
             if Cf <= INLINE_MAX_FEATURES:
                 feat = None if features is None else features.contiguous()
-                W0h, b0h = cache.host0(W0, b0)
                 out, out_pm = _ext.sa_fused_forward(xyz, new_xyz, idx, W0, b0, W1, b1, W2, b2, feat=feat,
-                                                    radius=radius, want_point_major=True, W0_host=W0h, b0_host=b0h)
+                                                    radius=radius, want_point_major=True)
             else:
                 # conv0 hoisted out of the grouping: ONE tcgen05 layer over the n points gives the
                 # per-point feature projection; the xyz columns stay in fp32 inside the kernel

@@ -48,7 +48,7 @@ def _q(t):
 
 
 def _split16(t):
-    """The kernels' fp16 (hi, lo) split of fp32 data (_ext.split_half, sai_split, put_group, pl_split), as float64."""
+    """The kernels' fp16 (hi, lo) split of fp32 data (_ext.split_half, split_f16, put_group), as float64."""
     f = t.float()
     assert torch.equal(f.double(), t), "value not representable in fp32"
     hi = f.half()
@@ -427,7 +427,7 @@ def test_pm_linear_exact(case):
         else:
             vote_xyz, out, (hi, lo) = res
             assert torch.equal(vote_xyz.double().cpu(), ref["vote_xyz"]), (hint, _mismatch(vote_xyz, ref["vote_xyz"]))
-            # The pair is the kernel's own fp32 result split by pl_split: exactly reproducible from `out`.
+            # The pair is the kernel's own fp32 result split by split_f16: exactly reproducible from `out`.
             pm = out.transpose(1, 2).reshape(M, N - 3)
             assert torch.equal(hi, pm.half()), hint
             if want_lo:
