@@ -220,7 +220,7 @@ def group_grad_big_cases():
     c["sa2_like_two_partitions"] = (padded(2, 2048, 1024, 32, 40), 9, 2048)       # S=32768 -> H=2, CT=1
     c["sa3_like"] = (padded(2, 1024, 512, 16, 25), 10, 1024)                      # S=8192  -> H=1, CT=2
     c["sa4_like_ct4"] = (padded(3, 512, 256, 16, 10), 7, 512)                     # S=4096  -> CT=4, C%4 != 0
-    c["three_partitions"] = (padded(1, 3000, 1000, 60, 100), 4, 3000)             # S=60000 -> H=3
+    c["three_partitions"] = (padded(1, 3000, 1000, 60, 100), 6, 3000)             # S=60000 -> H=3 (N <= 512*C)
     c["odd_unaligned"] = (padded(2, 333, 77, 13, 5), 5, 333)                      # S=1001: no bulk copy
     c["one_hub"] = (np.zeros((1, 64, 16), np.int32) + 7, 6, 50)                   # every position -> point 7
     # N > 8192: one list per point over all positions + point-owned gather (atomic cursors: order not deterministic)
