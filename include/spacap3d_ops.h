@@ -269,6 +269,47 @@ int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint8_t *argmax
                                        int npoint, int nsample, float *dy, float *dgamma, float *dbeta,
                                        void *stream);
 
+/* ---- synchronised training-mode BatchNorm (+ ReLU, + max-pool) across the ranks of a process group -------------
+ * torch.nn.SyncBatchNorm semantics on the kernels above: the statistics and the backward sums of dm and dm*xhat are
+ * taken over the elements of every rank; dgamma / dbeta stay the local sums (the gradient all-reduce adds them).
+ * Each pass is split at its one cross-rank reduction.  A rank writes its row `stats` (C, SPC_BN_SYNC_K) fp64:
+ *   forward : (n, mean, M2) of its B*S elements per channel       (spc_bn_relu_sync_stats, both variants)
+ *   backward: (n, sum dm, sum dm * xhat) per channel              (..._sync_backward_reduce)
+ * The caller gathers the rows of all `world` ranks into `stats_all` (world, C, SPC_BN_SYNC_K), rank r at row r (a SUM
+ * all-reduce of a zero-initialised buffer does that exactly), and the next call combines them in rank order on the
+ * device: every rank gets bit-identical statistics, whatever the collective's reduction order.  The global count
+ * comes from the rows, so ranks may hold different B.  No host synchronisation; any B >= 0 (no B*C limit; with
+ * B = 0, an empty shard, the rank still takes part: its rows have n = 0 and its tensor pointers may be NULL).
+ * The backward apply calls use the workspace (spc_bn_relu_workspace_bytes(C) bytes) as scratch. */
+#define SPC_BN_SYNC_K 3
+int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, double *stats, void *workspace,
+                           size_t workspace_bytes, void *stream);
+int spc_bn_relu_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S, int world,
+                             const double *stats_all, float eps, float momentum, float *running_mean,
+                             float *running_var, float *z, float *save_mean, float *save_invstd, void *stream);
+int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y, const float *gamma, const float *beta,
+                                     const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                     float *dgamma, float *dbeta, double *stats, void *workspace,
+                                     size_t workspace_bytes, void *stream);
+int spc_bn_relu_sync_backward(const float *dz, const float *y, const float *gamma, const float *beta,
+                              const float *save_mean, const float *save_invstd, int B, int C, int S, int world,
+                              const double *stats_all, float *dy, void *workspace, size_t workspace_bytes,
+                              void *stream);
+/* max-pool variant; its statistics phase is the plain one with S = npoint*nsample */
+int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C, int npoint,
+                                     int nsample, int world, const double *stats_all, float eps, float momentum,
+                                     float *running_mean, float *running_var, float *pooled, uint8_t *argmax,
+                                     float *ymax, float *save_mean, float *save_invstd, void *stream);
+int spc_bn_relu_maxpool_sync_backward_reduce(const float *dpool, const float *ymax, const float *gamma,
+                                             const float *beta, const float *save_mean, const float *save_invstd,
+                                             int B, int C, int npoint, int nsample, float *dgamma, float *dbeta,
+                                             double *stats, void *stream);
+int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8_t *argmax, const float *ymax, const float *y,
+                                      const float *gamma, const float *beta, const float *save_mean,
+                                      const float *save_invstd, int B, int C, int npoint, int nsample, int world,
+                                      const double *stats_all, float *dy, void *workspace, size_t workspace_bytes,
+                                      void *stream);
+
 /* ---- detection post-processing (SURVEY row N3): device side of parse_predictions, lib/ap_helper.py:44-160 ----
  * spc_box_point_counts: counts[b,k] = number of points of scene b inside predicted box k (the reference's
  *   extract_pc_in_box3d / scipy Delaunay hull test per box, ap_helper.py:69-79, data/scannet/model_util_scannet.py:

@@ -7,6 +7,7 @@ Differences, all invisible to callers: outputs are allocated with torch.empty (e
 written by the kernels), launches go to torch's *current* stream under a device guard taken from
 the input tensor, and a failed launch raises instead of calling exit(-1).
 """
+import math
 import threading
 
 import torch
@@ -505,6 +506,144 @@ def bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, mean, in
                   y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C,
                   npoint, nsample, dy.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _stream())
     return dy, dgamma, dbeta
+
+
+# ---- synchronised BatchNorm: the phases around the cross-rank exchange (include/spacap3d_ops.h) ----------------------
+BN_SYNC_K = 3          # SPC_BN_SYNC_K: fp64 values per channel in an exchanged row
+
+
+def _check_rows(rows, C, what):
+    _check(rows, what, torch.float64)
+    if rows.dim() < 2 or tuple(rows.shape[-2:]) != (C, BN_SYNC_K):
+        raise RuntimeError("%s must have shape (..., %d, %d)" % (what, C, BN_SYNC_K))
+
+
+def _bn_sizes(y):
+    """(B, C, S) of y (B,C,*); B may be 0 (a rank with an empty shard still takes part in the exchange)."""
+    return y.shape[0], y.shape[1], math.prod(y.shape[2:])
+
+
+def bn_relu_sync_stats(y, row):
+    """This rank's per-channel (n, mean, M2) of y (B,C,*) f32 into row (C, BN_SYNC_K) f64; also the statistics phase
+    of the max-pool variant."""
+    _check(y, "y", torch.float32)
+    B, C, S = _bn_sizes(y)
+    _check_rows(row, C, "row")
+    _same_device(y, row)
+    with torch.cuda.device(y.device):
+        ws, nbytes = _bn_workspace(C, y.device)
+        _lib.call("spc_bn_relu_sync_stats", y.data_ptr(), B, C, S, row.data_ptr(), ws.data_ptr(), nbytes, _stream())
+
+
+def bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps, rows):
+    """z = relu(batch_norm(y)) with the statistics combined from rows (world, C, BN_SYNC_K), every rank's
+    bn_relu_sync_stats row: returns (z, save_mean, save_invstd); running_mean / running_var (or None) are updated
+    in place with the global mean and unbiased variance."""
+    _check(y, "y", torch.float32)
+    _check(gamma, "gamma", torch.float32)
+    _check(beta, "beta", torch.float32)
+    B, C, S = _bn_sizes(y)
+    _check_rows(rows, C, "rows")
+    _same_device(y, gamma, beta, rows)
+    z = torch.empty_like(y)
+    mean = torch.empty(C, dtype=torch.float32, device=y.device)
+    invstd = torch.empty(C, dtype=torch.float32, device=y.device)
+    with torch.cuda.device(y.device):
+        _lib.call("spc_bn_relu_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
+                  rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
+                  running_mean.data_ptr() if running_mean is not None else None,
+                  running_var.data_ptr() if running_var is not None else None,
+                  z.data_ptr(), mean.data_ptr(), invstd.data_ptr(), _stream())
+    return z, mean, invstd
+
+
+def bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, row):
+    """-> (dgamma, dbeta) of this rank; writes its (n, sum dm, sum dm * xhat) into row (C, BN_SYNC_K) f64."""
+    _check(dz, "dz", torch.float32)
+    _check(y, "y", torch.float32)
+    B, C, S = _bn_sizes(y)
+    _check_rows(row, C, "row")
+    _same_device(dz, y, row)
+    dgamma = torch.empty(C, dtype=torch.float32, device=y.device)
+    dbeta = torch.empty(C, dtype=torch.float32, device=y.device)
+    with torch.cuda.device(y.device):
+        ws, nbytes = _bn_workspace(C, y.device)
+        _lib.call("spc_bn_relu_sync_backward_reduce", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+                  mean.data_ptr(), invstd.data_ptr(), B, C, S, dgamma.data_ptr(), dbeta.data_ptr(), row.data_ptr(),
+                  ws.data_ptr(), nbytes, _stream())
+    return dgamma, dbeta
+
+
+def bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, rows):
+    """-> dy from dz, y and every rank's bn_relu_sync_backward_reduce row (rows (world, C, BN_SYNC_K))."""
+    _check(dz, "dz", torch.float32)
+    _check(y, "y", torch.float32)
+    B, C, S = _bn_sizes(y)
+    _check_rows(rows, C, "rows")
+    _same_device(dz, y, rows)
+    dy = torch.empty_like(y)
+    with torch.cuda.device(y.device):
+        ws, nbytes = _bn_workspace(C, y.device)
+        _lib.call("spc_bn_relu_sync_backward", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+                  mean.data_ptr(), invstd.data_ptr(), B, C, S, rows.shape[0], rows.data_ptr(), dy.data_ptr(),
+                  ws.data_ptr(), nbytes, _stream())
+    return dy
+
+
+def bn_relu_maxpool_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps, rows):
+    """bn_relu_maxpool_train_forward with the statistics combined from rows (world, C, BN_SYNC_K), every rank's
+    bn_relu_sync_stats row of its y (B,C,npoint,nsample): -> (pooled, argmax, ymax, save_mean, save_invstd)."""
+    _check(y, "y", torch.float32)
+    _check(gamma, "gamma", torch.float32)
+    _check(beta, "beta", torch.float32)
+    B, C, npoint, nsample = y.shape
+    _check_rows(rows, C, "rows")
+    _same_device(y, gamma, beta, rows)
+    dev = y.device
+    pooled = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
+    argmax = torch.empty((B, C, npoint), dtype=torch.uint8, device=dev)
+    ymax = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
+    mean = torch.empty(C, dtype=torch.float32, device=dev)
+    invstd = torch.empty(C, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.call("spc_bn_relu_maxpool_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
+                  npoint, nsample, rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
+                  running_mean.data_ptr() if running_mean is not None else None,
+                  running_var.data_ptr() if running_var is not None else None,
+                  pooled.data_ptr(), argmax.data_ptr(), ymax.data_ptr(), mean.data_ptr(), invstd.data_ptr(), _stream())
+    return pooled, argmax, ymax, mean, invstd
+
+
+def bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, row):
+    """-> (dgamma, dbeta) of this rank for the max-pool variant; writes its row (C, BN_SYNC_K) f64."""
+    _check(dpool, "dpool", torch.float32)
+    _check(ymax, "ymax", torch.float32)
+    _same_device(dpool, ymax, row)
+    B, C, npoint, nsample = y.shape
+    _check_rows(row, C, "row")
+    dgamma = torch.empty(C, dtype=torch.float32, device=dpool.device)
+    dbeta = torch.empty(C, dtype=torch.float32, device=dpool.device)
+    with torch.cuda.device(dpool.device):
+        _lib.call("spc_bn_relu_maxpool_sync_backward_reduce", dpool.data_ptr(), ymax.data_ptr(), gamma.data_ptr(),
+                  beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C, npoint, nsample, dgamma.data_ptr(),
+                  dbeta.data_ptr(), row.data_ptr(), _stream())
+    return dgamma, dbeta
+
+
+def bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd, rows):
+    """-> dy (B,C,npoint,nsample) from dpool and every rank's bn_relu_maxpool_sync_backward_reduce row."""
+    _check(dpool, "dpool", torch.float32)
+    _check(y, "y", torch.float32)
+    B, C, npoint, nsample = y.shape
+    _check_rows(rows, C, "rows")
+    _same_device(dpool, y, rows)
+    dy = torch.empty_like(y)
+    with torch.cuda.device(y.device):
+        ws, nbytes = _bn_workspace(C, y.device)
+        _lib.call("spc_bn_relu_maxpool_sync_backward", dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
+                  y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C,
+                  npoint, nsample, rows.shape[0], rows.data_ptr(), dy.data_ptr(), ws.data_ptr(), nbytes, _stream())
+    return dy
 
 
 def box_point_counts(points, corners):

@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # SPC_LIB_PATH lets a developer load an instrumented build of the same library (profiling only)
 LIB_PATH = os.environ.get("SPC_LIB_PATH") or os.path.join(_HERE, "libspacap3d_ops.so")
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 _p = ctypes.c_void_p
 _i = ctypes.c_int
@@ -38,6 +38,14 @@ SIGNATURES = {
                                           ctypes.c_size_t, _p],
     "spc_bn_relu_maxpool_train_backward": [_p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p],
     "spc_bn_relu_train_backward": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, ctypes.c_size_t, _p],
+    "spc_bn_relu_sync_stats": [_p, _i, _i, _i, _p, _p, ctypes.c_size_t, _p],
+    "spc_bn_relu_sync_forward": [_p, _p, _p, _i, _i, _i, _i, _p, _f, _f, _p, _p, _p, _p, _p, _p],
+    "spc_bn_relu_sync_backward_reduce": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, ctypes.c_size_t, _p],
+    "spc_bn_relu_sync_backward": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, ctypes.c_size_t, _p],
+    "spc_bn_relu_maxpool_sync_forward": [_p, _p, _p, _i, _i, _i, _i, _i, _p, _f, _f, _p, _p, _p, _p, _p, _p, _p, _p],
+    "spc_bn_relu_maxpool_sync_backward_reduce": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p],
+    "spc_bn_relu_maxpool_sync_backward": [_p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _p,
+                                          ctypes.c_size_t, _p],
     "spc_group_points_grad_ex": [_p, _p, _i, _i, _i, _i, _i, _p, _p, ctypes.c_size_t, _p],
     "spc_three_nn": [_p, _p, _i, _i, _i, _p, _p, _p],
     "spc_three_interpolate": [_p, _p, _p, _i, _i, _i, _i, _p, _p],

@@ -340,6 +340,124 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
   }
 }
 
+// ----------------------------------------------------------------------------------------------------
+// Synchronised BatchNorm (torch.nn.SyncBatchNorm semantics) over the ranks of a process group.  The entry points
+// split each pass at its one cross-channel reduction: a rank writes its per-channel fp64 row of BN_SYNC_K values,
+//   forward : (n, mean, M2)                  n = B*S elements, M2 = sum (x - mean)^2,
+//   backward: (n, sum dm, sum dm * xhat),
+// the caller gathers the rows of all ranks into a (world, C, BN_SYNC_K) buffer, and the next entry point combines
+// them in rank order on the device, so every rank derives bit-identical statistics and nothing depends on the
+// collective's reduction order.  The global count comes from the rows, so ranks may hold different batch sizes.
+// The reduction and normalise/apply kernels are the ones above; only the per-channel finalisations are new.
+// ----------------------------------------------------------------------------------------------------
+constexpr int BN_SYNC_K = 3;
+
+// forward, local: (n, mean, M2) from the shifted partial sums s1 = sum (x-K), s2 = sum (x-K)^2 of bn_reduce_kernel<0>
+__global__ void bn_sync_moments_kernel(const float *__restrict__ y, const double *__restrict__ partial, int C, int S,
+                                       int splits, double M, double *__restrict__ row) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double s1 = 0.0, s2 = 0.0;
+  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+  const double K = (double)__ldg(y + (size_t)c * S);
+  const double m1 = s1 / M;
+  double m2 = s2 - s1 * m1;
+  if (m2 < 0.0) m2 = 0.0;
+  row[(size_t)c * BN_SYNC_K + 0] = M;
+  row[(size_t)c * BN_SYNC_K + 1] = K + m1;
+  row[(size_t)c * BN_SYNC_K + 2] = m2;
+}
+
+// forward, global: Chan's pairwise merge of the ranks' (n, mean, M2) in rank order, then what
+// bn_finalize_forward_kernel does with the merged moments.  Empty rows (n = 0) are skipped.
+__global__ void bn_sync_finalize_forward_kernel(const double *__restrict__ rows, int world, int C, float eps,
+                                                float momentum, float *__restrict__ running_mean,
+                                                float *__restrict__ running_var, float *__restrict__ save_mean,
+                                                float *__restrict__ save_invstd) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double n = 0.0, mean = 0.0, m2 = 0.0;
+  for (int r = 0; r < world; ++r) {
+    const double *q = rows + ((size_t)r * C + c) * BN_SYNC_K;
+    const double nb = q[0];
+    if (!(nb > 0.0)) continue;
+    const double nn = n + nb, d = q[1] - mean;
+    mean += d * (nb / nn);
+    m2 += q[2] + d * d * (n * nb / nn);
+    n = nn;
+  }
+  const double var = n > 0.0 ? m2 / n : 0.0;
+  save_mean[c] = (float)mean;
+  save_invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
+  if (running_mean) running_mean[c] = (float)((1.0 - momentum) * running_mean[c] + momentum * mean);
+  if (running_var) {
+    const double unbiased = n > 1.0 ? var * n / (n - 1.0) : var;
+    running_var[c] = (float)((1.0 - momentum) * running_var[c] + momentum * unbiased);
+  }
+}
+
+// backward, local: dgamma / dbeta of this rank (what bn_finalize_backward_kernel writes) and its row (n, s1, s2)
+__global__ void bn_sync_backward_local_kernel(const double *__restrict__ partial, int C, int splits, double M,
+                                              float *__restrict__ dgamma, float *__restrict__ dbeta,
+                                              double *__restrict__ row) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double s1 = 0.0, s2 = 0.0;
+  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+  dbeta[c] = (float)s1;
+  dgamma[c] = (float)s2;
+  row[(size_t)c * BN_SYNC_K + 0] = M;
+  row[(size_t)c * BN_SYNC_K + 1] = s1;
+  row[(size_t)c * BN_SYNC_K + 2] = s2;
+}
+
+// max-pool variant of the local backward reduction: bn_pool_bwd_reduce_kernel's loop, plus the row (a separate
+// kernel so that the existing one keeps its code)
+__global__ void __launch_bounds__(BN_THREADS) bn_pool_sync_bwd_reduce_kernel(
+    const float *__restrict__ dpool, const float *__restrict__ ymax, const float *__restrict__ gamma,
+    const float *__restrict__ beta, const float *__restrict__ mean, const float *__restrict__ invstd, int B, int C,
+    int np, double M, float *__restrict__ dgamma, float *__restrict__ dbeta, double *__restrict__ row) {
+  __shared__ double s_red[BN_THREADS / 32];
+  const int c = blockIdx.x;
+  const float mu = __ldg(mean + c), is = __ldg(invstd + c), g = __ldg(gamma + c), bt = __ldg(beta + c);
+  float a0 = 0.f, a1 = 0.f;
+  for (int b = 0; b < B; ++b) {
+    const size_t base = ((size_t)b * C + c) * np;
+    for (int j = threadIdx.x; j < np; j += BN_THREADS) {
+      const float xh = (__ldg(ymax + base + j) - mu) * is;
+      const float dm = fmaf(xh, g, bt) > 0.f ? __ldg(dpool + base + j) : 0.f;
+      a0 += dm;
+      a1 = fmaf(dm, xh, a1);
+    }
+  }
+  const double t0 = block_sum_double((double)a0, s_red);
+  const double t1 = block_sum_double((double)a1, s_red);
+  if (threadIdx.x == 0) {
+    dbeta[c] = (float)t0;
+    dgamma[c] = (float)t1;
+    row[(size_t)c * BN_SYNC_K + 0] = M;
+    row[(size_t)c * BN_SYNC_K + 1] = t0;
+    row[(size_t)c * BN_SYNC_K + 2] = t1;
+  }
+}
+
+// backward, global: k0 = sum dm / n and k1 = sum dm * xhat / n over all ranks, rounded once to fp32.  The apply
+// kernels read them in place of dbeta / dgamma with inv_M = 1, which leaves them unchanged.
+__global__ void bn_sync_combine_backward_kernel(const double *__restrict__ rows, int world, int C,
+                                                float *__restrict__ k0, float *__restrict__ k1) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double n = 0.0, s1 = 0.0, s2 = 0.0;
+  for (int r = 0; r < world; ++r) {
+    const double *q = rows + ((size_t)r * C + c) * BN_SYNC_K;
+    n += q[0];
+    s1 += q[1];
+    s2 += q[2];
+  }
+  k0[c] = n > 0.0 ? (float)(s1 / n) : 0.f;
+  k1[c] = n > 0.0 ? (float)(s2 / n) : 0.f;
+}
+
 }  // namespace spc
 
 using namespace spc;
@@ -452,5 +570,188 @@ extern "C" int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint
   if (nsample == 16) BP_BWD(16); else if (nsample == 32) BP_BWD(32); else BP_BWD(64);
 #undef BP_BWD
   SPC_LAUNCH_CHECK("bn_relu_maxpool_train_backward");
+  return SPC_OK;
+}
+
+// ---- synchronised BatchNorm (see BN_SYNC_K above) ----------------------------------------------------------------
+// The reductions take any B; the normalise / apply kernels put B*C rows on grid.y, so they are launched once per
+// slice of at most 65535 / C batch rows.  The synced path therefore accepts every local batch size a rank can get,
+// B = 0 included: a rank with an empty shard contributes a row with n = 0 (skipped by the combination) and still
+// takes part in every exchange, so the other ranks are not left waiting.  Its tensor pointers may then be NULL.
+static int sync_batch_slice(int C) { return max(1, 65535 / C); }
+
+#define SPC_SYNC_CHECK(what, B, C, world)                                                                         \
+  SPC_CHECK_ARG((B) >= 0 && (C) >= 1 && (C) <= 65535 && (world) >= 1, what ": bad sizes B=%d C=%d world=%d", B, C, \
+                world)
+
+extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, double *stats, void *workspace,
+                                      size_t workspace_bytes, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_sync_stats", B, C, 1);
+  SPC_CHECK_ARG(S >= 1 && (y || B == 0) && stats, "bn_relu_sync_stats: bad size or null pointer");
+  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
+                "bn_relu_sync_stats: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  if (B == 0) {                                   // (n, mean, M2) = 0: an empty shard
+    SPC_CUDA(cudaMemsetAsync(stats, 0, (size_t)C * BN_SYNC_K * sizeof(double), stream));
+    return SPC_OK;
+  }
+  double *partial = reinterpret_cast<double *>(workspace);
+  const BnPlan p = plan_bn(y, y, y, C, S);
+  dim3 rgrid(p.splits, C);
+  if (p.vec) bn_reduce_kernel<0, true><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, p.chunk, partial);
+  else bn_reduce_kernel<0, false><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, p.chunk, partial);
+  bn_sync_moments_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, stats);
+  SPC_LAUNCH_CHECK("bn_relu_sync_stats");
+  return SPC_OK;
+}
+
+extern "C" int spc_bn_relu_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
+                                        int world, const double *stats_all, float eps, float momentum,
+                                        float *running_mean, float *running_var, float *z, float *save_mean,
+                                        float *save_invstd, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_sync_forward", B, C, world);
+  SPC_CHECK_ARG(S >= 1 && ((y && z) || B == 0) && gamma && beta && stats_all && save_mean && save_invstd,
+                "bn_relu_sync_forward: bad size or null pointer");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
+                                                                        running_var, save_mean, save_invstd);
+  const BnPlan p = plan_bn(y, z, y, C, S);
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t off = (size_t)b0 * C * S;
+    dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
+    if (p.vec) bn_apply_kernel<0, true><<<agrid, BN_THREADS, 0, stream>>>(y + off, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z + off);
+    else bn_apply_kernel<0, false><<<agrid, BN_THREADS, 0, stream>>>(y + off, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z + off);
+  }
+  SPC_LAUNCH_CHECK("bn_relu_sync_forward");
+  return SPC_OK;
+}
+
+extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y, const float *gamma, const float *beta,
+                                                const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                                float *dgamma, float *dbeta, double *stats, void *workspace,
+                                                size_t workspace_bytes, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_sync_backward_reduce", B, C, 1);
+  SPC_CHECK_ARG(S >= 1 && ((dz && y) || B == 0) && gamma && beta && save_mean && save_invstd && dgamma && dbeta && stats,
+                "bn_relu_sync_backward_reduce: bad size or null pointer");
+  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
+                "bn_relu_sync_backward_reduce: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  if (B == 0) {                                   // empty shard: zero local sums and an n = 0 row
+    SPC_CUDA(cudaMemsetAsync(stats, 0, (size_t)C * BN_SYNC_K * sizeof(double), stream));
+    SPC_CUDA(cudaMemsetAsync(dgamma, 0, (size_t)C * sizeof(float), stream));
+    SPC_CUDA(cudaMemsetAsync(dbeta, 0, (size_t)C * sizeof(float), stream));
+    return SPC_OK;
+  }
+  double *partial = reinterpret_cast<double *>(workspace);
+  const BnPlan p = plan_bn(y, dz, dz, C, S);
+  dim3 rgrid(p.splits, C);
+  if (p.vec) bn_reduce_kernel<1, true><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
+  else bn_reduce_kernel<1, false><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
+  bn_sync_backward_local_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, (double)B * S, dgamma, dbeta, stats);
+  SPC_LAUNCH_CHECK("bn_relu_sync_backward_reduce");
+  return SPC_OK;
+}
+
+extern "C" int spc_bn_relu_sync_backward(const float *dz, const float *y, const float *gamma, const float *beta,
+                                         const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                         int world, const double *stats_all, float *dy, void *workspace,
+                                         size_t workspace_bytes, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_sync_backward", B, C, world);
+  SPC_CHECK_ARG(S >= 1 && ((dz && y && dy) || B == 0) && gamma && beta && save_mean && save_invstd && stats_all,
+                "bn_relu_sync_backward: bad size or null pointer");
+  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
+                "bn_relu_sync_backward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
+  bn_sync_combine_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, k0, k1);
+  const BnPlan p = plan_bn(y, dz, dy, C, S);
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t off = (size_t)b0 * C * S;
+    dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
+    if (p.vec) bn_apply_kernel<1, true><<<agrid, BN_THREADS, 0, stream>>>(y + off, dz + off, gamma, beta, save_mean, save_invstd, k1, k0, C, S, 1.f, dy + off);
+    else bn_apply_kernel<1, false><<<agrid, BN_THREADS, 0, stream>>>(y + off, dz + off, gamma, beta, save_mean, save_invstd, k1, k0, C, S, 1.f, dy + off);
+  }
+  SPC_LAUNCH_CHECK("bn_relu_sync_backward");
+  return SPC_OK;
+}
+
+// Max-pool variant.  Its statistics phase is spc_bn_relu_sync_stats with S = npoint * nsample.
+extern "C" int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C,
+                                                int npoint, int nsample, int world, const double *stats_all,
+                                                float eps, float momentum, float *running_mean, float *running_var,
+                                                float *pooled, uint8_t *argmax, float *ymax, float *save_mean,
+                                                float *save_invstd, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_maxpool_sync_forward", B, C, world);
+  SPC_CHECK_ARG(npoint >= 1 && (long long)npoint * nsample < (1LL << 31), "bn_relu_maxpool_sync_forward: bad sizes");
+  if (!pool_ns_supported(nsample) || (reinterpret_cast<uintptr_t>(y) & 15)) {
+    set_error("bn_relu_maxpool_sync: nsample=%d not in {16,32,64} or y not 16-byte aligned", nsample);
+    return SPC_ERR_UNSUPPORTED;
+  }
+  SPC_CHECK_ARG(((y && pooled && argmax && ymax) || B == 0) && gamma && beta && stats_all && save_mean && save_invstd,
+                "bn_relu_maxpool_sync_forward: null pointer");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
+                                                                        running_var, save_mean, save_invstd);
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
+#define BP_FWD(NS)                                                                                                  \
+  bn_relu_pool_fwd_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), min(slice, B - b0) * C), \
+                                BN_THREADS, 0, stream>>>(y + yo, gamma, beta, save_mean, save_invstd, C, npoint,     \
+                                                         pooled + po, argmax + po, ymax + po)
+    if (nsample == 16) BP_FWD(16); else if (nsample == 32) BP_FWD(32); else BP_FWD(64);
+#undef BP_FWD
+  }
+  SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_forward");
+  return SPC_OK;
+}
+
+extern "C" int spc_bn_relu_maxpool_sync_backward_reduce(const float *dpool, const float *ymax, const float *gamma,
+                                                        const float *beta, const float *save_mean,
+                                                        const float *save_invstd, int B, int C, int npoint,
+                                                        int nsample, float *dgamma, float *dbeta, double *stats,
+                                                        void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_maxpool_sync_backward_reduce", B, C, 1);
+  SPC_CHECK_ARG(npoint >= 1 && nsample >= 1, "bn_relu_maxpool_sync_backward_reduce: bad sizes");
+  SPC_CHECK_ARG(((dpool && ymax) || B == 0) && gamma && beta && save_mean && save_invstd && dgamma && dbeta && stats,
+                "bn_relu_maxpool_sync_backward_reduce: null pointer");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  bn_pool_sync_bwd_reduce_kernel<<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
+                                                               npoint, (double)B * npoint * nsample, dgamma, dbeta, stats);
+  SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward_reduce");
+  return SPC_OK;
+}
+
+extern "C" int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8_t *argmax, const float *ymax,
+                                                 const float *y, const float *gamma, const float *beta,
+                                                 const float *save_mean, const float *save_invstd, int B, int C,
+                                                 int npoint, int nsample, int world, const double *stats_all,
+                                                 float *dy, void *workspace, size_t workspace_bytes, void *stream_) {
+  SPC_SYNC_CHECK("bn_relu_maxpool_sync_backward", B, C, world);
+  SPC_CHECK_ARG(npoint >= 1 && (long long)npoint * nsample < (1LL << 31), "bn_relu_maxpool_sync_backward: bad sizes");
+  if (!pool_ns_supported(nsample) || ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
+    set_error("bn_relu_maxpool_sync: nsample=%d not in {16,32,64} or tensors not 16-byte aligned", nsample);
+    return SPC_ERR_UNSUPPORTED;
+  }
+  SPC_CHECK_ARG(((dpool && argmax && ymax && y && dy) || B == 0) && gamma && beta && save_mean && save_invstd && stats_all,
+                "bn_relu_maxpool_sync_backward: null pointer");
+  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
+                "bn_relu_maxpool_sync_backward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
+  bn_sync_combine_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, k0, k1);
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
+#define BP_BWD(NS)                                                                                                   \
+  bn_pool_bwd_apply_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), min(slice, B - b0) * C), \
+                                 BN_THREADS, 0, stream>>>(y + yo, dpool + po, argmax + po, ymax + po, gamma, beta,     \
+                                                          save_mean, save_invstd, k1, k0, C, npoint, 1.f, dy + yo)
+    if (nsample == 16) BP_BWD(16); else if (nsample == 32) BP_BWD(32); else BP_BWD(64);
+#undef BP_BWD
+  }
+  SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward");
   return SPC_OK;
 }

@@ -3,8 +3,12 @@
 Inference needs no collective.  Training needs exactly one gradient all-reduce per step: the
 reference does it implicitly through torch.nn.DataParallel (scripts/train.py:198-200); the
 one-process-per-GPU equivalent is a single flat bucket (0.95 M detector parameters = 3.8 MB, one
-latency-bound NCCL call over NVLink) -- `allreduce_gradients`.  BatchNorm statistics stay per rank,
-which is what DataParallel does as well.
+latency-bound NCCL call over NVLink) -- `allreduce_gradients`.  BatchNorm statistics stay per rank by
+default, which is what DataParallel does as well.  `nn.SyncBatchNorm.convert_sync_batchnorm(model)` makes every
+BatchNorm take its statistics over all ranks: the fused BatchNorm + ReLU blocks of the SA, FP and vote-aggregation
+MLPs then exchange one small fp64 buffer per block in the forward and one in the backward (pytorch_utils.py), the
+other BatchNorm layers run torch's SyncBatchNorm.  Their dgamma / dbeta stay per rank and are summed by the same
+gradient all-reduce.
 """
 import torch
 import torch.distributed as dist

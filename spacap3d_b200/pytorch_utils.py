@@ -7,12 +7,14 @@ a sequential block with `conv` (bias only when there is no BN), `bn` (itself a b
 child `bn`) and `activation`, so keys read `...layer0.conv.weight`, `...layer0.bn.bn.running_mean`.
 """
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 import torch.nn.functional as F
 
 # Training mode: run BatchNorm2d + ReLU of a conv block through the fused sm_100a kernels (csrc/bn_relu.cu)
 # instead of cuDNN batch-norm + a separate ReLU pass.  Same parameters, buffers and results (fp32, within
-# summation-order rounding); set to False to get the plain module sequence.
+# summation-order rounding); set to False to get the plain module sequence.  A BatchNorm converted to
+# nn.SyncBatchNorm runs the synced variants of the same kernels when torch's SyncBatchNorm would synchronise.
 FUSED_BN_RELU_TRAINING = True
 
 
@@ -57,6 +59,81 @@ class _BnReluMaxPoolTrain(torch.autograd.Function):
         dy, dgamma, dbeta = _ext.bn_relu_maxpool_train_backward(dpool.contiguous(), argmax, ymax, y, gamma, beta,
                                                                 mean, invstd)
         return dy, dgamma, dbeta, None, None, None, None
+
+
+def _exchange_rows(C, group, device):
+    """Zeroed (world, C, BN_SYNC_K) f64 buffer and this rank's row of it."""
+    from . import _ext
+    rows = torch.zeros((dist.get_world_size(group), C, _ext.BN_SYNC_K), dtype=torch.float64, device=device)
+    return rows, rows[dist.get_rank(group)]
+
+
+def _all_gather_rows(rows, group):
+    """Every rank filled only its own row of a zeroed buffer, so the SUM all-reduce is an exact all-gather (no
+    floating-point addition ever meets two non-zero terms); the rows are then combined in rank order on the device."""
+    dist.all_reduce(rows, op=dist.ReduceOp.SUM, group=group)
+    return rows
+
+
+class _BnReluSyncTrain(torch.autograd.Function):
+    """_BnReluTrain with the statistics of every rank of `group` (torch.nn.SyncBatchNorm semantics): one exchange of
+    (n, mean, M2) per channel in the forward and one of (n, sum dm, sum dm * xhat) in the backward."""
+
+    @staticmethod
+    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
+        from . import _ext
+        rows, mine = _exchange_rows(y.shape[1], group, y.device)
+        _ext.bn_relu_sync_stats(y, mine)
+        z, mean, invstd = _ext.bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps,
+                                                    _all_gather_rows(rows, group))
+        ctx.save_for_backward(y, gamma, beta, mean, invstd)
+        ctx.group = group
+        return z
+
+    @staticmethod
+    def backward(ctx, dz):
+        from . import _ext
+        y, gamma, beta, mean, invstd = ctx.saved_tensors
+        dz = dz.contiguous()
+        rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
+        dgamma, dbeta = _ext.bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, mine)
+        dy = _ext.bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, _all_gather_rows(rows, ctx.group))
+        return dy, dgamma, dbeta, None, None, None, None, None
+
+
+class _BnReluMaxPoolSyncTrain(torch.autograd.Function):
+    """_BnReluMaxPoolTrain with the statistics of every rank of `group`."""
+
+    @staticmethod
+    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
+        from . import _ext
+        rows, mine = _exchange_rows(y.shape[1], group, y.device)
+        _ext.bn_relu_sync_stats(y, mine)
+        pooled, argmax, ymax, mean, invstd = _ext.bn_relu_maxpool_sync_forward(
+            y, gamma, beta, running_mean, running_var, momentum, eps, _all_gather_rows(rows, group))
+        ctx.save_for_backward(y, gamma, beta, mean, invstd, argmax, ymax)
+        ctx.group = group
+        return pooled
+
+    @staticmethod
+    def backward(ctx, dpool):
+        from . import _ext
+        y, gamma, beta, mean, invstd, argmax, ymax = ctx.saved_tensors
+        dpool = dpool.contiguous()
+        rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
+        dgamma, dbeta = _ext.bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, mine)
+        dy = _ext.bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd,
+                                                _all_gather_rows(rows, ctx.group))
+        return dy, dgamma, dbeta, None, None, None, None, None
+
+
+def _sync_group(bn):
+    """The process group a training-mode nn.SyncBatchNorm synchronises over, or None when it would not (not a
+    SyncBatchNorm, torch.distributed not initialised, or a group of one rank): torch's own rule."""
+    if not (isinstance(bn, nn.SyncBatchNorm) and dist.is_available() and dist.is_initialized()):
+        return None
+    group = bn.process_group if bn.process_group is not None else dist.group.WORLD
+    return group if dist.get_world_size(group) > 1 else None
 
 
 _CONV = {1: nn.Conv1d, 2: nn.Conv2d, 3: nn.Conv3d}
@@ -139,12 +216,19 @@ class _ConvBase(nn.Sequential):
         if self._fused_training_ok(x):
             bn = getattr(self, self._bn_name)[0]
             y = run_conv(x)
-            if y.is_contiguous() and y.shape[0] * y.shape[1] <= 65535:
-                args = (y, bn.weight, bn.bias, bn.running_mean, bn.running_var, float(bn.momentum), float(bn.eps))
+            group = _sync_group(bn)
+            # SyncBatchNorm: the synced kernels take any local batch, so whether they run depends only on C, nsample
+            # and the module, never on this rank's share of the batch, and all ranks issue the same collectives
+            if group is not None or (y.is_contiguous() and y.shape[0] * y.shape[1] <= 65535):
+                args = (y.contiguous(), bn.weight, bn.bias, bn.running_mean, bn.running_var, float(bn.momentum),
+                        float(bn.eps))
+                plain, pool = _BnReluTrain, _BnReluMaxPoolTrain
+                if group is not None:
+                    args, plain, pool = args + (group,), _BnReluSyncTrain, _BnReluMaxPoolSyncTrain
                 if max_pool_last_dim and y.dim() == 4 and y.shape[3] in (16, 32, 64):
-                    out = _BnReluMaxPoolTrain.apply(*args)
+                    out = pool.apply(*args)
                 else:
-                    out = _BnReluTrain.apply(*args)
+                    out = plain.apply(*args)
                     if max_pool_last_dim:
                         out = _max_pool_last(out)
                 if bn.num_batches_tracked is not None:

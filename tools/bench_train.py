@@ -3,6 +3,7 @@
 
     python tools/bench_train.py [--points 40000,80000,120000,200000] [--scenes 4] [--iters 5] [--ref]
     python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/bench_train.py
+    python -m torch.distributed.run --nproc-per-node 8 tools/bench_train.py --points 40000 --sync-bn fused
 
 Training mode: autograd through the unfused sm_100a kernels (FPS, ball query, grouping, three_nn,
 interpolate and their backward passes) + cuDNN convolutions, exactly the reference's op sequence
@@ -10,10 +11,17 @@ interpolate and their backward passes) + cuDNN convolutions, exactly the referen
 reference's loss (lib/loss_helper.py) is outside the hot path.  SA npoint is scaled with the cloud
 (x1, x2, x3, x5 -> 2048..8192+, SURVEY 8d config 5).  `--ref` also times the reference's own CUDA
 extension (oracle/_ref) driving the same modules on rank 0.  One JSON line per cloud size.
+
+`--sync-bn` sets how BatchNorm statistics are taken across ranks: `off` (the default, per rank), `fused`
+(nn.SyncBatchNorm.convert_sync_batchnorm: the fused BatchNorm + ReLU kernels with one exchange in the forward and one
+in the backward of each block, torch's SyncBatchNorm for the voting and proposal heads) or `torch` (the converted
+model with the fused kernels switched off: torch's SyncBatchNorm everywhere).  Each line records the GPU's name and
+power limit.
 """
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -23,14 +31,28 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 
-def build_model(scale, device):
+def build_model(scale, device, sync_bn="off"):
     from spacap3d_b200.detector import VoteNetDetector
     torch.manual_seed(0)
     model = VoteNetDetector(input_feature_dim=1)
     bb = model.backbone_net
     for sa, base in ((bb.sa1, 2048), (bb.sa2, 1024), (bb.sa3, 512), (bb.sa4, 256)):
         sa.npoint = base * scale
+    if sync_bn != "off":
+        model = torch.nn.SyncBatchNorm.convert_sync_batchnorm(model)
     return model.to(device).train()
+
+
+def gpu_info(index):
+    """Name and power limit of the GPU the numbers were measured on."""
+    info = {"gpu": torch.cuda.get_device_name(index)}
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", str(index), "--query-gpu=power.limit", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        info["power_limit"] = out or None
+    except (OSError, subprocess.SubprocessError):
+        info["power_limit"] = None
+    return info
 
 
 def surrogate_loss(out):
@@ -69,6 +91,8 @@ def main():
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--ref", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--sync-bn", choices=("off", "fused", "torch"), default="off",
+                    help="BatchNorm statistics per rank (off) or across ranks with the fused kernels or torch's")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -76,7 +100,11 @@ def main():
     dev = torch.device("cuda", local)
     if world > 1:
         torch.distributed.init_process_group("nccl", device_id=dev)
+    from spacap3d_b200 import pytorch_utils
     from spacap3d_b200.dist import max_over_ranks
+    if args.sync_bn == "torch":
+        pytorch_utils.FUSED_BN_RELU_TRAINING = False
+    info = gpu_info(local)
     from spacap3d_b200.scenes import make_scene
     ref = None
     if args.ref and rank == 0:
@@ -84,7 +112,7 @@ def main():
         ref = load_ref()
     for n in [int(x) for x in args.points.split(",")]:
         scale = max(1, round(n / 40000))
-        model = build_model(scale, dev)
+        model = build_model(scale, dev, args.sync_bn)
         pc = torch.from_numpy(np.stack([make_scene(5000 + rank * 100 + i, n) for i in range(args.scenes)], 0)).to(dev)
 
         def ours():
@@ -94,7 +122,8 @@ def main():
         ms = time_steps(ours, args.iters)
         ms = max_over_ranks(ms, device=dev) if world > 1 else ms
         rec = {"config": "fwd+bwd, %d scenes/GPU x %d pts, SA npoint x%d" % (args.scenes, n, scale), "n_gpus": world,
-               "ms_per_step": round(ms, 3), "scenes_per_s": round(world * args.scenes / ms * 1e3, 2)}
+               "ms_per_step": round(ms, 3), "scenes_per_s": round(world * args.scenes / ms * 1e3, 2),
+               "sync_bn": args.sync_bn, **info}
         if world == 1 and not args.no_graph:
             # the step has no host synchronisation (box decode stays on the device), so forward + backward can be
             # captured once and replayed: removes the ~3 ms/step of Python/launch overhead of ~600 small launches
@@ -114,8 +143,6 @@ def main():
         if ref is not None:
             import bench
 
-            from spacap3d_b200 import pytorch_utils
-
             def theirs():      # reference extension + the plain cuDNN BatchNorm / ReLU / max_pool2d sequence
                 model.zero_grad(set_to_none=True)
                 pytorch_utils.FUSED_BN_RELU_TRAINING = False
@@ -123,7 +150,7 @@ def main():
                     with bench.swapped_ops(ref, host_decode=False):
                         step(model, pc, 1)
                 finally:
-                    pytorch_utils.FUSED_BN_RELU_TRAINING = True
+                    pytorch_utils.FUSED_BN_RELU_TRAINING = args.sync_bn != "torch"
 
             try:
                 rms = time_steps(theirs, max(2, args.iters // 2), warmup=1)
