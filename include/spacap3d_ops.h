@@ -241,7 +241,7 @@ int spc_pm_linear(const void *X_hi, const void *X_lo, int M, int K, const void *
  *             saved for backward;
  *   backward: dy, dgamma, dbeta from dz (gradient w.r.t. z), y and the saved statistics; the ReLU mask is
  *             recomputed from y.
- * workspace: spc_bn_relu_workspace_bytes(C) bytes, 8-byte aligned. */
+ * Any B >= 1 and 1 <= C <= 65535 (no B*C limit).  workspace: spc_bn_relu_workspace_bytes(C) bytes, 8-byte aligned. */
 size_t spc_bn_relu_workspace_bytes(int C);
 int spc_bn_relu_train_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
                               float eps, float momentum, float *running_mean, float *running_var, float *z,
@@ -257,7 +257,7 @@ int spc_bn_relu_train_backward(const float *dz, const float *y, const float *gam
  * y (B,C,npoint,nsample) -> pooled (B,C,npoint); the normalised activation is never materialised.
  * argmax (B,C,npoint) uint8 = winning slot (lowest slot on ties, like ATen), ymax = y at that slot; both
  * are consumed by the backward, which produces dy (B,C,npoint,nsample), dgamma, dbeta from dpool.
- * nsample must be 16, 32 or 64 (SPC_ERR_UNSUPPORTED otherwise: nothing launched). */
+ * nsample must be 16, 32 or 64 (SPC_ERR_UNSUPPORTED otherwise: nothing launched); any B >= 1 and 1 <= C <= 65535. */
 int spc_bn_relu_maxpool_train_forward(const float *y, const float *gamma, const float *beta, int B, int C,
                                       int npoint, int nsample, float eps, float momentum,
                                       float *running_mean, float *running_var, float *pooled,

@@ -428,6 +428,25 @@ def _bn_workspace(C, device):
     return torch.empty((nbytes + 7) // 8, dtype=torch.float64, device=device), nbytes
 
 
+def _bn_sizes(y):
+    """(B, C, S) of y (B,C,*); B may be 0 (a rank with an empty shard still takes part in the exchange)."""
+    return y.shape[0], y.shape[1], math.prod(y.shape[2:])
+
+
+def _per_channel(C, device):
+    """Two per-channel f32 outputs: (save_mean, save_invstd) or (dgamma, dbeta)."""
+    return (torch.empty(C, dtype=torch.float32, device=device), torch.empty(C, dtype=torch.float32, device=device))
+
+
+def _pool_outputs(y):
+    """(pooled, argmax, ymax, save_mean, save_invstd) of a max-pool forward of y (B,C,npoint,nsample)."""
+    B, C, npoint, _ = y.shape
+    pooled = torch.empty((B, C, npoint), dtype=torch.float32, device=y.device)
+    argmax = torch.empty((B, C, npoint), dtype=torch.uint8, device=y.device)
+    ymax = torch.empty((B, C, npoint), dtype=torch.float32, device=y.device)
+    return (pooled, argmax, ymax) + _per_channel(C, y.device)
+
+
 def bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, eps):
     """Training-mode BatchNorm + ReLU of y (B,C,*) f32 (pytorch_utils.py:11-36,39-64): returns
     (z, save_mean, save_invstd); running_mean / running_var (or None) are updated in place."""
@@ -435,11 +454,9 @@ def bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, e
     _check(gamma, "gamma", torch.float32)
     _check(beta, "beta", torch.float32)
     _same_device(y, gamma, beta)
-    B, C = y.shape[0], y.shape[1]
-    S = y.numel() // max(B * C, 1)
+    B, C, S = _bn_sizes(y)
     z = torch.empty_like(y)
-    mean = torch.empty(C, dtype=torch.float32, device=y.device)
-    invstd = torch.empty(C, dtype=torch.float32, device=y.device)
+    mean, invstd = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
         _lib.call("spc_bn_relu_train_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
@@ -455,11 +472,9 @@ def bn_relu_train_backward(dz, y, gamma, beta, mean, invstd):
     _check(dz, "dz", torch.float32)
     _check(y, "y", torch.float32)
     _same_device(dz, y)
-    B, C = y.shape[0], y.shape[1]
-    S = y.numel() // max(B * C, 1)
+    B, C, S = _bn_sizes(y)
     dy = torch.empty_like(y)
-    dgamma = torch.empty(C, dtype=torch.float32, device=y.device)
-    dbeta = torch.empty(C, dtype=torch.float32, device=y.device)
+    dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
         _lib.call("spc_bn_relu_train_backward", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
@@ -476,21 +491,15 @@ def bn_relu_maxpool_train_forward(y, gamma, beta, running_mean, running_var, mom
     _check(y, "y", torch.float32)
     _same_device(y, gamma, beta)
     B, C, npoint, nsample = y.shape
-    dev = y.device
-    pooled = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
-    argmax = torch.empty((B, C, npoint), dtype=torch.uint8, device=dev)
-    ymax = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
-    mean = torch.empty(C, dtype=torch.float32, device=dev)
-    invstd = torch.empty(C, dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        ws, nbytes = _bn_workspace(C, dev)
+    out = _pool_outputs(y)
+    with torch.cuda.device(y.device):
+        ws, nbytes = _bn_workspace(C, y.device)
         _lib.call("spc_bn_relu_maxpool_train_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
                   npoint, nsample, float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
-                  pooled.data_ptr(), argmax.data_ptr(), ymax.data_ptr(), mean.data_ptr(), invstd.data_ptr(),
-                  ws.data_ptr(), nbytes, _stream())
-    return pooled, argmax, ymax, mean, invstd
+                  *(t.data_ptr() for t in out), ws.data_ptr(), nbytes, _stream())
+    return out
 
 
 def bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd):
@@ -499,8 +508,7 @@ def bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, mean, in
     _same_device(dpool, y)
     B, C, npoint, nsample = y.shape
     dy = torch.empty_like(y)
-    dgamma = torch.empty(C, dtype=torch.float32, device=y.device)
-    dbeta = torch.empty(C, dtype=torch.float32, device=y.device)
+    dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         _lib.call("spc_bn_relu_maxpool_train_backward", dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
                   y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C,
@@ -516,11 +524,6 @@ def _check_rows(rows, C, what):
     _check(rows, what, torch.float64)
     if rows.dim() < 2 or tuple(rows.shape[-2:]) != (C, BN_SYNC_K):
         raise RuntimeError("%s must have shape (..., %d, %d)" % (what, C, BN_SYNC_K))
-
-
-def _bn_sizes(y):
-    """(B, C, S) of y (B,C,*); B may be 0 (a rank with an empty shard still takes part in the exchange)."""
-    return y.shape[0], y.shape[1], math.prod(y.shape[2:])
 
 
 def bn_relu_sync_stats(y, row):
@@ -546,8 +549,7 @@ def bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, ep
     _check_rows(rows, C, "rows")
     _same_device(y, gamma, beta, rows)
     z = torch.empty_like(y)
-    mean = torch.empty(C, dtype=torch.float32, device=y.device)
-    invstd = torch.empty(C, dtype=torch.float32, device=y.device)
+    mean, invstd = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         _lib.call("spc_bn_relu_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
                   rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
@@ -564,8 +566,7 @@ def bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, row):
     B, C, S = _bn_sizes(y)
     _check_rows(row, C, "row")
     _same_device(dz, y, row)
-    dgamma = torch.empty(C, dtype=torch.float32, device=y.device)
-    dbeta = torch.empty(C, dtype=torch.float32, device=y.device)
+    dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
         _lib.call("spc_bn_relu_sync_backward_reduce", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
@@ -599,19 +600,14 @@ def bn_relu_maxpool_sync_forward(y, gamma, beta, running_mean, running_var, mome
     B, C, npoint, nsample = y.shape
     _check_rows(rows, C, "rows")
     _same_device(y, gamma, beta, rows)
-    dev = y.device
-    pooled = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
-    argmax = torch.empty((B, C, npoint), dtype=torch.uint8, device=dev)
-    ymax = torch.empty((B, C, npoint), dtype=torch.float32, device=dev)
-    mean = torch.empty(C, dtype=torch.float32, device=dev)
-    invstd = torch.empty(C, dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
+    out = _pool_outputs(y)
+    with torch.cuda.device(y.device):
         _lib.call("spc_bn_relu_maxpool_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
                   npoint, nsample, rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
-                  pooled.data_ptr(), argmax.data_ptr(), ymax.data_ptr(), mean.data_ptr(), invstd.data_ptr(), _stream())
-    return pooled, argmax, ymax, mean, invstd
+                  *(t.data_ptr() for t in out), _stream())
+    return out
 
 
 def bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, row):
@@ -621,8 +617,7 @@ def bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invs
     _same_device(dpool, ymax, row)
     B, C, npoint, nsample = y.shape
     _check_rows(row, C, "row")
-    dgamma = torch.empty(C, dtype=torch.float32, device=dpool.device)
-    dbeta = torch.empty(C, dtype=torch.float32, device=dpool.device)
+    dgamma, dbeta = _per_channel(C, dpool.device)
     with torch.cuda.device(dpool.device):
         _lib.call("spc_bn_relu_maxpool_sync_backward_reduce", dpool.data_ptr(), ymax.data_ptr(), gamma.data_ptr(),
                   beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C, npoint, nsample, dgamma.data_ptr(),

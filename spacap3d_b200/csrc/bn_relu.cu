@@ -15,6 +15,9 @@
 // Semantics = torch.nn.functional.batch_norm(training=True) + relu: biased variance for normalisation,
 // running_mean/var updated with `momentum` and the unbiased variance, save_mean / save_invstd for backward,
 // gradient of ReLU taken where the OUTPUT is > 0.
+#include <initializer_list>
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace spc {
@@ -22,6 +25,7 @@ namespace spc {
 constexpr int BN_THREADS = 256;
 constexpr int BN_MAX_SPLITS = 64;
 constexpr int BN_UNR = 4;
+constexpr int BN_SYNC_K = 3;      // fp64 values per channel in a rank's synced-BatchNorm row (see below)
 
 __device__ __forceinline__ double block_sum_double(double v, double *s_red) {
 #pragma unroll
@@ -104,14 +108,22 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float *__re
   }
 }
 
+// channel c's two sums over the splits of bn_reduce_kernel, in split order
+__device__ __forceinline__ void sum_partials(const double *__restrict__ partial, int c, int splits, double &s1,
+                                             double &s2) {
+  s1 = 0.0;
+  s2 = 0.0;
+  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+}
+
 __global__ void bn_finalize_forward_kernel(const float *__restrict__ y, const double *__restrict__ partial, int C, int S,
                                            int splits, double M, float eps, float momentum,
                                            float *__restrict__ running_mean, float *__restrict__ running_var,
                                            float *__restrict__ save_mean, float *__restrict__ save_invstd) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  double s1 = 0.0, s2 = 0.0;
-  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+  double s1, s2;
+  sum_partials(partial, c, splits, s1, s2);
   const double K = (double)__ldg(y + (size_t)c * S);
   const double m1 = s1 / M;
   const double mean = K + m1;
@@ -126,14 +138,22 @@ __global__ void bn_finalize_forward_kernel(const float *__restrict__ y, const do
   }
 }
 
+// dgamma / dbeta; ROW (synced backward) also writes this rank's row (n, sum dm, sum dm * xhat) with n = M
+template <bool ROW>
 __global__ void bn_finalize_backward_kernel(const double *__restrict__ partial, int C, int splits,
-                                            float *__restrict__ dgamma, float *__restrict__ dbeta) {
+                                            float *__restrict__ dgamma, float *__restrict__ dbeta, double M,
+                                            double *__restrict__ row) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  double s1 = 0.0, s2 = 0.0;
-  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+  double s1, s2;
+  sum_partials(partial, c, splits, s1, s2);
   dbeta[c] = (float)s1;
   dgamma[c] = (float)s2;
+  if (ROW) {
+    row[(size_t)c * BN_SYNC_K + 0] = M;
+    row[(size_t)c * BN_SYNC_K + 1] = s1;
+    row[(size_t)c * BN_SYNC_K + 2] = s2;
+  }
 }
 
 // grid (position tiles, B*C).  MODE 0: z = relu(bn(y)).  MODE 1: dy from dz, y and the channel sums.
@@ -266,15 +286,13 @@ __global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const floa
   }
 }
 
-// one CTA per channel: dbeta = sum dm, dgamma = sum dm * xhat over the (B, npoint) winners
-__global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(const float *__restrict__ dpool,
-                                                                         const float *__restrict__ ymax,
-                                                                         const float *__restrict__ gamma,
-                                                                         const float *__restrict__ beta,
-                                                                         const float *__restrict__ mean,
-                                                                         const float *__restrict__ invstd, int B, int C,
-                                                                         int np, float *__restrict__ dgamma,
-                                                                         float *__restrict__ dbeta) {
+// one CTA per channel: dbeta = sum dm, dgamma = sum dm * xhat over the (B, npoint) winners; ROW as in
+// bn_finalize_backward_kernel
+template <bool ROW>
+__global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(
+    const float *__restrict__ dpool, const float *__restrict__ ymax, const float *__restrict__ gamma,
+    const float *__restrict__ beta, const float *__restrict__ mean, const float *__restrict__ invstd, int B, int C,
+    int np, float *__restrict__ dgamma, float *__restrict__ dbeta, double M, double *__restrict__ row) {
   __shared__ double s_red[BN_THREADS / 32];
   const int c = blockIdx.x;
   const float mu = __ldg(mean + c), is = __ldg(invstd + c), g = __ldg(gamma + c), bt = __ldg(beta + c);
@@ -290,7 +308,15 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(const fl
   }
   const double t0 = block_sum_double((double)a0, s_red);
   const double t1 = block_sum_double((double)a1, s_red);
-  if (threadIdx.x == 0) { dbeta[c] = (float)t0; dgamma[c] = (float)t1; }
+  if (threadIdx.x == 0) {
+    dbeta[c] = (float)t0;
+    dgamma[c] = (float)t1;
+    if (ROW) {
+      row[(size_t)c * BN_SYNC_K + 0] = M;
+      row[(size_t)c * BN_SYNC_K + 1] = t0;
+      row[(size_t)c * BN_SYNC_K + 2] = t1;
+    }
+  }
 }
 
 template <int NS>
@@ -348,17 +374,20 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
 // the caller gathers the rows of all ranks into a (world, C, BN_SYNC_K) buffer, and the next entry point combines
 // them in rank order on the device, so every rank derives bit-identical statistics and nothing depends on the
 // collective's reduction order.  The global count comes from the rows, so ranks may hold different batch sizes.
-// The reduction and normalise/apply kernels are the ones above; only the per-channel finalisations are new.
+// The reduction, normalise, pool and apply kernels are the ones above; the backward reductions write the row when
+// ROW.  The finalisations below are kept apart from the plain ones on purpose: the plain variance s2/M - m1^2 and
+// the merged M2 = s2 - s1*m1 can round differently, and so can the plain fp32(sum dm) * fp32(1/M) and the synced
+// fp32(sum dm / n), so running the plain pass as a synced one of one rank would change its results (and add two
+// launches per pass).
 // ----------------------------------------------------------------------------------------------------
-constexpr int BN_SYNC_K = 3;
 
 // forward, local: (n, mean, M2) from the shifted partial sums s1 = sum (x-K), s2 = sum (x-K)^2 of bn_reduce_kernel<0>
 __global__ void bn_sync_moments_kernel(const float *__restrict__ y, const double *__restrict__ partial, int C, int S,
                                        int splits, double M, double *__restrict__ row) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  double s1 = 0.0, s2 = 0.0;
-  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
+  double s1, s2;
+  sum_partials(partial, c, splits, s1, s2);
   const double K = (double)__ldg(y + (size_t)c * S);
   const double m1 = s1 / M;
   double m2 = s2 - s1 * m1;
@@ -396,51 +425,6 @@ __global__ void bn_sync_finalize_forward_kernel(const double *__restrict__ rows,
   }
 }
 
-// backward, local: dgamma / dbeta of this rank (what bn_finalize_backward_kernel writes) and its row (n, s1, s2)
-__global__ void bn_sync_backward_local_kernel(const double *__restrict__ partial, int C, int splits, double M,
-                                              float *__restrict__ dgamma, float *__restrict__ dbeta,
-                                              double *__restrict__ row) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= C) return;
-  double s1 = 0.0, s2 = 0.0;
-  for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
-  dbeta[c] = (float)s1;
-  dgamma[c] = (float)s2;
-  row[(size_t)c * BN_SYNC_K + 0] = M;
-  row[(size_t)c * BN_SYNC_K + 1] = s1;
-  row[(size_t)c * BN_SYNC_K + 2] = s2;
-}
-
-// max-pool variant of the local backward reduction: bn_pool_bwd_reduce_kernel's loop, plus the row (a separate
-// kernel so that the existing one keeps its code)
-__global__ void __launch_bounds__(BN_THREADS) bn_pool_sync_bwd_reduce_kernel(
-    const float *__restrict__ dpool, const float *__restrict__ ymax, const float *__restrict__ gamma,
-    const float *__restrict__ beta, const float *__restrict__ mean, const float *__restrict__ invstd, int B, int C,
-    int np, double M, float *__restrict__ dgamma, float *__restrict__ dbeta, double *__restrict__ row) {
-  __shared__ double s_red[BN_THREADS / 32];
-  const int c = blockIdx.x;
-  const float mu = __ldg(mean + c), is = __ldg(invstd + c), g = __ldg(gamma + c), bt = __ldg(beta + c);
-  float a0 = 0.f, a1 = 0.f;
-  for (int b = 0; b < B; ++b) {
-    const size_t base = ((size_t)b * C + c) * np;
-    for (int j = threadIdx.x; j < np; j += BN_THREADS) {
-      const float xh = (__ldg(ymax + base + j) - mu) * is;
-      const float dm = fmaf(xh, g, bt) > 0.f ? __ldg(dpool + base + j) : 0.f;
-      a0 += dm;
-      a1 = fmaf(dm, xh, a1);
-    }
-  }
-  const double t0 = block_sum_double((double)a0, s_red);
-  const double t1 = block_sum_double((double)a1, s_red);
-  if (threadIdx.x == 0) {
-    dbeta[c] = (float)t0;
-    dgamma[c] = (float)t1;
-    row[(size_t)c * BN_SYNC_K + 0] = M;
-    row[(size_t)c * BN_SYNC_K + 1] = t0;
-    row[(size_t)c * BN_SYNC_K + 2] = t1;
-  }
-}
-
 // backward, global: k0 = sum dm / n and k1 = sum dm * xhat / n over all ranks, rounded once to fp32.  The apply
 // kernels read them in place of dbeta / dgamma with inv_M = 1, which leaves them unchanged.
 __global__ void bn_sync_combine_backward_kernel(const double *__restrict__ rows, int world, int C,
@@ -466,26 +450,122 @@ extern "C" size_t spc_bn_relu_workspace_bytes(int C) {
   return C > 0 ? (size_t)C * BN_MAX_SPLITS * 2 * sizeof(double) : 0;
 }
 
+// ---- checks and launchers shared by the plain and the synced entry points ----------------------------------------
+// Sizes and pointers of a pass over y (B, C, np * ns); the passes without max-pool give ns = 1.  The plain passes need
+// B >= 1; the synced ones take B = 0 (min_B = 0): a rank with an empty shard still takes part in every exchange, so
+// the other ranks are not left waiting, and its per-sample tensors may then be NULL.  Per-channel tensors never.
+static int check_bn(const char *what, int B, int min_B, int C, int np, int ns, int world,
+                    std::initializer_list<const void *> samples, std::initializer_list<const void *> channels) {
+  SPC_CHECK_ARG(B >= min_B && C >= 1 && C <= 65535 && np >= 1 && ns >= 1 && (long long)np * ns < (1LL << 31) && world >= 1,
+                "%s: bad sizes B=%d C=%d S=%d*%d world=%d", what, B, C, np, ns, world);
+  bool ok = true;
+  for (const void *q : channels) ok = ok && q;
+  if (B > 0) for (const void *q : samples) ok = ok && q;
+  SPC_CHECK_ARG(ok, "%s: null pointer", what);
+  return SPC_OK;
+}
+
+static int check_workspace(const char *what, const void *workspace, size_t workspace_bytes, int C) {
+  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
+                "%s: workspace of spc_bn_relu_workspace_bytes(C) bytes required", what);
+  return SPC_OK;
+}
+
+// the pool kernels exist for nsample 16, 32 and 64, and read y and write dy with 16-byte accesses
+static int check_pool(const char *what, int nsample, const void *y, const void *dy) {
+  if (!(nsample == 16 || nsample == 32 || nsample == 64) ||
+      ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
+    set_error("%s: nsample=%d not in {16,32,64} or tensors not 16-byte aligned", what, nsample);
+    return SPC_ERR_UNSUPPORTED;
+  }
+  return SPC_OK;
+}
+
+// The reductions take any B.  The normalise / apply / pool kernels put B*C rows on grid.y, so they are launched once
+// per slice of at most 65535 / C batch rows: one launch whenever B*C <= 65535.
+static int sync_batch_slice(int C) { return max(1, 65535 / C); }
+
+template <int MODE>
+static void launch_reduce(const BnPlan &p, const float *y, const float *dz, const float *gamma, const float *beta,
+                          const float *mean, const float *invstd, int B, int C, int S, double *partial,
+                          cudaStream_t stream) {
+  const dim3 grid(p.splits, C);
+  if (p.vec) bn_reduce_kernel<MODE, true><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
+  else bn_reduce_kernel<MODE, false><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
+}
+
+// MODE 0: out = z (dz, dgamma, dbeta unused).  MODE 1: out = dy with k0 = dbeta * inv_M, k1 = dgamma * inv_M.
+template <int MODE>
+static void launch_apply(bool vec, const float *y, const float *dz, const float *gamma, const float *beta,
+                         const float *mean, const float *invstd, const float *dgamma, const float *dbeta, int B, int C,
+                         int S, float inv_M, float *out, cudaStream_t stream) {
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t off = (size_t)b0 * C * S;
+    const float *dzs = MODE == 1 ? dz + off : nullptr;
+    const dim3 grid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
+    if (vec) bn_apply_kernel<MODE, true><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
+    else bn_apply_kernel<MODE, false><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
+  }
+}
+
+// calls launch(std::integral_constant<int, NS>) for the nsample check_pool accepted
+template <class F>
+static void dispatch_nsample(int nsample, F &&launch) {
+  if (nsample == 16) launch(std::integral_constant<int, 16>());
+  else if (nsample == 32) launch(std::integral_constant<int, 32>());
+  else launch(std::integral_constant<int, 64>());
+}
+
+// grid.x of the pool kernels: BN_THREADS / 32 warps, each over 32 / (nsample / 4) groups BP_UNR times
+static int pool_tiles(int npoint, int nsample) {
+  return ceil_div(npoint, (BN_THREADS / 32) * (32 / (nsample / 4)) * BP_UNR);
+}
+
+static void launch_pool_fwd(const float *y, const float *gamma, const float *beta, const float *mean,
+                            const float *invstd, int B, int C, int npoint, int nsample, float *pooled, uint8_t *argmax,
+                            float *ymax, cudaStream_t stream) {
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
+    const dim3 grid(pool_tiles(npoint, nsample), min(slice, B - b0) * C);
+    dispatch_nsample(nsample, [&](auto ns) {
+      bn_relu_pool_fwd_kernel<decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
+          y + yo, gamma, beta, mean, invstd, C, npoint, pooled + po, argmax + po, ymax + po);
+    });
+  }
+}
+
+// dy from dpool, with k0 = dbeta * inv_M, k1 = dgamma * inv_M
+static void launch_pool_bwd(const float *y, const float *dpool, const uint8_t *argmax, const float *ymax,
+                            const float *gamma, const float *beta, const float *mean, const float *invstd,
+                            const float *dgamma, const float *dbeta, int B, int C, int npoint, int nsample, float inv_M,
+                            float *dy, cudaStream_t stream) {
+  const int slice = sync_batch_slice(C);
+  for (int b0 = 0; b0 < B; b0 += slice) {
+    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
+    const dim3 grid(pool_tiles(npoint, nsample), min(slice, B - b0) * C);
+    dispatch_nsample(nsample, [&](auto ns) {
+      bn_pool_bwd_apply_kernel<decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
+          y + yo, dpool + po, argmax + po, ymax + po, gamma, beta, mean, invstd, dgamma, dbeta, C, npoint, inv_M, dy + yo);
+    });
+  }
+}
+
+// ---- plain passes -------------------------------------------------------------------------------------------------
 extern "C" int spc_bn_relu_train_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
                                          float eps, float momentum, float *running_mean, float *running_var,
                                          float *z, float *save_mean, float *save_invstd, void *workspace,
                                          size_t workspace_bytes, void *stream_) {
-  SPC_CHECK_ARG(B >= 1 && C >= 1 && S >= 1, "bn_relu_forward: bad sizes B=%d C=%d S=%d", B, C, S);
-  SPC_CHECK_ARG(y && gamma && beta && z && save_mean && save_invstd, "bn_relu_forward: null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_forward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
-  SPC_CHECK_ARG((long long)B * C <= 65535 && C <= 65535, "bn_relu_forward: B*C too large");
+  if (const int e = check_bn("bn_relu_forward", B, 1, C, S, 1, 1, {y, z}, {gamma, beta, save_mean, save_invstd})) return e;
+  if (const int e = check_workspace("bn_relu_forward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   double *partial = reinterpret_cast<double *>(workspace);
   const BnPlan p = plan_bn(y, z, y, C, S);
-  dim3 rgrid(p.splits, C);
-  if (p.vec) bn_reduce_kernel<0, true><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, p.chunk, partial);
-  else bn_reduce_kernel<0, false><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, p.chunk, partial);
+  launch_reduce<0>(p, y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
   bn_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, eps, momentum,
                                                                    running_mean, running_var, save_mean, save_invstd);
-  dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), B * C);
-  if (p.vec) bn_apply_kernel<0, true><<<agrid, BN_THREADS, 0, stream>>>(y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z);
-  else bn_apply_kernel<0, false><<<agrid, BN_THREADS, 0, stream>>>(y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z);
+  launch_apply<0>(p.vec, y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
   SPC_LAUNCH_CHECK("bn_relu_train_forward");
   return SPC_OK;
 }
@@ -494,55 +574,37 @@ extern "C" int spc_bn_relu_train_backward(const float *dz, const float *y, const
                                           const float *save_mean, const float *save_invstd, int B, int C, int S,
                                           float *dy, float *dgamma, float *dbeta, void *workspace,
                                           size_t workspace_bytes, void *stream_) {
-  SPC_CHECK_ARG(B >= 1 && C >= 1 && S >= 1, "bn_relu_backward: bad sizes B=%d C=%d S=%d", B, C, S);
-  SPC_CHECK_ARG(dz && y && gamma && beta && save_mean && save_invstd && dy && dgamma && dbeta, "bn_relu_backward: null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_backward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
-  SPC_CHECK_ARG((long long)B * C <= 65535 && C <= 65535, "bn_relu_backward: B*C too large");
+  if (const int e = check_bn("bn_relu_backward", B, 1, C, S, 1, 1, {dz, y, dy},
+                             {gamma, beta, save_mean, save_invstd, dgamma, dbeta})) return e;
+  if (const int e = check_workspace("bn_relu_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   double *partial = reinterpret_cast<double *>(workspace);
   const BnPlan p = plan_bn(y, dz, dy, C, S);
-  dim3 rgrid(p.splits, C);
-  if (p.vec) bn_reduce_kernel<1, true><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
-  else bn_reduce_kernel<1, false><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
-  bn_finalize_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, dgamma, dbeta);
-  dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), B * C);
+  launch_reduce<1>(p, y, dz, gamma, beta, save_mean, save_invstd, B, C, S, partial, stream);
+  bn_finalize_backward_kernel<false><<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, dgamma, dbeta, 0.0, nullptr);
   const float inv_M = (float)(1.0 / ((double)B * S));
-  if (p.vec) bn_apply_kernel<1, true><<<agrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, dgamma, dbeta, C, S, inv_M, dy);
-  else bn_apply_kernel<1, false><<<agrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, dgamma, dbeta, C, S, inv_M, dy);
+  launch_apply<1>(p.vec, y, dz, gamma, beta, save_mean, save_invstd, dgamma, dbeta, B, C, S, inv_M, dy, stream);
   SPC_LAUNCH_CHECK("bn_relu_train_backward");
   return SPC_OK;
 }
-
-// ---- BatchNorm + ReLU + max over nsample (last block of a set-abstraction MLP) ---------------------------
-static bool pool_ns_supported(int ns) { return ns == 16 || ns == 32 || ns == 64; }
 
 extern "C" int spc_bn_relu_maxpool_train_forward(const float *y, const float *gamma, const float *beta, int B, int C,
                                                  int npoint, int nsample, float eps, float momentum,
                                                  float *running_mean, float *running_var, float *pooled,
                                                  uint8_t *argmax, float *ymax, float *save_mean, float *save_invstd,
                                                  void *workspace, size_t workspace_bytes, void *stream_) {
-  SPC_CHECK_ARG(B >= 1 && C >= 1 && npoint >= 1 && nsample >= 1, "bn_relu_maxpool_forward: bad sizes");
-  if (!pool_ns_supported(nsample) || (reinterpret_cast<uintptr_t>(y) & 15)) {
-    set_error("bn_relu_maxpool: nsample=%d not in {16,32,64} or y not 16-byte aligned", nsample);
-    return SPC_ERR_UNSUPPORTED;
-  }
-  SPC_CHECK_ARG(y && gamma && beta && pooled && argmax && ymax && save_mean && save_invstd, "bn_relu_maxpool_forward: null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_maxpool_forward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
-  SPC_CHECK_ARG((long long)B * C <= 65535 && (long long)npoint * nsample < (1LL << 31), "bn_relu_maxpool_forward: too large");
+  if (const int e = check_bn("bn_relu_maxpool_forward", B, 1, C, npoint, nsample, 1, {y, pooled, argmax, ymax},
+                             {gamma, beta, save_mean, save_invstd})) return e;
+  if (const int e = check_pool("bn_relu_maxpool_forward", nsample, y, nullptr)) return e;
+  if (const int e = check_workspace("bn_relu_maxpool_forward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   const int S = npoint * nsample;
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, y, y, C, S);
-  bn_reduce_kernel<0, true><<<dim3(p.splits, C), BN_THREADS, 0, stream>>>(y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, p.chunk, partial);
+  const BnPlan p = plan_bn(y, y, y, C, S);     // vector: y is 16-byte aligned and S a multiple of 16
+  launch_reduce<0>(p, y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
   bn_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, eps, momentum,
                                                                    running_mean, running_var, save_mean, save_invstd);
-#define BP_FWD(NS)                                                                                          \
-  bn_relu_pool_fwd_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), B * C), \
-                                BN_THREADS, 0, stream>>>(y, gamma, beta, save_mean, save_invstd, C, npoint, pooled, argmax, ymax)
-  if (nsample == 16) BP_FWD(16); else if (nsample == 32) BP_FWD(32); else BP_FWD(64);
-#undef BP_FWD
+  launch_pool_fwd(y, gamma, beta, save_mean, save_invstd, B, C, npoint, nsample, pooled, argmax, ymax, stream);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_train_forward");
   return SPC_OK;
 }
@@ -552,44 +614,25 @@ extern "C" int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint
                                                   const float *save_mean, const float *save_invstd, int B, int C,
                                                   int npoint, int nsample, float *dy, float *dgamma, float *dbeta,
                                                   void *stream_) {
-  SPC_CHECK_ARG(B >= 1 && C >= 1 && npoint >= 1 && nsample >= 1, "bn_relu_maxpool_backward: bad sizes");
-  if (!pool_ns_supported(nsample) || ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
-    set_error("bn_relu_maxpool: nsample=%d not in {16,32,64} or tensors not 16-byte aligned", nsample);
-    return SPC_ERR_UNSUPPORTED;
-  }
-  SPC_CHECK_ARG(dpool && argmax && ymax && y && gamma && beta && save_mean && save_invstd && dy && dgamma && dbeta,
-                "bn_relu_maxpool_backward: null pointer");
-  SPC_CHECK_ARG((long long)B * C <= 65535 && C <= 65535, "bn_relu_maxpool_backward: too large");
+  if (const int e = check_bn("bn_relu_maxpool_backward", B, 1, C, npoint, nsample, 1, {dpool, argmax, ymax, y, dy},
+                             {gamma, beta, save_mean, save_invstd, dgamma, dbeta})) return e;
+  if (const int e = check_pool("bn_relu_maxpool_backward", nsample, y, dy)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
-  bn_pool_bwd_reduce_kernel<<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C, npoint, dgamma, dbeta);
+  bn_pool_bwd_reduce_kernel<false><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
+                                                                 npoint, dgamma, dbeta, 0.0, nullptr);
   const float inv_M = (float)(1.0 / ((double)B * npoint * nsample));
-#define BP_BWD(NS)                                                                                            \
-  bn_pool_bwd_apply_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), B * C),  \
-                                 BN_THREADS, 0, stream>>>(y, dpool, argmax, ymax, gamma, beta, save_mean, save_invstd, \
-                                                          dgamma, dbeta, C, npoint, inv_M, dy)
-  if (nsample == 16) BP_BWD(16); else if (nsample == 32) BP_BWD(32); else BP_BWD(64);
-#undef BP_BWD
+  launch_pool_bwd(y, dpool, argmax, ymax, gamma, beta, save_mean, save_invstd, dgamma, dbeta, B, C, npoint, nsample,
+                  inv_M, dy, stream);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_train_backward");
   return SPC_OK;
 }
 
-// ---- synchronised BatchNorm (see BN_SYNC_K above) ----------------------------------------------------------------
-// The reductions take any B; the normalise / apply kernels put B*C rows on grid.y, so they are launched once per
-// slice of at most 65535 / C batch rows.  The synced path therefore accepts every local batch size a rank can get,
-// B = 0 included: a rank with an empty shard contributes a row with n = 0 (skipped by the combination) and still
-// takes part in every exchange, so the other ranks are not left waiting.  Its tensor pointers may then be NULL.
-static int sync_batch_slice(int C) { return max(1, 65535 / C); }
-
-#define SPC_SYNC_CHECK(what, B, C, world)                                                                         \
-  SPC_CHECK_ARG((B) >= 0 && (C) >= 1 && (C) <= 65535 && (world) >= 1, what ": bad sizes B=%d C=%d world=%d", B, C, \
-                world)
-
+// ---- synchronised passes (see BN_SYNC_K above) --------------------------------------------------------------------
+// Each takes any local B >= 0; a rank with B = 0 contributes a row with n = 0, which the combinations skip.
 extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, double *stats, void *workspace,
                                       size_t workspace_bytes, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_sync_stats", B, C, 1);
-  SPC_CHECK_ARG(S >= 1 && (y || B == 0) && stats, "bn_relu_sync_stats: bad size or null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_sync_stats: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  if (const int e = check_bn("bn_relu_sync_stats", B, 0, C, S, 1, 1, {y}, {stats})) return e;
+  if (const int e = check_workspace("bn_relu_sync_stats", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   if (B == 0) {                                   // (n, mean, M2) = 0: an empty shard
     SPC_CUDA(cudaMemsetAsync(stats, 0, (size_t)C * BN_SYNC_K * sizeof(double), stream));
@@ -597,9 +640,7 @@ extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, doubl
   }
   double *partial = reinterpret_cast<double *>(workspace);
   const BnPlan p = plan_bn(y, y, y, C, S);
-  dim3 rgrid(p.splits, C);
-  if (p.vec) bn_reduce_kernel<0, true><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, p.chunk, partial);
-  else bn_reduce_kernel<0, false><<<rgrid, BN_THREADS, 0, stream>>>(y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, p.chunk, partial);
+  launch_reduce<0>(p, y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, partial, stream);
   bn_sync_moments_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, stats);
   SPC_LAUNCH_CHECK("bn_relu_sync_stats");
   return SPC_OK;
@@ -609,20 +650,13 @@ extern "C" int spc_bn_relu_sync_forward(const float *y, const float *gamma, cons
                                         int world, const double *stats_all, float eps, float momentum,
                                         float *running_mean, float *running_var, float *z, float *save_mean,
                                         float *save_invstd, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_sync_forward", B, C, world);
-  SPC_CHECK_ARG(S >= 1 && ((y && z) || B == 0) && gamma && beta && stats_all && save_mean && save_invstd,
-                "bn_relu_sync_forward: bad size or null pointer");
+  if (const int e = check_bn("bn_relu_sync_forward", B, 0, C, S, 1, world, {y, z},
+                             {gamma, beta, stats_all, save_mean, save_invstd})) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
                                                                         running_var, save_mean, save_invstd);
   const BnPlan p = plan_bn(y, z, y, C, S);
-  const int slice = sync_batch_slice(C);
-  for (int b0 = 0; b0 < B; b0 += slice) {
-    const size_t off = (size_t)b0 * C * S;
-    dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
-    if (p.vec) bn_apply_kernel<0, true><<<agrid, BN_THREADS, 0, stream>>>(y + off, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z + off);
-    else bn_apply_kernel<0, false><<<agrid, BN_THREADS, 0, stream>>>(y + off, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, C, S, 0.f, z + off);
-  }
+  launch_apply<0>(p.vec, y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
   SPC_LAUNCH_CHECK("bn_relu_sync_forward");
   return SPC_OK;
 }
@@ -631,11 +665,9 @@ extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y,
                                                 const float *save_mean, const float *save_invstd, int B, int C, int S,
                                                 float *dgamma, float *dbeta, double *stats, void *workspace,
                                                 size_t workspace_bytes, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_sync_backward_reduce", B, C, 1);
-  SPC_CHECK_ARG(S >= 1 && ((dz && y) || B == 0) && gamma && beta && save_mean && save_invstd && dgamma && dbeta && stats,
-                "bn_relu_sync_backward_reduce: bad size or null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_sync_backward_reduce: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  if (const int e = check_bn("bn_relu_sync_backward_reduce", B, 0, C, S, 1, 1, {dz, y},
+                             {gamma, beta, save_mean, save_invstd, dgamma, dbeta, stats})) return e;
+  if (const int e = check_workspace("bn_relu_sync_backward_reduce", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   if (B == 0) {                                   // empty shard: zero local sums and an n = 0 row
     SPC_CUDA(cudaMemsetAsync(stats, 0, (size_t)C * BN_SYNC_K * sizeof(double), stream));
@@ -645,10 +677,9 @@ extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y,
   }
   double *partial = reinterpret_cast<double *>(workspace);
   const BnPlan p = plan_bn(y, dz, dz, C, S);
-  dim3 rgrid(p.splits, C);
-  if (p.vec) bn_reduce_kernel<1, true><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
-  else bn_reduce_kernel<1, false><<<rgrid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, save_mean, save_invstd, B, C, S, p.chunk, partial);
-  bn_sync_backward_local_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, (double)B * S, dgamma, dbeta, stats);
+  launch_reduce<1>(p, y, dz, gamma, beta, save_mean, save_invstd, B, C, S, partial, stream);
+  bn_finalize_backward_kernel<true><<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, dgamma, dbeta,
+                                                                          (double)B * S, stats);
   SPC_LAUNCH_CHECK("bn_relu_sync_backward_reduce");
   return SPC_OK;
 }
@@ -657,22 +688,14 @@ extern "C" int spc_bn_relu_sync_backward(const float *dz, const float *y, const 
                                          const float *save_mean, const float *save_invstd, int B, int C, int S,
                                          int world, const double *stats_all, float *dy, void *workspace,
                                          size_t workspace_bytes, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_sync_backward", B, C, world);
-  SPC_CHECK_ARG(S >= 1 && ((dz && y && dy) || B == 0) && gamma && beta && save_mean && save_invstd && stats_all,
-                "bn_relu_sync_backward: bad size or null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_sync_backward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  if (const int e = check_bn("bn_relu_sync_backward", B, 0, C, S, 1, world, {dz, y, dy},
+                             {gamma, beta, save_mean, save_invstd, stats_all})) return e;
+  if (const int e = check_workspace("bn_relu_sync_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
   bn_sync_combine_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, k0, k1);
   const BnPlan p = plan_bn(y, dz, dy, C, S);
-  const int slice = sync_batch_slice(C);
-  for (int b0 = 0; b0 < B; b0 += slice) {
-    const size_t off = (size_t)b0 * C * S;
-    dim3 agrid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
-    if (p.vec) bn_apply_kernel<1, true><<<agrid, BN_THREADS, 0, stream>>>(y + off, dz + off, gamma, beta, save_mean, save_invstd, k1, k0, C, S, 1.f, dy + off);
-    else bn_apply_kernel<1, false><<<agrid, BN_THREADS, 0, stream>>>(y + off, dz + off, gamma, beta, save_mean, save_invstd, k1, k0, C, S, 1.f, dy + off);
-  }
+  launch_apply<1>(p.vec, y, dz, gamma, beta, save_mean, save_invstd, k1, k0, B, C, S, 1.f, dy, stream);
   SPC_LAUNCH_CHECK("bn_relu_sync_backward");
   return SPC_OK;
 }
@@ -683,27 +706,13 @@ extern "C" int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gam
                                                 float eps, float momentum, float *running_mean, float *running_var,
                                                 float *pooled, uint8_t *argmax, float *ymax, float *save_mean,
                                                 float *save_invstd, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_maxpool_sync_forward", B, C, world);
-  SPC_CHECK_ARG(npoint >= 1 && (long long)npoint * nsample < (1LL << 31), "bn_relu_maxpool_sync_forward: bad sizes");
-  if (!pool_ns_supported(nsample) || (reinterpret_cast<uintptr_t>(y) & 15)) {
-    set_error("bn_relu_maxpool_sync: nsample=%d not in {16,32,64} or y not 16-byte aligned", nsample);
-    return SPC_ERR_UNSUPPORTED;
-  }
-  SPC_CHECK_ARG(((y && pooled && argmax && ymax) || B == 0) && gamma && beta && stats_all && save_mean && save_invstd,
-                "bn_relu_maxpool_sync_forward: null pointer");
+  if (const int e = check_bn("bn_relu_maxpool_sync_forward", B, 0, C, npoint, nsample, world, {y, pooled, argmax, ymax},
+                             {gamma, beta, stats_all, save_mean, save_invstd})) return e;
+  if (const int e = check_pool("bn_relu_maxpool_sync_forward", nsample, y, nullptr)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
                                                                         running_var, save_mean, save_invstd);
-  const int slice = sync_batch_slice(C);
-  for (int b0 = 0; b0 < B; b0 += slice) {
-    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
-#define BP_FWD(NS)                                                                                                  \
-  bn_relu_pool_fwd_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), min(slice, B - b0) * C), \
-                                BN_THREADS, 0, stream>>>(y + yo, gamma, beta, save_mean, save_invstd, C, npoint,     \
-                                                         pooled + po, argmax + po, ymax + po)
-    if (nsample == 16) BP_FWD(16); else if (nsample == 32) BP_FWD(32); else BP_FWD(64);
-#undef BP_FWD
-  }
+  launch_pool_fwd(y, gamma, beta, save_mean, save_invstd, B, C, npoint, nsample, pooled, argmax, ymax, stream);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_forward");
   return SPC_OK;
 }
@@ -713,13 +722,11 @@ extern "C" int spc_bn_relu_maxpool_sync_backward_reduce(const float *dpool, cons
                                                         const float *save_invstd, int B, int C, int npoint,
                                                         int nsample, float *dgamma, float *dbeta, double *stats,
                                                         void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_maxpool_sync_backward_reduce", B, C, 1);
-  SPC_CHECK_ARG(npoint >= 1 && nsample >= 1, "bn_relu_maxpool_sync_backward_reduce: bad sizes");
-  SPC_CHECK_ARG(((dpool && ymax) || B == 0) && gamma && beta && save_mean && save_invstd && dgamma && dbeta && stats,
-                "bn_relu_maxpool_sync_backward_reduce: null pointer");
+  if (const int e = check_bn("bn_relu_maxpool_sync_backward_reduce", B, 0, C, npoint, nsample, 1, {dpool, ymax},
+                             {gamma, beta, save_mean, save_invstd, dgamma, dbeta, stats})) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
-  bn_pool_sync_bwd_reduce_kernel<<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
-                                                               npoint, (double)B * npoint * nsample, dgamma, dbeta, stats);
+  bn_pool_bwd_reduce_kernel<true><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
+                                                                npoint, dgamma, dbeta, (double)B * npoint * nsample, stats);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward_reduce");
   return SPC_OK;
 }
@@ -729,29 +736,15 @@ extern "C" int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8
                                                  const float *save_mean, const float *save_invstd, int B, int C,
                                                  int npoint, int nsample, int world, const double *stats_all,
                                                  float *dy, void *workspace, size_t workspace_bytes, void *stream_) {
-  SPC_SYNC_CHECK("bn_relu_maxpool_sync_backward", B, C, world);
-  SPC_CHECK_ARG(npoint >= 1 && (long long)npoint * nsample < (1LL << 31), "bn_relu_maxpool_sync_backward: bad sizes");
-  if (!pool_ns_supported(nsample) || ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
-    set_error("bn_relu_maxpool_sync: nsample=%d not in {16,32,64} or tensors not 16-byte aligned", nsample);
-    return SPC_ERR_UNSUPPORTED;
-  }
-  SPC_CHECK_ARG(((dpool && argmax && ymax && y && dy) || B == 0) && gamma && beta && save_mean && save_invstd && stats_all,
-                "bn_relu_maxpool_sync_backward: null pointer");
-  SPC_CHECK_ARG(workspace && workspace_bytes >= spc_bn_relu_workspace_bytes(C) && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0,
-                "bn_relu_maxpool_sync_backward: workspace of spc_bn_relu_workspace_bytes(C) bytes required");
+  if (const int e = check_bn("bn_relu_maxpool_sync_backward", B, 0, C, npoint, nsample, world,
+                             {dpool, argmax, ymax, y, dy}, {gamma, beta, save_mean, save_invstd, stats_all})) return e;
+  if (const int e = check_pool("bn_relu_maxpool_sync_backward", nsample, y, dy)) return e;
+  if (const int e = check_workspace("bn_relu_maxpool_sync_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
   bn_sync_combine_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, k0, k1);
-  const int slice = sync_batch_slice(C);
-  for (int b0 = 0; b0 < B; b0 += slice) {
-    const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
-#define BP_BWD(NS)                                                                                                   \
-  bn_pool_bwd_apply_kernel<NS><<<dim3(ceil_div(npoint, (BN_THREADS / 32) * (32 / (NS / 4)) * BP_UNR), min(slice, B - b0) * C), \
-                                 BN_THREADS, 0, stream>>>(y + yo, dpool + po, argmax + po, ymax + po, gamma, beta,     \
-                                                          save_mean, save_invstd, k1, k0, C, npoint, 1.f, dy + yo)
-    if (nsample == 16) BP_BWD(16); else if (nsample == 32) BP_BWD(32); else BP_BWD(64);
-#undef BP_BWD
-  }
+  launch_pool_bwd(y, dpool, argmax, ymax, gamma, beta, save_mean, save_invstd, k1, k0, B, C, npoint, nsample, 1.f, dy,
+                  stream);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward");
   return SPC_OK;
 }

@@ -19,21 +19,36 @@ FUSED_BN_RELU_TRAINING = True
 
 
 class _BnReluTrain(torch.autograd.Function):
-    """z = relu(batch_norm(y, training=True)); saves y and the batch statistics, recomputes the ReLU mask."""
+    """z = relu(batch_norm(y, training=True)); saves y and the batch statistics, recomputes the ReLU mask.  With a
+    process `group`, the statistics are those of every rank of it (torch.nn.SyncBatchNorm semantics): one exchange of
+    (n, mean, M2) per channel in the forward and one of (n, sum dm, sum dm * xhat) in the backward."""
 
     @staticmethod
-    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps):
+    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
         from . import _ext
-        z, mean, invstd = _ext.bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, eps)
+        if group is None:
+            z, mean, invstd = _ext.bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, eps)
+        else:
+            rows, mine = _exchange_rows(y.shape[1], group, y.device)
+            _ext.bn_relu_sync_stats(y, mine)
+            z, mean, invstd = _ext.bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps,
+                                                        _all_gather_rows(rows, group))
         ctx.save_for_backward(y, gamma, beta, mean, invstd)
+        ctx.group = group
         return z
 
     @staticmethod
     def backward(ctx, dz):
         from . import _ext
         y, gamma, beta, mean, invstd = ctx.saved_tensors
-        dy, dgamma, dbeta = _ext.bn_relu_train_backward(dz.contiguous(), y, gamma, beta, mean, invstd)
-        return dy, dgamma, dbeta, None, None, None, None
+        dz = dz.contiguous()
+        if ctx.group is None:
+            dy, dgamma, dbeta = _ext.bn_relu_train_backward(dz, y, gamma, beta, mean, invstd)
+        else:
+            rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
+            dgamma, dbeta = _ext.bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, mine)
+            dy = _ext.bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, _all_gather_rows(rows, ctx.group))
+        return dy, dgamma, dbeta, None, None, None, None, None
 
 
 def _max_pool_last(x):
@@ -42,23 +57,37 @@ def _max_pool_last(x):
 
 
 class _BnReluMaxPoolTrain(torch.autograd.Function):
-    """pooled = max_k relu(batch_norm(y, training=True))[..., k] for y (B,C,npoint,nsample)."""
+    """pooled = max_k relu(batch_norm(y, training=True))[..., k] for y (B,C,npoint,nsample); `group` as in
+    _BnReluTrain."""
 
     @staticmethod
-    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps):
+    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
         from . import _ext
-        pooled, argmax, ymax, mean, invstd = _ext.bn_relu_maxpool_train_forward(
-            y, gamma, beta, running_mean, running_var, momentum, eps)
+        if group is None:
+            pooled, argmax, ymax, mean, invstd = _ext.bn_relu_maxpool_train_forward(
+                y, gamma, beta, running_mean, running_var, momentum, eps)
+        else:
+            rows, mine = _exchange_rows(y.shape[1], group, y.device)
+            _ext.bn_relu_sync_stats(y, mine)
+            pooled, argmax, ymax, mean, invstd = _ext.bn_relu_maxpool_sync_forward(
+                y, gamma, beta, running_mean, running_var, momentum, eps, _all_gather_rows(rows, group))
         ctx.save_for_backward(y, gamma, beta, mean, invstd, argmax, ymax)
+        ctx.group = group
         return pooled
 
     @staticmethod
     def backward(ctx, dpool):
         from . import _ext
         y, gamma, beta, mean, invstd, argmax, ymax = ctx.saved_tensors
-        dy, dgamma, dbeta = _ext.bn_relu_maxpool_train_backward(dpool.contiguous(), argmax, ymax, y, gamma, beta,
-                                                                mean, invstd)
-        return dy, dgamma, dbeta, None, None, None, None
+        dpool = dpool.contiguous()
+        if ctx.group is None:
+            dy, dgamma, dbeta = _ext.bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd)
+        else:
+            rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
+            dgamma, dbeta = _ext.bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, mine)
+            dy = _ext.bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd,
+                                                    _all_gather_rows(rows, ctx.group))
+        return dy, dgamma, dbeta, None, None, None, None, None
 
 
 def _exchange_rows(C, group, device):
@@ -73,58 +102,6 @@ def _all_gather_rows(rows, group):
     floating-point addition ever meets two non-zero terms); the rows are then combined in rank order on the device."""
     dist.all_reduce(rows, op=dist.ReduceOp.SUM, group=group)
     return rows
-
-
-class _BnReluSyncTrain(torch.autograd.Function):
-    """_BnReluTrain with the statistics of every rank of `group` (torch.nn.SyncBatchNorm semantics): one exchange of
-    (n, mean, M2) per channel in the forward and one of (n, sum dm, sum dm * xhat) in the backward."""
-
-    @staticmethod
-    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
-        from . import _ext
-        rows, mine = _exchange_rows(y.shape[1], group, y.device)
-        _ext.bn_relu_sync_stats(y, mine)
-        z, mean, invstd = _ext.bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps,
-                                                    _all_gather_rows(rows, group))
-        ctx.save_for_backward(y, gamma, beta, mean, invstd)
-        ctx.group = group
-        return z
-
-    @staticmethod
-    def backward(ctx, dz):
-        from . import _ext
-        y, gamma, beta, mean, invstd = ctx.saved_tensors
-        dz = dz.contiguous()
-        rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
-        dgamma, dbeta = _ext.bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, mine)
-        dy = _ext.bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, _all_gather_rows(rows, ctx.group))
-        return dy, dgamma, dbeta, None, None, None, None, None
-
-
-class _BnReluMaxPoolSyncTrain(torch.autograd.Function):
-    """_BnReluMaxPoolTrain with the statistics of every rank of `group`."""
-
-    @staticmethod
-    def forward(ctx, y, gamma, beta, running_mean, running_var, momentum, eps, group):
-        from . import _ext
-        rows, mine = _exchange_rows(y.shape[1], group, y.device)
-        _ext.bn_relu_sync_stats(y, mine)
-        pooled, argmax, ymax, mean, invstd = _ext.bn_relu_maxpool_sync_forward(
-            y, gamma, beta, running_mean, running_var, momentum, eps, _all_gather_rows(rows, group))
-        ctx.save_for_backward(y, gamma, beta, mean, invstd, argmax, ymax)
-        ctx.group = group
-        return pooled
-
-    @staticmethod
-    def backward(ctx, dpool):
-        from . import _ext
-        y, gamma, beta, mean, invstd, argmax, ymax = ctx.saved_tensors
-        dpool = dpool.contiguous()
-        rows, mine = _exchange_rows(y.shape[1], ctx.group, y.device)
-        dgamma, dbeta = _ext.bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, mine)
-        dy = _ext.bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd,
-                                                _all_gather_rows(rows, ctx.group))
-        return dy, dgamma, dbeta, None, None, None, None, None
 
 
 def _sync_group(bn):
@@ -215,27 +192,21 @@ class _ConvBase(nn.Sequential):
             run_conv = conv
         if self._fused_training_ok(x):
             bn = getattr(self, self._bn_name)[0]
-            y = run_conv(x)
-            group = _sync_group(bn)
-            # SyncBatchNorm: the synced kernels take any local batch, so whether they run depends only on C, nsample
-            # and the module, never on this rank's share of the batch, and all ranks issue the same collectives
-            if group is not None or (y.is_contiguous() and y.shape[0] * y.shape[1] <= 65535):
-                args = (y.contiguous(), bn.weight, bn.bias, bn.running_mean, bn.running_var, float(bn.momentum),
-                        float(bn.eps))
-                plain, pool = _BnReluTrain, _BnReluMaxPoolTrain
-                if group is not None:
-                    args, plain, pool = args + (group,), _BnReluSyncTrain, _BnReluMaxPoolSyncTrain
-                if max_pool_last_dim and y.dim() == 4 and y.shape[3] in (16, 32, 64):
-                    out = pool.apply(*args)
-                else:
-                    out = plain.apply(*args)
-                    if max_pool_last_dim:
-                        out = _max_pool_last(out)
-                if bn.num_batches_tracked is not None:
-                    bn.num_batches_tracked.add_(1)
-                return out
-            out = torch.relu_(getattr(self, self._bn_name)(y))
-        elif run_conv is not conv:
+            # the kernels take any batch, so whether they run depends only on the module, C and nsample, never on this
+            # rank's share of the batch: with SyncBatchNorm all ranks issue the same collectives
+            y = run_conv(x).contiguous()
+            args = (y, bn.weight, bn.bias, bn.running_mean, bn.running_var, float(bn.momentum), float(bn.eps),
+                    _sync_group(bn))
+            if max_pool_last_dim and y.dim() == 4 and y.shape[3] in (16, 32, 64):
+                out = _BnReluMaxPoolTrain.apply(*args)
+            else:
+                out = _BnReluTrain.apply(*args)
+                if max_pool_last_dim:
+                    out = _max_pool_last(out)
+            if bn.num_batches_tracked is not None:
+                bn.num_batches_tracked.add_(1)
+            return out
+        if run_conv is not conv:
             out = x
             for name, mod in self.named_children():
                 out = run_conv(out) if name == self._conv_name else mod(out)

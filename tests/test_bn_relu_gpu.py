@@ -1,6 +1,7 @@
 """Training-mode BatchNorm + ReLU kernels (csrc/bn_relu.cu) against torch.nn.BatchNorm2d + ReLU in fp32
 (the reference's pytorch_utils.Conv2d block, :11-36,39-64): forward values, running statistics,
-num_batches_tracked, input / affine gradients; then a whole SA module trained with and without the fusion."""
+num_batches_tracked, input / affine gradients; then a whole SA module, a channels_last block and a block with
+B*C > 65535 trained with and without the fusion."""
 import zlib
 
 import numpy as np
@@ -150,3 +151,55 @@ def test_bn_relu_maxpool_matches_torch(ns):
     torch.testing.assert_close(dy, yr.grad, rtol=1e-4, atol=1e-4 * max(1.0, yr.grad.abs().max().item()))
     torch.testing.assert_close(dg, gr.grad, rtol=1e-4, atol=1e-4 * max(1.0, gr.grad.abs().max().item()))
     torch.testing.assert_close(db, br.grad, rtol=1e-4, atol=1e-4 * max(1.0, br.grad.abs().max().item()))
+
+
+@pytest.mark.parametrize("case", ["channels_last", "BC72000-pool"])
+def test_conv_block_fuses_any_layout_and_batch(case, monkeypatch):
+    """A conv block whose output is not contiguous (a channels_last model) or has B*C > 65535 rows (the kernels then
+    run in slices of at most 65535 / C batch rows) takes the fused kernels too, with the same results as the plain
+    module sequence.  beta = 10 keeps every normalised value far from the ReLU kink, where the two may round apart."""
+    from spacap3d_b200 import _lib, pytorch_utils
+    pool = case.endswith("-pool")
+    B, Cin, C, H, W = (3, 4, 24000, 2, 16) if pool else (2, 8, 16, 64, 32)
+    g = torch.Generator().manual_seed(5)
+    x = torch.randn(B, Cin, H, W, generator=g).to(DEV)
+    wout = torch.randn((B, C, H) if pool else (B, C, H, W), generator=g).to(DEV)
+    names, real = [], _lib.call
+
+    def spy(name, *args):
+        names.append(name)
+        return real(name, *args)
+
+    monkeypatch.setattr(_lib, "call", spy)
+    # fp32 convolutions: with TF32 the conv backward rounds dy to 10 mantissa bits, which turns the fp32 rounding
+    # difference between the two BatchNorm implementations into 1e-3-level differences of the input gradient
+    monkeypatch.setattr(torch.backends.cudnn, "allow_tf32", False)
+    monkeypatch.setattr(torch.backends.cuda.matmul, "allow_tf32", False)
+    res = []
+    try:
+        for fused in (True, False):
+            pytorch_utils.FUSED_BN_RELU_TRAINING = fused
+            torch.manual_seed(7)
+            m = pytorch_utils.Conv2d(Cin, C, bn=True).to(DEV).train()
+            torch.nn.init.constant_(m.bn.bn.bias, 10.0)
+            xi = x.clone()
+            if not pool:
+                m = m.to(memory_format=torch.channels_last)
+                xi = xi.to(memory_format=torch.channels_last)
+                assert not m.conv(xi).is_contiguous()
+            xi.requires_grad_(True)
+            out = m(xi, max_pool_last_dim=pool)
+            (out * wout).sum().backward()
+            res.append((out.detach(), xi.grad, [p.grad for p in m.parameters()],
+                        {n: b.clone() for n, b in m.named_buffers()}))
+    finally:
+        pytorch_utils.FUSED_BN_RELU_TRAINING = True
+    fwd = "spc_bn_relu_maxpool_train_forward" if pool else "spc_bn_relu_train_forward"
+    assert names.count(fwd) == 1 and not [n for n in names if "_sync" in n], names
+    (o1, g1, p1, b1), (o2, g2, p2, b2) = res
+    torch.testing.assert_close(o1, o2, rtol=1e-4, atol=1e-5)
+    torch.testing.assert_close(g1, g2, rtol=1e-3, atol=1e-5 * max(1.0, g2.abs().max().item()))
+    for a, b in zip(p1, p2):
+        torch.testing.assert_close(a, b, rtol=1e-3, atol=1e-5 * max(1.0, b.abs().max().item()))
+    for k in b1:
+        torch.testing.assert_close(b1[k], b2[k], rtol=1e-5, atol=1e-6)

@@ -89,6 +89,7 @@ def _constants():
         "BN_MAX_SPLITS": ("bn_relu.cu", r"constexpr int BN_MAX_SPLITS = (\d+);"),
         "BN_CTAS_PER_SM": ("bn_relu.cu", r"int splits = ceil_div\((\d+) \* kNumSMs, C\);"),
         "BP_UNR": ("bn_relu.cu", r"constexpr int BP_UNR = (\d+);"),
+        "BN_SLICE_ROWS": ("bn_relu.cu", r"static int sync_batch_slice\(int C\) \{ return max\(1, (\d+) / C\); \}"),
     }
     k = {}
     for name, (f, pat) in pats.items():
@@ -416,6 +417,7 @@ BN_CASES = [                      # shape (B, C, ...): the statistics run over e
     dict(id="scalar-S2047", shape=(16, 5, 2047)),
     dict(id="C1-64splits", shape=(4, 1, 65536)),
     dict(id="BC65535", shape=(3, 21845, 16)),
+    dict(id="BC80000-slices", shape=(2, 40000, 16)),                     # two apply launches of one batch row
     dict(id="c5-160k-bn", shape=(4, 64, 8192, 64), dz1=True),            # M = 2^21
 ]
 POOL_CASES = [                    # shape (B, C, npoint, nsample)
@@ -425,6 +427,7 @@ POOL_CASES = [                    # shape (B, C, npoint, nsample)
     dict(id="ns16-ctas", shape=(2, 8, 1024, 16)),
     dict(id="ns32-ctas-np1000", shape=(2, 6, 1000, 32)),
     dict(id="ns64-ctas-eps3a2", shape=(4, 4, 512, 64), eps3=True),
+    dict(id="ns16-BC66000-slices", shape=(2, 33000, 2, 16)),             # two pool launches of one batch row
     dict(id="c5-200k-bnpool", shape=(4, 128, 10240, 64), dz1=True),       # M = 2 621 440
 ]
 BN_MOMENTUM = 0.125
@@ -646,6 +649,8 @@ def bn_branches(K, c, pool=False):
             br.add("bn C=1, 64 splits")
         if B * C == 65535:
             br.add("bn B*C=65535")
+    if B > max(1, K["BN_SLICE_ROWS"] // C):
+        br.add("sliced apply")
     if c.get("eps3"):
         br.add("bn eps=3a^2")
     if c["id"].startswith("c5-"):
@@ -686,7 +691,7 @@ BRANCHES = {
     "interp grad smem", "interp grad opt-in smem", "interp grad global", "interp grad smem, n=0",
     "interp grad global, n=0",
     "bn vector, one split", "bn vector, several splits", "bn scalar, several splits", "bn S%4!=0",
-    "bn C=1, 64 splits", "bn B*C=65535", "bn eps=3a^2",
+    "bn C=1, 64 splits", "bn B*C=65535", "bn eps=3a^2", "sliced apply",
     "pool ns=16", "pool ns=32", "pool ns=64", "pool below one CTA", "pool several CTAs",
     "pool npoint not a power of two",
     "c5-80k-sa1-xyz", "c5-80k-sa1-feat", "c5-80k-sa2", "c5-160k-sa2", "c5-160k-sa3", "c5-160k-bn",
@@ -778,4 +783,6 @@ def test_cases_reach_their_branches():
     assert {"gather 16 tiles", "gather long lists"} <= reached["c5-200k-sa2"]
     assert "interp grad opt-in smem" in reached["interp c5-200k-fp2"]
     assert "pool several CTAs" in reached["pool c5-200k-bnpool"]
+    assert "sliced apply" in reached["bn BC80000-slices"] and "sliced apply" in reached["pool ns16-BC66000-slices"]
+    assert "sliced apply" not in reached["bn BC65535"]
     assert plan_bn(K, 64, 8192 * 64, True) == (True, 10)
