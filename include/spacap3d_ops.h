@@ -131,6 +131,21 @@ int spc_group_points_grad_ex(const float *grad_out, const int32_t *idx, int B, i
                              int npoint, int nsample, float *grad_points, void *workspace,
                              size_t workspace_bytes, void *stream);
 
+/* bf16 storage (torch.autocast(dtype=torch.bfloat16) training) of the three entries above: the same operators and
+ * argument lists with points / out / grad_out as __nv_bfloat16 device tensors (void pointers).
+ *   spc_group_points_bf16        group_points(points, idx)        bf16 in, bf16 out (a copy: no rounding);
+ *                                rows of up to ~100 k points are staged (the budget counts bytes)
+ *   spc_group_points_grad_bf16   group_points_grad(grad_out, idx, n)   bf16 grad_out in, FP32 grad_points out,
+ *   spc_group_points_grad_ex_bf16                                       fp32 accumulation, same kernel choice
+ * The gradient stays fp32 (it is nsample times smaller than grad_out): no bf16 atomics, one rounding by the caller. */
+int spc_group_points_bf16(const void *points, const int32_t *idx, int B, int C, int N, int npoint,
+                          int nsample, void *out, void *stream);
+int spc_group_points_grad_bf16(const void *grad_out, const int32_t *idx, int B, int C, int N,
+                               int npoint, int nsample, float *grad_points, void *stream);
+int spc_group_points_grad_ex_bf16(const void *grad_out, const int32_t *idx, int B, int C, int N,
+                                  int npoint, int nsample, float *grad_points, void *workspace,
+                                  size_t workspace_bytes, void *stream);
+
 /* three_nn(unknowns, knows)                              interpolate.cpp:14-40, interpolate_gpu.cu:9-68
  * unknown (B,n,3), known (B,m,3) -> dist2 (B,n,3) SQUARED distances ascending, idx (B,n,3).
  * m < 3 leaves +inf / index 0 in the unfilled slots, like the reference. */
@@ -146,6 +161,15 @@ int spc_three_interpolate(const float *points, const int32_t *idx, const float *
  * grad_out (B,C,n), idx (B,n,3), weight (B,n,3) -> grad_points (B,C,m) */
 int spc_three_interpolate_grad(const float *grad_out, const int32_t *idx, const float *weight,
                                int B, int C, int n, int m, float *grad_points, void *stream);
+
+/* bf16 storage of the two entries above (same argument lists; idx and weight stay int32 / fp32):
+ *   spc_three_interpolate_bf16       three_interpolate(points, idx, weight)        bf16 points -> bf16 out
+ *                                    (fp32 arithmetic, one rounding per output)
+ *   spc_three_interpolate_grad_bf16  three_interpolate_grad(grad_out, idx, weight, m)  bf16 grad_out -> FP32 grad_points */
+int spc_three_interpolate_bf16(const void *points, const int32_t *idx, const float *weight, int B,
+                               int C, int m, int n, void *out, void *stream);
+int spc_three_interpolate_grad_bf16(const void *grad_out, const int32_t *idx, const float *weight,
+                                    int B, int C, int n, int m, float *grad_points, void *stream);
 
 
 /* Fused set-abstraction forward, eval mode (no reference C++ counterpart: it replaces the whole
@@ -309,6 +333,61 @@ int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8_t *argmax,
                                       const float *save_invstd, int B, int C, int npoint, int nsample, int world,
                                       const double *stats_all, float *dy, void *workspace, size_t workspace_bytes,
                                       void *stream);
+
+/* ---- bf16 storage of the eleven training-mode BatchNorm + ReLU entries above ---------------------------------------
+ * The same passes and argument lists (each `_bf16` entry replaces the same reference code as its fp32 twin) with
+ * y, z, dz, dy, dpool, pooled and ymax as __nv_bfloat16 device tensors (void pointers): what
+ * nn.BatchNorm2d + nn.ReLU + F.max_pool2d compute on the bf16 output of a 1x1 convolution under
+ * torch.autocast(dtype=torch.bfloat16).  gamma, beta, save_mean / save_invstd, dgamma / dbeta and the running
+ * statistics stay fp32, the partial sums and the exchanged (world, C, SPC_BN_SYNC_K) rows fp64, and the arithmetic
+ * fp32; each bf16 output is rounded once (to nearest even).  The ReLU gradient passes where the bf16 output is > 0,
+ * and the max-pool compares the bf16-ROUNDED values of relu(bn(y)): slots that round to the same value tie and the
+ * lowest one wins, as F.max_pool2d on the bf16 tensor.  Vector kernels need 8-byte (not 16-byte) alignment. */
+int spc_bn_relu_train_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C, int S,
+                                   float eps, float momentum, float *running_mean, float *running_var, void *z,
+                                   float *save_mean, float *save_invstd, void *workspace, size_t workspace_bytes,
+                                   void *stream);
+int spc_bn_relu_train_backward_bf16(const void *dz, const void *y, const float *gamma, const float *beta,
+                                    const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                    void *dy, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes,
+                                    void *stream);
+int spc_bn_relu_maxpool_train_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C,
+                                           int npoint, int nsample, float eps, float momentum,
+                                           float *running_mean, float *running_var, void *pooled,
+                                           uint8_t *argmax, void *ymax, float *save_mean, float *save_invstd,
+                                           void *workspace, size_t workspace_bytes, void *stream);
+int spc_bn_relu_maxpool_train_backward_bf16(const void *dpool, const uint8_t *argmax, const void *ymax,
+                                            const void *y, const float *gamma, const float *beta,
+                                            const float *save_mean, const float *save_invstd, int B, int C,
+                                            int npoint, int nsample, void *dy, float *dgamma, float *dbeta,
+                                            void *stream);
+int spc_bn_relu_sync_stats_bf16(const void *y, int B, int C, int S, double *stats, void *workspace,
+                                size_t workspace_bytes, void *stream);
+int spc_bn_relu_sync_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C, int S, int world,
+                                  const double *stats_all, float eps, float momentum, float *running_mean,
+                                  float *running_var, void *z, float *save_mean, float *save_invstd, void *stream);
+int spc_bn_relu_sync_backward_reduce_bf16(const void *dz, const void *y, const float *gamma, const float *beta,
+                                          const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                          float *dgamma, float *dbeta, double *stats, void *workspace,
+                                          size_t workspace_bytes, void *stream);
+int spc_bn_relu_sync_backward_bf16(const void *dz, const void *y, const float *gamma, const float *beta,
+                                   const float *save_mean, const float *save_invstd, int B, int C, int S, int world,
+                                   const double *stats_all, void *dy, void *workspace, size_t workspace_bytes,
+                                   void *stream);
+int spc_bn_relu_maxpool_sync_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C,
+                                          int npoint, int nsample, int world, const double *stats_all, float eps,
+                                          float momentum, float *running_mean, float *running_var, void *pooled,
+                                          uint8_t *argmax, void *ymax, float *save_mean, float *save_invstd,
+                                          void *stream);
+int spc_bn_relu_maxpool_sync_backward_reduce_bf16(const void *dpool, const void *ymax, const float *gamma,
+                                                  const float *beta, const float *save_mean, const float *save_invstd,
+                                                  int B, int C, int npoint, int nsample, float *dgamma, float *dbeta,
+                                                  double *stats, void *stream);
+int spc_bn_relu_maxpool_sync_backward_bf16(const void *dpool, const uint8_t *argmax, const void *ymax, const void *y,
+                                           const float *gamma, const float *beta, const float *save_mean,
+                                           const float *save_invstd, int B, int C, int npoint, int nsample, int world,
+                                           const double *stats_all, void *dy, void *workspace, size_t workspace_bytes,
+                                           void *stream);
 
 /* ---- detection post-processing (SURVEY row N3): device side of parse_predictions, lib/ap_helper.py:44-160 ----
  * spc_box_point_counts: counts[b,k] = number of points of scene b inside predicted box k (the reference's

@@ -30,6 +30,22 @@ def _check(t, name, dtype):
         raise RuntimeError("%s must be %s tensor" % (name, kind))
 
 
+def _storage(t, name):
+    """Entry-point suffix of a tensor the training-path kernels store as fp32 ('') or bf16 ('_bf16': the
+    torch.autocast(dtype=torch.bfloat16) twins).  Any other dtype raises the fp32 check's message."""
+    if isinstance(t, torch.Tensor) and t.dtype == torch.bfloat16:
+        _check(t, name, torch.bfloat16)
+        return "_bf16"
+    _check(t, name, torch.float32)
+    return ""
+
+
+def _grad_as(grad, t):
+    """The bf16 twins write fp32 gradients (no bf16 atomics); autograd wants them in the dtype of the forward input,
+    which is that of the incoming gradient t: one rounding."""
+    return grad if t.dtype == grad.dtype else grad.to(t.dtype)
+
+
 def _same_device(a, *rest):
     """Checked after dtype/contiguity of every argument, like the reference (sampling.cpp:15-35)."""
     if not a.is_cuda:
@@ -205,22 +221,23 @@ def ball_query(new_xyz, xyz, radius, nsample):
 
 
 def group_points(points, idx):
-    """(B,C,N), (B,npoint,nsample) -> (B,C,npoint,nsample).   group_points.cpp:12-36"""
-    _check(points, "points", torch.float32)
+    """(B,C,N), (B,npoint,nsample) -> (B,C,npoint,nsample), f32 or bf16 like points.   group_points.cpp:12-36"""
+    sfx = _storage(points, "points")
     _check(idx, "idx", torch.int32)
     _same_device(points, idx)
     B, C, N = points.shape
     _, npoint, nsample = idx.shape
-    out = torch.empty((B, C, npoint, nsample), dtype=torch.float32, device=points.device)
+    out = torch.empty((B, C, npoint, nsample), dtype=points.dtype, device=points.device)
     with torch.cuda.device(points.device):
-        _lib.call("spc_group_points", points.data_ptr(), idx.data_ptr(), B, C, N, npoint, nsample,
+        _lib.call("spc_group_points" + sfx, points.data_ptr(), idx.data_ptr(), B, C, N, npoint, nsample,
                   out.data_ptr(), _stream())
     return out
 
 
 def group_points_grad(grad_out, idx, n):
-    """(B,C,npoint,nsample), (B,npoint,nsample) -> (B,C,n).   group_points.cpp:38-62"""
-    _check(grad_out, "grad_out", torch.float32)
+    """(B,C,npoint,nsample), (B,npoint,nsample) -> (B,C,n) in grad_out's dtype (f32 or bf16; accumulated in
+    fp32).   group_points.cpp:38-62"""
+    sfx = _storage(grad_out, "grad_out")
     _check(idx, "idx", torch.int32)
     _same_device(grad_out, idx)
     B, C, npoint, nsample = grad_out.shape
@@ -229,12 +246,12 @@ def group_points_grad(grad_out, idx, n):
         nbytes = _lib.load().spc_group_points_grad_workspace_bytes(B, int(n), npoint, nsample) if C >= 4 else 0
         if nbytes:
             ws = torch.empty((nbytes + 3) // 4, dtype=torch.int32, device=grad_out.device)
-            _lib.call("spc_group_points_grad_ex", grad_out.data_ptr(), idx.data_ptr(), B, C, int(n),
+            _lib.call("spc_group_points_grad_ex" + sfx, grad_out.data_ptr(), idx.data_ptr(), B, C, int(n),
                       npoint, nsample, out.data_ptr(), ws.data_ptr(), nbytes, _stream())
         else:
-            _lib.call("spc_group_points_grad", grad_out.data_ptr(), idx.data_ptr(), B, C, int(n),
+            _lib.call("spc_group_points_grad" + sfx, grad_out.data_ptr(), idx.data_ptr(), B, C, int(n),
                       npoint, nsample, out.data_ptr(), _stream())
-    return out
+    return _grad_as(out, grad_out)
 
 
 def three_nn(unknowns, knows):
@@ -253,32 +270,33 @@ def three_nn(unknowns, knows):
 
 
 def three_interpolate(points, idx, weight):
-    """(B,C,m), (B,n,3), (B,n,3) -> (B,C,n).   interpolate.cpp:42-70"""
-    _check(points, "points", torch.float32)
+    """(B,C,m), (B,n,3), (B,n,3) f32 -> (B,C,n), f32 or bf16 like points.   interpolate.cpp:42-70"""
+    sfx = _storage(points, "points")
     _check(idx, "idx", torch.int32)
     _check(weight, "weight", torch.float32)
     _same_device(points, idx, weight)
     B, C, m = points.shape
     n = idx.shape[1]
-    out = torch.empty((B, C, n), dtype=torch.float32, device=points.device)
+    out = torch.empty((B, C, n), dtype=points.dtype, device=points.device)
     with torch.cuda.device(points.device):
-        _lib.call("spc_three_interpolate", points.data_ptr(), idx.data_ptr(), weight.data_ptr(),
+        _lib.call("spc_three_interpolate" + sfx, points.data_ptr(), idx.data_ptr(), weight.data_ptr(),
                   B, C, m, n, out.data_ptr(), _stream())
     return out
 
 
 def three_interpolate_grad(grad_out, idx, weight, m):
-    """(B,C,n), (B,n,3), (B,n,3) -> (B,C,m).   interpolate.cpp:71-99"""
-    _check(grad_out, "grad_out", torch.float32)
+    """(B,C,n), (B,n,3), (B,n,3) f32 -> (B,C,m) in grad_out's dtype (f32 or bf16; accumulated in fp32).
+    interpolate.cpp:71-99"""
+    sfx = _storage(grad_out, "grad_out")
     _check(idx, "idx", torch.int32)
     _check(weight, "weight", torch.float32)
     _same_device(grad_out, idx, weight)
     B, C, n = grad_out.shape
     out = torch.empty((B, C, int(m)), dtype=torch.float32, device=grad_out.device)
     with torch.cuda.device(grad_out.device):
-        _lib.call("spc_three_interpolate_grad", grad_out.data_ptr(), idx.data_ptr(),
+        _lib.call("spc_three_interpolate_grad" + sfx, grad_out.data_ptr(), idx.data_ptr(),
                   weight.data_ptr(), B, C, n, int(m), out.data_ptr(), _stream())
-    return out
+    return _grad_as(out, grad_out)
 
 
 def sa_fused_forward(xyz, new_xyz, idx, W0, b0, W1, b1, W2, b2, *, G=None, feat=None, radius=1.0,
@@ -441,16 +459,19 @@ def _per_channel(C, device):
 def _pool_outputs(y):
     """(pooled, argmax, ymax, save_mean, save_invstd) of a max-pool forward of y (B,C,npoint,nsample)."""
     B, C, npoint, _ = y.shape
-    pooled = torch.empty((B, C, npoint), dtype=torch.float32, device=y.device)
+    pooled = torch.empty((B, C, npoint), dtype=y.dtype, device=y.device)
     argmax = torch.empty((B, C, npoint), dtype=torch.uint8, device=y.device)
-    ymax = torch.empty((B, C, npoint), dtype=torch.float32, device=y.device)
+    ymax = torch.empty((B, C, npoint), dtype=y.dtype, device=y.device)
     return (pooled, argmax, ymax) + _per_channel(C, y.device)
 
 
+# The BatchNorm + ReLU wrappers below take y (and dz / dpool / ymax) as f32 or bf16 and return z / pooled / ymax / dy
+# in the same dtype; gamma, beta, the saved statistics, dgamma / dbeta and the running statistics are f32.
+
 def bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, eps):
-    """Training-mode BatchNorm + ReLU of y (B,C,*) f32 (pytorch_utils.py:11-36,39-64): returns
+    """Training-mode BatchNorm + ReLU of y (B,C,*) f32 or bf16 (pytorch_utils.py:11-36,39-64): returns
     (z, save_mean, save_invstd); running_mean / running_var (or None) are updated in place."""
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
     _check(gamma, "gamma", torch.float32)
     _check(beta, "beta", torch.float32)
     _same_device(y, gamma, beta)
@@ -459,7 +480,7 @@ def bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, e
     mean, invstd = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_train_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
+        _lib.call("spc_bn_relu_train_forward" + sfx, y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
                   float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
@@ -469,15 +490,15 @@ def bn_relu_train_forward(y, gamma, beta, running_mean, running_var, momentum, e
 
 def bn_relu_train_backward(dz, y, gamma, beta, mean, invstd):
     """-> (dy, dgamma, dbeta) for z = relu(batch_norm(y)) given dz."""
-    _check(dz, "dz", torch.float32)
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
+    _check(dz, "dz", y.dtype)
     _same_device(dz, y)
     B, C, S = _bn_sizes(y)
     dy = torch.empty_like(y)
     dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_train_backward", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+        _lib.call("spc_bn_relu_train_backward" + sfx, dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
                   mean.data_ptr(), invstd.data_ptr(), B, C, S, dy.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(),
                   ws.data_ptr(), nbytes, _stream())
     return dy, dgamma, dbeta
@@ -488,13 +509,13 @@ def bn_relu_maxpool_train_forward(y, gamma, beta, running_mean, running_var, mom
     BatchNorm(train) + ReLU + max over nsample without materialising the activation
     (pytorch_utils.py:11-36 + pointnet2_modules.py:256-259).  Raises SpcUnsupported for nsample not in
     {16,32,64}."""
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
     _same_device(y, gamma, beta)
     B, C, npoint, nsample = y.shape
     out = _pool_outputs(y)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_maxpool_train_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
+        _lib.call("spc_bn_relu_maxpool_train_forward" + sfx, y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
                   npoint, nsample, float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
@@ -504,13 +525,15 @@ def bn_relu_maxpool_train_forward(y, gamma, beta, running_mean, running_var, mom
 
 def bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd):
     """-> (dy (B,C,npoint,nsample), dgamma, dbeta)."""
-    _check(dpool, "dpool", torch.float32)
+    sfx = _storage(y, "y")
+    _check(dpool, "dpool", y.dtype)
+    _check(ymax, "ymax", y.dtype)
     _same_device(dpool, y)
     B, C, npoint, nsample = y.shape
     dy = torch.empty_like(y)
     dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
-        _lib.call("spc_bn_relu_maxpool_train_backward", dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
+        _lib.call("spc_bn_relu_maxpool_train_backward" + sfx, dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
                   y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C,
                   npoint, nsample, dy.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _stream())
     return dy, dgamma, dbeta
@@ -529,20 +552,20 @@ def _check_rows(rows, C, what):
 def bn_relu_sync_stats(y, row):
     """This rank's per-channel (n, mean, M2) of y (B,C,*) f32 into row (C, BN_SYNC_K) f64; also the statistics phase
     of the max-pool variant."""
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
     B, C, S = _bn_sizes(y)
     _check_rows(row, C, "row")
     _same_device(y, row)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_sync_stats", y.data_ptr(), B, C, S, row.data_ptr(), ws.data_ptr(), nbytes, _stream())
+        _lib.call("spc_bn_relu_sync_stats" + sfx, y.data_ptr(), B, C, S, row.data_ptr(), ws.data_ptr(), nbytes, _stream())
 
 
 def bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps, rows):
     """z = relu(batch_norm(y)) with the statistics combined from rows (world, C, BN_SYNC_K), every rank's
     bn_relu_sync_stats row: returns (z, save_mean, save_invstd); running_mean / running_var (or None) are updated
     in place with the global mean and unbiased variance."""
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
     _check(gamma, "gamma", torch.float32)
     _check(beta, "beta", torch.float32)
     B, C, S = _bn_sizes(y)
@@ -551,7 +574,7 @@ def bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, ep
     z = torch.empty_like(y)
     mean, invstd = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
-        _lib.call("spc_bn_relu_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
+        _lib.call("spc_bn_relu_sync_forward" + sfx, y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C, S,
                   rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
@@ -561,15 +584,15 @@ def bn_relu_sync_forward(y, gamma, beta, running_mean, running_var, momentum, ep
 
 def bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, row):
     """-> (dgamma, dbeta) of this rank; writes its (n, sum dm, sum dm * xhat) into row (C, BN_SYNC_K) f64."""
-    _check(dz, "dz", torch.float32)
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
+    _check(dz, "dz", y.dtype)
     B, C, S = _bn_sizes(y)
     _check_rows(row, C, "row")
     _same_device(dz, y, row)
     dgamma, dbeta = _per_channel(C, y.device)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_sync_backward_reduce", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+        _lib.call("spc_bn_relu_sync_backward_reduce" + sfx, dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
                   mean.data_ptr(), invstd.data_ptr(), B, C, S, dgamma.data_ptr(), dbeta.data_ptr(), row.data_ptr(),
                   ws.data_ptr(), nbytes, _stream())
     return dgamma, dbeta
@@ -577,15 +600,15 @@ def bn_relu_sync_backward_reduce(dz, y, gamma, beta, mean, invstd, row):
 
 def bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, rows):
     """-> dy from dz, y and every rank's bn_relu_sync_backward_reduce row (rows (world, C, BN_SYNC_K))."""
-    _check(dz, "dz", torch.float32)
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
+    _check(dz, "dz", y.dtype)
     B, C, S = _bn_sizes(y)
     _check_rows(rows, C, "rows")
     _same_device(dz, y, rows)
     dy = torch.empty_like(y)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_sync_backward", dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
+        _lib.call("spc_bn_relu_sync_backward" + sfx, dz.data_ptr(), y.data_ptr(), gamma.data_ptr(), beta.data_ptr(),
                   mean.data_ptr(), invstd.data_ptr(), B, C, S, rows.shape[0], rows.data_ptr(), dy.data_ptr(),
                   ws.data_ptr(), nbytes, _stream())
     return dy
@@ -594,7 +617,7 @@ def bn_relu_sync_backward(dz, y, gamma, beta, mean, invstd, rows):
 def bn_relu_maxpool_sync_forward(y, gamma, beta, running_mean, running_var, momentum, eps, rows):
     """bn_relu_maxpool_train_forward with the statistics combined from rows (world, C, BN_SYNC_K), every rank's
     bn_relu_sync_stats row of its y (B,C,npoint,nsample): -> (pooled, argmax, ymax, save_mean, save_invstd)."""
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
     _check(gamma, "gamma", torch.float32)
     _check(beta, "beta", torch.float32)
     B, C, npoint, nsample = y.shape
@@ -602,7 +625,7 @@ def bn_relu_maxpool_sync_forward(y, gamma, beta, running_mean, running_var, mome
     _same_device(y, gamma, beta, rows)
     out = _pool_outputs(y)
     with torch.cuda.device(y.device):
-        _lib.call("spc_bn_relu_maxpool_sync_forward", y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
+        _lib.call("spc_bn_relu_maxpool_sync_forward" + sfx, y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), B, C,
                   npoint, nsample, rows.shape[0], rows.data_ptr(), float(eps), float(momentum),
                   running_mean.data_ptr() if running_mean is not None else None,
                   running_var.data_ptr() if running_var is not None else None,
@@ -612,14 +635,14 @@ def bn_relu_maxpool_sync_forward(y, gamma, beta, running_mean, running_var, mome
 
 def bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invstd, row):
     """-> (dgamma, dbeta) of this rank for the max-pool variant; writes its row (C, BN_SYNC_K) f64."""
-    _check(dpool, "dpool", torch.float32)
-    _check(ymax, "ymax", torch.float32)
+    sfx = _storage(dpool, "dpool")
+    _check(ymax, "ymax", dpool.dtype)
     _same_device(dpool, ymax, row)
     B, C, npoint, nsample = y.shape
     _check_rows(row, C, "row")
     dgamma, dbeta = _per_channel(C, dpool.device)
     with torch.cuda.device(dpool.device):
-        _lib.call("spc_bn_relu_maxpool_sync_backward_reduce", dpool.data_ptr(), ymax.data_ptr(), gamma.data_ptr(),
+        _lib.call("spc_bn_relu_maxpool_sync_backward_reduce" + sfx, dpool.data_ptr(), ymax.data_ptr(), gamma.data_ptr(),
                   beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C, npoint, nsample, dgamma.data_ptr(),
                   dbeta.data_ptr(), row.data_ptr(), _stream())
     return dgamma, dbeta
@@ -627,15 +650,15 @@ def bn_relu_maxpool_sync_backward_reduce(dpool, ymax, y, gamma, beta, mean, invs
 
 def bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, mean, invstd, rows):
     """-> dy (B,C,npoint,nsample) from dpool and every rank's bn_relu_maxpool_sync_backward_reduce row."""
-    _check(dpool, "dpool", torch.float32)
-    _check(y, "y", torch.float32)
+    sfx = _storage(y, "y")
+    _check(dpool, "dpool", y.dtype)
     B, C, npoint, nsample = y.shape
     _check_rows(rows, C, "rows")
     _same_device(dpool, y, rows)
     dy = torch.empty_like(y)
     with torch.cuda.device(y.device):
         ws, nbytes = _bn_workspace(C, y.device)
-        _lib.call("spc_bn_relu_maxpool_sync_backward", dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
+        _lib.call("spc_bn_relu_maxpool_sync_backward" + sfx, dpool.data_ptr(), argmax.data_ptr(), ymax.data_ptr(),
                   y.data_ptr(), gamma.data_ptr(), beta.data_ptr(), mean.data_ptr(), invstd.data_ptr(), B, C,
                   npoint, nsample, rows.shape[0], rows.data_ptr(), dy.data_ptr(), ws.data_ptr(), nbytes, _stream())
     return dy

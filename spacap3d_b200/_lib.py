@@ -9,7 +9,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # SPC_LIB_PATH lets a developer load an instrumented build of the same library (profiling only)
 LIB_PATH = os.environ.get("SPC_LIB_PATH") or os.path.join(_HERE, "libspacap3d_ops.so")
-ABI_VERSION = 19
+ABI_VERSION = 20
 
 _p = ctypes.c_void_p
 _i = ctypes.c_int
@@ -58,6 +58,16 @@ SIGNATURES = {
     "spc_sa_fused_forward_ex": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _f, _p, _p, _p, _p,
                                 _i, _i, _i, _i, _i, _i, _i, _p, _p, _i, _p],
 }
+# bf16-storage twins (torch.autocast training): the same argument lists, the bf16 tensors passed as void pointers
+BF16_TWINS = (
+    "spc_group_points", "spc_group_points_grad", "spc_group_points_grad_ex",
+    "spc_three_interpolate", "spc_three_interpolate_grad",
+    "spc_bn_relu_train_forward", "spc_bn_relu_train_backward",
+    "spc_bn_relu_maxpool_train_forward", "spc_bn_relu_maxpool_train_backward",
+    "spc_bn_relu_sync_stats", "spc_bn_relu_sync_forward", "spc_bn_relu_sync_backward_reduce", "spc_bn_relu_sync_backward",
+    "spc_bn_relu_maxpool_sync_forward", "spc_bn_relu_maxpool_sync_backward_reduce", "spc_bn_relu_maxpool_sync_backward",
+)
+SIGNATURES.update({name + "_bf16": SIGNATURES[name] for name in BF16_TWINS})
 
 _lib = None
 

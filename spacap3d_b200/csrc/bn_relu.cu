@@ -1,4 +1,4 @@
-// bn_relu.cu -- training-mode BatchNorm + ReLU over (B, C, S) fp32 activations, forward and backward (sm_100a).
+// bn_relu.cu -- training-mode BatchNorm + ReLU over (B, C, S) fp32 or bf16 activations, forward and backward (sm_100a).
 //
 // Replaces, for the shared-MLP blocks in TRAINING mode, the reference's
 //     nn.BatchNorm2d (pytorch_utils.py:39-64, cuDNN bn_fw_tr / bn_bw kernels) followed by nn.ReLU(inplace=True)
@@ -15,6 +15,9 @@
 // Semantics = torch.nn.functional.batch_norm(training=True) + relu: biased variance for normalisation,
 // running_mean/var updated with `momentum` and the unbiased variance, save_mean / save_invstd for backward,
 // gradient of ReLU taken where the OUTPUT is > 0.
+// Every kernel is instantiated for float and bf16 storage of y, z, dz, dy, dpool, pooled and ymax (common.cuh):
+// arithmetic, partial sums and per-channel tensors stay fp32 / fp64, and a bf16 pass compares and masks the
+// bf16-ROUNDED relu(bn(y)), as torch's own bf16 sequence (batch_norm -> relu -> max_pool2d) sees it.
 #include <initializer_list>
 #include <type_traits>
 
@@ -45,8 +48,8 @@ __device__ __forceinline__ double block_sum_double(double v, double *s_red) {
 
 // grid (splits, C): CTA (s, c) reduces positions [p0, p1) of every batch row of channel c.
 // MODE 0: sums of (x-K), (x-K)^2.   MODE 1 (backward): sums of dzm, dzm * xhat.
-template <int MODE, bool VEC>
-__global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float *__restrict__ y, const float *__restrict__ dz,
+template <class T, int MODE, bool VEC>
+__global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const T *__restrict__ y, const T *__restrict__ dz,
                                                                 const float *__restrict__ gamma,
                                                                 const float *__restrict__ beta,
                                                                 const float *__restrict__ mean,
@@ -57,7 +60,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float *__re
   const int p0 = s * chunk, p1 = min(S, p0 + chunk);
   float a0 = 0.f, a1 = 0.f;
   float K = 0.f, mu = 0.f, is = 0.f, g = 0.f, bt = 0.f;
-  if (MODE == 0) K = __ldg(y + (size_t)c * S);
+  if (MODE == 0) K = to_f32(__ldg(y + (size_t)c * S));
   else { mu = __ldg(mean + c); is = __ldg(invstd + c); g = __ldg(gamma + c); bt = __ldg(beta + c); }
   auto acc = [&](float yv, float dv) {
     if (MODE == 0) {
@@ -67,22 +70,22 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float *__re
     } else {
       const float xh = (yv - mu) * is;
       const float z = fmaf(xh, g, bt);
-      const float dm = z > 0.f ? dv : 0.f;
+      const float dm = stored<T>(z) > 0.f ? dv : 0.f;
       a0 += dm;
       a1 = fmaf(dm, xh, a1);
     }
   };
   for (int b = 0; b < B; ++b) {
-    const float *row = y + ((size_t)b * C + c) * S;
-    const float *drow = MODE == 1 ? dz + ((size_t)b * C + c) * S : nullptr;
+    const T *row = y + ((size_t)b * C + c) * S;
+    const T *drow = MODE == 1 ? dz + ((size_t)b * C + c) * S : nullptr;
     if (VEC) {
       int p = p0 + threadIdx.x * 4;
       for (; p + (BN_UNR - 1) * BN_THREADS * 4 < p1; p += BN_UNR * BN_THREADS * 4) {
         float4 v[BN_UNR], d[BN_UNR];
 #pragma unroll
         for (int u = 0; u < BN_UNR; ++u) {
-          v[u] = __ldg(reinterpret_cast<const float4 *>(row + p + u * BN_THREADS * 4));
-          if (MODE == 1) d[u] = __ldg(reinterpret_cast<const float4 *>(drow + p + u * BN_THREADS * 4));
+          v[u] = ldg4(row + p + u * BN_THREADS * 4);
+          if (MODE == 1) d[u] = ldg4(drow + p + u * BN_THREADS * 4);
         }
 #pragma unroll
         for (int u = 0; u < BN_UNR; ++u) {
@@ -91,13 +94,14 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float *__re
         }
       }
       for (; p < p1; p += BN_THREADS * 4) {
-        const float4 v = __ldg(reinterpret_cast<const float4 *>(row + p));
+        const float4 v = ldg4(row + p);
         float4 d = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (MODE == 1) d = __ldg(reinterpret_cast<const float4 *>(drow + p));
+        if (MODE == 1) d = ldg4(drow + p);
         acc(v.x, d.x); acc(v.y, d.y); acc(v.z, d.z); acc(v.w, d.w);
       }
     } else {
-      for (int p = p0 + threadIdx.x; p < p1; p += BN_THREADS) acc(__ldg(row + p), MODE == 1 ? __ldg(drow + p) : 0.f);
+      for (int p = p0 + threadIdx.x; p < p1; p += BN_THREADS)
+        acc(to_f32(__ldg(row + p)), MODE == 1 ? to_f32(__ldg(drow + p)) : 0.f);
     }
   }
   const double t0 = block_sum_double((double)a0, s_red);
@@ -116,7 +120,8 @@ __device__ __forceinline__ void sum_partials(const double *__restrict__ partial,
   for (int s = 0; s < splits; ++s) { s1 += partial[((size_t)c * splits + s) * 2]; s2 += partial[((size_t)c * splits + s) * 2 + 1]; }
 }
 
-__global__ void bn_finalize_forward_kernel(const float *__restrict__ y, const double *__restrict__ partial, int C, int S,
+template <class T>
+__global__ void bn_finalize_forward_kernel(const T *__restrict__ y, const double *__restrict__ partial, int C, int S,
                                            int splits, double M, float eps, float momentum,
                                            float *__restrict__ running_mean, float *__restrict__ running_var,
                                            float *__restrict__ save_mean, float *__restrict__ save_invstd) {
@@ -124,7 +129,7 @@ __global__ void bn_finalize_forward_kernel(const float *__restrict__ y, const do
   if (c >= C) return;
   double s1, s2;
   sum_partials(partial, c, splits, s1, s2);
-  const double K = (double)__ldg(y + (size_t)c * S);
+  const double K = (double)to_f32(__ldg(y + (size_t)c * S));
   const double m1 = s1 / M;
   const double mean = K + m1;
   double var = s2 / M - m1 * m1;
@@ -157,25 +162,25 @@ __global__ void bn_finalize_backward_kernel(const double *__restrict__ partial, 
 }
 
 // grid (position tiles, B*C).  MODE 0: z = relu(bn(y)).  MODE 1: dy from dz, y and the channel sums.
-template <int MODE, bool VEC>
-__global__ void __launch_bounds__(BN_THREADS) bn_apply_kernel(const float *__restrict__ y, const float *__restrict__ dz,
+template <class T, int MODE, bool VEC>
+__global__ void __launch_bounds__(BN_THREADS) bn_apply_kernel(const T *__restrict__ y, const T *__restrict__ dz,
                                                                const float *__restrict__ gamma, const float *__restrict__ beta,
                                                                const float *__restrict__ mean, const float *__restrict__ invstd,
                                                                const float *__restrict__ dgamma, const float *__restrict__ dbeta,
-                                                               int C, int S, float inv_M, float *__restrict__ out) {
+                                                               int C, int S, float inv_M, T *__restrict__ out) {
   const int rowi = blockIdx.y;
   const int c = rowi % C;
   const float mu = __ldg(mean + c), is = __ldg(invstd + c), g = __ldg(gamma + c), bt = __ldg(beta + c);
   float k0 = 0.f, k1 = 0.f, gs = 0.f;
   if (MODE == 1) { k0 = __ldg(dbeta + c) * inv_M; k1 = __ldg(dgamma + c) * inv_M; gs = g * is; }
-  const float *row = y + (size_t)rowi * S;
-  const float *drow = MODE == 1 ? dz + (size_t)rowi * S : nullptr;
-  float *orow = out + (size_t)rowi * S;
+  const T *row = y + (size_t)rowi * S;
+  const T *drow = MODE == 1 ? dz + (size_t)rowi * S : nullptr;
+  T *orow = out + (size_t)rowi * S;
   auto f = [&](float yv, float dv) -> float {
     const float xh = (yv - mu) * is;
     const float z = fmaf(xh, g, bt);
     if (MODE == 0) return fmaxf(z, 0.f);
-    const float dm = z > 0.f ? dv : 0.f;
+    const float dm = stored<T>(z) > 0.f ? dv : 0.f;
     return gs * ((dm - k0) - xh * k1);
   };
   const int tile = BN_THREADS * 4 * BN_UNR;
@@ -186,8 +191,8 @@ __global__ void __launch_bounds__(BN_THREADS) bn_apply_kernel(const float *__res
     for (int u = 0; u < BN_UNR; ++u) {
       const int p = base + u * BN_THREADS * 4;
       if (p < S) {
-        v[u] = __ldg(reinterpret_cast<const float4 *>(row + p));
-        if (MODE == 1) d[u] = __ldg(reinterpret_cast<const float4 *>(drow + p));
+        v[u] = ldg4(row + p);
+        if (MODE == 1) d[u] = ldg4(drow + p);
       }
     }
 #pragma unroll
@@ -197,12 +202,12 @@ __global__ void __launch_bounds__(BN_THREADS) bn_apply_kernel(const float *__res
         float4 o;
         o.x = f(v[u].x, MODE == 1 ? d[u].x : 0.f); o.y = f(v[u].y, MODE == 1 ? d[u].y : 0.f);
         o.z = f(v[u].z, MODE == 1 ? d[u].z : 0.f); o.w = f(v[u].w, MODE == 1 ? d[u].w : 0.f);
-        *reinterpret_cast<float4 *>(orow + p) = o;
+        st4(orow + p, o);
       }
     }
   } else {
     for (int p = blockIdx.x * tile + threadIdx.x; p < min(S, (int)(blockIdx.x + 1) * tile); p += BN_THREADS)
-      orow[p] = f(__ldg(row + p), MODE == 1 ? __ldg(drow + p) : 0.f);
+      orow[p] = from_f32<T>(f(to_f32(__ldg(row + p)), MODE == 1 ? to_f32(__ldg(drow + p)) : 0.f));
   }
 }
 
@@ -211,9 +216,12 @@ struct BnPlan {
   bool vec;
 };
 
+// the vector kernels move four elements of T per access: S % 4 == 0 and 4 * sizeof(T)-byte aligned rows
+template <class T>
 static BnPlan plan_bn(const void *a, const void *b, const void *c, int C, int S) {
   BnPlan p;
-  p.vec = (S % 4 == 0) && ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c)) & 15) == 0;
+  p.vec = (S % 4 == 0) && ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) |
+                            reinterpret_cast<uintptr_t>(c)) & (4 * sizeof(T) - 1)) == 0;
   int splits = ceil_div(4 * kNumSMs, C);                       // ~4 CTAs per SM in total
   splits = max(1, min(min(splits, BN_MAX_SPLITS), ceil_div(S, BN_THREADS * 4)));
   int chunk = ceil_div(S, splits);
@@ -229,21 +237,22 @@ static BnPlan plan_bn(const void *a, const void *b, const void *c, int C, int S)
 // never written: the forward emits the pooled (B,C,npoint) tensor, the winning slot and the pre-BN value at
 // that slot; the backward needs one pass (read y, write dy) because the incoming gradient is non-zero at one
 // slot per group only, so the channel sums come from (B,C,npoint) data.
-// A group of NS contiguous floats is handled by NS/4 adjacent lanes (one float4 each): fully coalesced.
+// A group of NS contiguous elements is handled by NS/4 adjacent lanes (four each): fully coalesced.
 // Ties keep the lowest slot, like ATen's max_pool2d (strict '>'), which matters because ball-query padding
-// repeats the first neighbour.
+// repeats the first neighbour.  With bf16 storage the candidates are compared after rounding to bf16, so two slots
+// that differ only below bf16 resolution tie and the lower one wins, as in max_pool2d on the rounded tensor.
 // ----------------------------------------------------------------------------------------------------
 constexpr int BP_UNR = 4;
 
-template <int NS>
-__global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const float *__restrict__ y,
+template <class T, int NS>
+__global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const T *__restrict__ y,
                                                                        const float *__restrict__ gamma,
                                                                        const float *__restrict__ beta,
                                                                        const float *__restrict__ mean,
                                                                        const float *__restrict__ invstd, int C, int np,
-                                                                       float *__restrict__ pooled,
+                                                                       T *__restrict__ pooled,
                                                                        uint8_t *__restrict__ argmax,
-                                                                       float *__restrict__ ymax) {
+                                                                       T *__restrict__ ymax) {
   constexpr int LPG = NS / 4;                 // lanes per group
   constexpr int GPW = 32 / LPG;               // groups per warp per step
   const int rowi = blockIdx.y, c = rowi % C;
@@ -251,12 +260,12 @@ __global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const floa
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int sub = lane % LPG, gl = lane / LPG;
   const int j0 = (blockIdx.x * (BN_THREADS / 32) + warp) * GPW * BP_UNR + gl;
-  const float *row = y + (size_t)rowi * np * NS;
+  const T *row = y + (size_t)rowi * np * NS;
   float4 v[BP_UNR];
 #pragma unroll
   for (int u = 0; u < BP_UNR; ++u) {
     const int j = j0 + u * GPW;
-    if (j < np) v[u] = __ldg(reinterpret_cast<const float4 *>(row + (size_t)j * NS + sub * 4));
+    if (j < np) v[u] = ldg4(row + (size_t)j * NS + sub * 4);
   }
 #pragma unroll
   for (int u = 0; u < BP_UNR; ++u) {
@@ -267,7 +276,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const floa
     int bi = 0;
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      const float z = ok ? fmaf((e[q] - mu) * is, g, bt) : 0.f;
+      const float z = ok ? stored<T>(fmaf((e[q] - mu) * is, g, bt)) : 0.f;
       if (z > bz) { bz = z; bi = sub * 4 + q; by = e[q]; }
     }
 #pragma unroll
@@ -279,18 +288,18 @@ __global__ void __launch_bounds__(BN_THREADS) bn_relu_pool_fwd_kernel(const floa
     }
     if (ok && sub == 0) {
       const size_t o = (size_t)rowi * np + j;
-      pooled[o] = fmaxf(bz, 0.f);
+      pooled[o] = from_f32<T>(fmaxf(bz, 0.f));
       argmax[o] = (uint8_t)bi;
-      ymax[o] = by;
+      ymax[o] = from_f32<T>(by);
     }
   }
 }
 
 // one CTA per channel: dbeta = sum dm, dgamma = sum dm * xhat over the (B, npoint) winners; ROW as in
 // bn_finalize_backward_kernel
-template <bool ROW>
+template <class T, bool ROW>
 __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(
-    const float *__restrict__ dpool, const float *__restrict__ ymax, const float *__restrict__ gamma,
+    const T *__restrict__ dpool, const T *__restrict__ ymax, const float *__restrict__ gamma,
     const float *__restrict__ beta, const float *__restrict__ mean, const float *__restrict__ invstd, int B, int C,
     int np, float *__restrict__ dgamma, float *__restrict__ dbeta, double M, double *__restrict__ row) {
   __shared__ double s_red[BN_THREADS / 32];
@@ -300,8 +309,8 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(
   for (int b = 0; b < B; ++b) {
     const size_t base = ((size_t)b * C + c) * np;
     for (int j = threadIdx.x; j < np; j += BN_THREADS) {
-      const float xh = (__ldg(ymax + base + j) - mu) * is;
-      const float dm = fmaf(xh, g, bt) > 0.f ? __ldg(dpool + base + j) : 0.f;
+      const float xh = (to_f32(__ldg(ymax + base + j)) - mu) * is;
+      const float dm = stored<T>(fmaf(xh, g, bt)) > 0.f ? to_f32(__ldg(dpool + base + j)) : 0.f;
       a0 += dm;
       a1 = fmaf(dm, xh, a1);
     }
@@ -319,12 +328,12 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_reduce_kernel(
   }
 }
 
-template <int NS>
+template <class T, int NS>
 __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
-    const float *__restrict__ y, const float *__restrict__ dpool, const uint8_t *__restrict__ argmax,
-    const float *__restrict__ ymax, const float *__restrict__ gamma, const float *__restrict__ beta,
+    const T *__restrict__ y, const T *__restrict__ dpool, const uint8_t *__restrict__ argmax,
+    const T *__restrict__ ymax, const float *__restrict__ gamma, const float *__restrict__ beta,
     const float *__restrict__ mean, const float *__restrict__ invstd, const float *__restrict__ dgamma,
-    const float *__restrict__ dbeta, int C, int np, float inv_M, float *__restrict__ dy) {
+    const float *__restrict__ dbeta, int C, int np, float inv_M, T *__restrict__ dy) {
   constexpr int LPG = NS / 4;
   constexpr int GPW = 32 / LPG;
   const int rowi = blockIdx.y, c = rowi % C;
@@ -333,8 +342,8 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int sub = lane % LPG, gl = lane / LPG;
   const int j0 = (blockIdx.x * (BN_THREADS / 32) + warp) * GPW * BP_UNR + gl;
-  const float *row = y + (size_t)rowi * np * NS;
-  float *orow = dy + (size_t)rowi * np * NS;
+  const T *row = y + (size_t)rowi * np * NS;
+  T *orow = dy + (size_t)rowi * np * NS;
   float4 v[BP_UNR];
   float dp[BP_UNR], ym[BP_UNR];
   int am[BP_UNR];
@@ -342,10 +351,10 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
   for (int u = 0; u < BP_UNR; ++u) {
     const int j = j0 + u * GPW;
     if (j < np) {
-      v[u] = __ldg(reinterpret_cast<const float4 *>(row + (size_t)j * NS + sub * 4));
+      v[u] = ldg4(row + (size_t)j * NS + sub * 4);
       const size_t o = (size_t)rowi * np + j;
-      dp[u] = __ldg(dpool + o);
-      ym[u] = __ldg(ymax + o);
+      dp[u] = to_f32(__ldg(dpool + o));
+      ym[u] = to_f32(__ldg(ymax + o));
       am[u] = (int)__ldg(argmax + o);
     }
   }
@@ -353,7 +362,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
   for (int u = 0; u < BP_UNR; ++u) {
     const int j = j0 + u * GPW;
     if (j >= np) continue;
-    const float dwin = fmaf((ym[u] - mu) * is, g, bt) > 0.f ? dp[u] : 0.f;
+    const float dwin = stored<T>(fmaf((ym[u] - mu) * is, g, bt)) > 0.f ? dp[u] : 0.f;
     const float e[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
     float o4[4];
 #pragma unroll
@@ -362,7 +371,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
       const float dm = (sub * 4 + q == am[u]) ? dwin : 0.f;
       o4[q] = gs * ((dm - k0) - xh * k1);
     }
-    *reinterpret_cast<float4 *>(orow + (size_t)j * NS + sub * 4) = make_float4(o4[0], o4[1], o4[2], o4[3]);
+    st4(orow + (size_t)j * NS + sub * 4, make_float4(o4[0], o4[1], o4[2], o4[3]));
   }
 }
 
@@ -382,13 +391,14 @@ __global__ void __launch_bounds__(BN_THREADS) bn_pool_bwd_apply_kernel(
 // ----------------------------------------------------------------------------------------------------
 
 // forward, local: (n, mean, M2) from the shifted partial sums s1 = sum (x-K), s2 = sum (x-K)^2 of bn_reduce_kernel<0>
-__global__ void bn_sync_moments_kernel(const float *__restrict__ y, const double *__restrict__ partial, int C, int S,
+template <class T>
+__global__ void bn_sync_moments_kernel(const T *__restrict__ y, const double *__restrict__ partial, int C, int S,
                                        int splits, double M, double *__restrict__ row) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
   double s1, s2;
   sum_partials(partial, c, splits, s1, s2);
-  const double K = (double)__ldg(y + (size_t)c * S);
+  const double K = (double)to_f32(__ldg(y + (size_t)c * S));
   const double m1 = s1 / M;
   double m2 = s2 - s1 * m1;
   if (m2 < 0.0) m2 = 0.0;
@@ -471,11 +481,12 @@ static int check_workspace(const char *what, const void *workspace, size_t works
   return SPC_OK;
 }
 
-// the pool kernels exist for nsample 16, 32 and 64, and read y and write dy with 16-byte accesses
+// the pool kernels exist for nsample 16, 32 and 64, and read y and write dy four elements of T at a time
+template <class T>
 static int check_pool(const char *what, int nsample, const void *y, const void *dy) {
   if (!(nsample == 16 || nsample == 32 || nsample == 64) ||
-      ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & 15)) {
-    set_error("%s: nsample=%d not in {16,32,64} or tensors not 16-byte aligned", what, nsample);
+      ((reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(dy)) & (4 * sizeof(T) - 1))) {
+    set_error("%s: nsample=%d not in {16,32,64} or tensors not %d-byte aligned", what, nsample, (int)(4 * sizeof(T)));
     return SPC_ERR_UNSUPPORTED;
   }
   return SPC_OK;
@@ -485,27 +496,27 @@ static int check_pool(const char *what, int nsample, const void *y, const void *
 // per slice of at most 65535 / C batch rows: one launch whenever B*C <= 65535.
 static int sync_batch_slice(int C) { return max(1, 65535 / C); }
 
-template <int MODE>
-static void launch_reduce(const BnPlan &p, const float *y, const float *dz, const float *gamma, const float *beta,
+template <int MODE, class T>
+static void launch_reduce(const BnPlan &p, const T *y, const T *dz, const float *gamma, const float *beta,
                           const float *mean, const float *invstd, int B, int C, int S, double *partial,
                           cudaStream_t stream) {
   const dim3 grid(p.splits, C);
-  if (p.vec) bn_reduce_kernel<MODE, true><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
-  else bn_reduce_kernel<MODE, false><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
+  if (p.vec) bn_reduce_kernel<T, MODE, true><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
+  else bn_reduce_kernel<T, MODE, false><<<grid, BN_THREADS, 0, stream>>>(y, dz, gamma, beta, mean, invstd, B, C, S, p.chunk, partial);
 }
 
 // MODE 0: out = z (dz, dgamma, dbeta unused).  MODE 1: out = dy with k0 = dbeta * inv_M, k1 = dgamma * inv_M.
-template <int MODE>
-static void launch_apply(bool vec, const float *y, const float *dz, const float *gamma, const float *beta,
+template <int MODE, class T>
+static void launch_apply(bool vec, const T *y, const T *dz, const float *gamma, const float *beta,
                          const float *mean, const float *invstd, const float *dgamma, const float *dbeta, int B, int C,
-                         int S, float inv_M, float *out, cudaStream_t stream) {
+                         int S, float inv_M, T *out, cudaStream_t stream) {
   const int slice = sync_batch_slice(C);
   for (int b0 = 0; b0 < B; b0 += slice) {
     const size_t off = (size_t)b0 * C * S;
-    const float *dzs = MODE == 1 ? dz + off : nullptr;
+    const T *dzs = MODE == 1 ? dz + off : nullptr;
     const dim3 grid(ceil_div(S, BN_THREADS * 4 * BN_UNR), min(slice, B - b0) * C);
-    if (vec) bn_apply_kernel<MODE, true><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
-    else bn_apply_kernel<MODE, false><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
+    if (vec) bn_apply_kernel<T, MODE, true><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
+    else bn_apply_kernel<T, MODE, false><<<grid, BN_THREADS, 0, stream>>>(y + off, dzs, gamma, beta, mean, invstd, dgamma, dbeta, C, S, inv_M, out + off);
   }
 }
 
@@ -522,64 +533,66 @@ static int pool_tiles(int npoint, int nsample) {
   return ceil_div(npoint, (BN_THREADS / 32) * (32 / (nsample / 4)) * BP_UNR);
 }
 
-static void launch_pool_fwd(const float *y, const float *gamma, const float *beta, const float *mean,
-                            const float *invstd, int B, int C, int npoint, int nsample, float *pooled, uint8_t *argmax,
-                            float *ymax, cudaStream_t stream) {
+template <class T>
+static void launch_pool_fwd(const T *y, const float *gamma, const float *beta, const float *mean,
+                            const float *invstd, int B, int C, int npoint, int nsample, T *pooled, uint8_t *argmax,
+                            T *ymax, cudaStream_t stream) {
   const int slice = sync_batch_slice(C);
   for (int b0 = 0; b0 < B; b0 += slice) {
     const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
     const dim3 grid(pool_tiles(npoint, nsample), min(slice, B - b0) * C);
     dispatch_nsample(nsample, [&](auto ns) {
-      bn_relu_pool_fwd_kernel<decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
+      bn_relu_pool_fwd_kernel<T, decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
           y + yo, gamma, beta, mean, invstd, C, npoint, pooled + po, argmax + po, ymax + po);
     });
   }
 }
 
 // dy from dpool, with k0 = dbeta * inv_M, k1 = dgamma * inv_M
-static void launch_pool_bwd(const float *y, const float *dpool, const uint8_t *argmax, const float *ymax,
+template <class T>
+static void launch_pool_bwd(const T *y, const T *dpool, const uint8_t *argmax, const T *ymax,
                             const float *gamma, const float *beta, const float *mean, const float *invstd,
                             const float *dgamma, const float *dbeta, int B, int C, int npoint, int nsample, float inv_M,
-                            float *dy, cudaStream_t stream) {
+                            T *dy, cudaStream_t stream) {
   const int slice = sync_batch_slice(C);
   for (int b0 = 0; b0 < B; b0 += slice) {
     const size_t po = (size_t)b0 * C * npoint, yo = po * nsample;
     const dim3 grid(pool_tiles(npoint, nsample), min(slice, B - b0) * C);
     dispatch_nsample(nsample, [&](auto ns) {
-      bn_pool_bwd_apply_kernel<decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
+      bn_pool_bwd_apply_kernel<T, decltype(ns)::value><<<grid, BN_THREADS, 0, stream>>>(
           y + yo, dpool + po, argmax + po, ymax + po, gamma, beta, mean, invstd, dgamma, dbeta, C, npoint, inv_M, dy + yo);
     });
   }
 }
 
 // ---- plain passes -------------------------------------------------------------------------------------------------
-extern "C" int spc_bn_relu_train_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
-                                         float eps, float momentum, float *running_mean, float *running_var,
-                                         float *z, float *save_mean, float *save_invstd, void *workspace,
-                                         size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_train_forward(const T *y, const float *gamma, const float *beta, int B, int C, int S, float eps,
+                                 float momentum, float *running_mean, float *running_var, T *z, float *save_mean,
+                                 float *save_invstd, void *workspace, size_t workspace_bytes, void *stream_) {
   if (const int e = check_bn("bn_relu_forward", B, 1, C, S, 1, 1, {y, z}, {gamma, beta, save_mean, save_invstd})) return e;
   if (const int e = check_workspace("bn_relu_forward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, z, y, C, S);
-  launch_reduce<0>(p, y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
+  const BnPlan p = plan_bn<T>(y, z, y, C, S);
+  launch_reduce<0>(p, y, (const T *)nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
   bn_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, eps, momentum,
                                                                    running_mean, running_var, save_mean, save_invstd);
-  launch_apply<0>(p.vec, y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
+  launch_apply<0>(p.vec, y, (const T *)nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
   SPC_LAUNCH_CHECK("bn_relu_train_forward");
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_train_backward(const float *dz, const float *y, const float *gamma, const float *beta,
-                                          const float *save_mean, const float *save_invstd, int B, int C, int S,
-                                          float *dy, float *dgamma, float *dbeta, void *workspace,
-                                          size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_train_backward(const T *dz, const T *y, const float *gamma, const float *beta, const float *save_mean,
+                                  const float *save_invstd, int B, int C, int S, T *dy, float *dgamma, float *dbeta,
+                                  void *workspace, size_t workspace_bytes, void *stream_) {
   if (const int e = check_bn("bn_relu_backward", B, 1, C, S, 1, 1, {dz, y, dy},
                              {gamma, beta, save_mean, save_invstd, dgamma, dbeta})) return e;
   if (const int e = check_workspace("bn_relu_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, dz, dy, C, S);
+  const BnPlan p = plan_bn<T>(y, dz, dy, C, S);
   launch_reduce<1>(p, y, dz, gamma, beta, save_mean, save_invstd, B, C, S, partial, stream);
   bn_finalize_backward_kernel<false><<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, dgamma, dbeta, 0.0, nullptr);
   const float inv_M = (float)(1.0 / ((double)B * S));
@@ -588,20 +601,20 @@ extern "C" int spc_bn_relu_train_backward(const float *dz, const float *y, const
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_maxpool_train_forward(const float *y, const float *gamma, const float *beta, int B, int C,
-                                                 int npoint, int nsample, float eps, float momentum,
-                                                 float *running_mean, float *running_var, float *pooled,
-                                                 uint8_t *argmax, float *ymax, float *save_mean, float *save_invstd,
-                                                 void *workspace, size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_maxpool_train_forward(const T *y, const float *gamma, const float *beta, int B, int C, int npoint,
+                                         int nsample, float eps, float momentum, float *running_mean,
+                                         float *running_var, T *pooled, uint8_t *argmax, T *ymax, float *save_mean,
+                                         float *save_invstd, void *workspace, size_t workspace_bytes, void *stream_) {
   if (const int e = check_bn("bn_relu_maxpool_forward", B, 1, C, npoint, nsample, 1, {y, pooled, argmax, ymax},
                              {gamma, beta, save_mean, save_invstd})) return e;
-  if (const int e = check_pool("bn_relu_maxpool_forward", nsample, y, nullptr)) return e;
+  if (const int e = check_pool<T>("bn_relu_maxpool_forward", nsample, y, nullptr)) return e;
   if (const int e = check_workspace("bn_relu_maxpool_forward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   const int S = npoint * nsample;
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, y, y, C, S);     // vector: y is 16-byte aligned and S a multiple of 16
-  launch_reduce<0>(p, y, nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
+  const BnPlan p = plan_bn<T>(y, y, y, C, S);     // vector: y is aligned (check_pool) and S a multiple of 16
+  launch_reduce<0>(p, y, (const T *)nullptr, gamma, beta, nullptr, nullptr, B, C, S, partial, stream);
   bn_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, eps, momentum,
                                                                    running_mean, running_var, save_mean, save_invstd);
   launch_pool_fwd(y, gamma, beta, save_mean, save_invstd, B, C, npoint, nsample, pooled, argmax, ymax, stream);
@@ -609,17 +622,17 @@ extern "C" int spc_bn_relu_maxpool_train_forward(const float *y, const float *ga
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint8_t *argmax, const float *ymax,
-                                                  const float *y, const float *gamma, const float *beta,
-                                                  const float *save_mean, const float *save_invstd, int B, int C,
-                                                  int npoint, int nsample, float *dy, float *dgamma, float *dbeta,
-                                                  void *stream_) {
+template <class T>
+static int bn_relu_maxpool_train_backward(const T *dpool, const uint8_t *argmax, const T *ymax, const T *y,
+                                          const float *gamma, const float *beta, const float *save_mean,
+                                          const float *save_invstd, int B, int C, int npoint, int nsample, T *dy,
+                                          float *dgamma, float *dbeta, void *stream_) {
   if (const int e = check_bn("bn_relu_maxpool_backward", B, 1, C, npoint, nsample, 1, {dpool, argmax, ymax, y, dy},
                              {gamma, beta, save_mean, save_invstd, dgamma, dbeta})) return e;
-  if (const int e = check_pool("bn_relu_maxpool_backward", nsample, y, dy)) return e;
+  if (const int e = check_pool<T>("bn_relu_maxpool_backward", nsample, y, dy)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
-  bn_pool_bwd_reduce_kernel<false><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
-                                                                 npoint, dgamma, dbeta, 0.0, nullptr);
+  bn_pool_bwd_reduce_kernel<T, false><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
+                                                                    npoint, dgamma, dbeta, 0.0, nullptr);
   const float inv_M = (float)(1.0 / ((double)B * npoint * nsample));
   launch_pool_bwd(y, dpool, argmax, ymax, gamma, beta, save_mean, save_invstd, dgamma, dbeta, B, C, npoint, nsample,
                   inv_M, dy, stream);
@@ -629,8 +642,9 @@ extern "C" int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint
 
 // ---- synchronised passes (see BN_SYNC_K above) --------------------------------------------------------------------
 // Each takes any local B >= 0; a rank with B = 0 contributes a row with n = 0, which the combinations skip.
-extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, double *stats, void *workspace,
-                                      size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_sync_stats(const T *y, int B, int C, int S, double *stats, void *workspace, size_t workspace_bytes,
+                              void *stream_) {
   if (const int e = check_bn("bn_relu_sync_stats", B, 0, C, S, 1, 1, {y}, {stats})) return e;
   if (const int e = check_workspace("bn_relu_sync_stats", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
@@ -639,32 +653,33 @@ extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, doubl
     return SPC_OK;
   }
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, y, y, C, S);
-  launch_reduce<0>(p, y, nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, partial, stream);
+  const BnPlan p = plan_bn<T>(y, y, y, C, S);
+  launch_reduce<0>(p, y, (const T *)nullptr, nullptr, nullptr, nullptr, nullptr, B, C, S, partial, stream);
   bn_sync_moments_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(y, partial, C, S, p.splits, (double)B * S, stats);
   SPC_LAUNCH_CHECK("bn_relu_sync_stats");
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
-                                        int world, const double *stats_all, float eps, float momentum,
-                                        float *running_mean, float *running_var, float *z, float *save_mean,
-                                        float *save_invstd, void *stream_) {
+template <class T>
+static int bn_relu_sync_forward(const T *y, const float *gamma, const float *beta, int B, int C, int S, int world,
+                                const double *stats_all, float eps, float momentum, float *running_mean,
+                                float *running_var, T *z, float *save_mean, float *save_invstd, void *stream_) {
   if (const int e = check_bn("bn_relu_sync_forward", B, 0, C, S, 1, world, {y, z},
                              {gamma, beta, stats_all, save_mean, save_invstd})) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
                                                                         running_var, save_mean, save_invstd);
-  const BnPlan p = plan_bn(y, z, y, C, S);
-  launch_apply<0>(p.vec, y, nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
+  const BnPlan p = plan_bn<T>(y, z, y, C, S);
+  launch_apply<0>(p.vec, y, (const T *)nullptr, gamma, beta, save_mean, save_invstd, nullptr, nullptr, B, C, S, 0.f, z, stream);
   SPC_LAUNCH_CHECK("bn_relu_sync_forward");
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y, const float *gamma, const float *beta,
-                                                const float *save_mean, const float *save_invstd, int B, int C, int S,
-                                                float *dgamma, float *dbeta, double *stats, void *workspace,
-                                                size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_sync_backward_reduce(const T *dz, const T *y, const float *gamma, const float *beta,
+                                        const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                        float *dgamma, float *dbeta, double *stats, void *workspace,
+                                        size_t workspace_bytes, void *stream_) {
   if (const int e = check_bn("bn_relu_sync_backward_reduce", B, 0, C, S, 1, 1, {dz, y},
                              {gamma, beta, save_mean, save_invstd, dgamma, dbeta, stats})) return e;
   if (const int e = check_workspace("bn_relu_sync_backward_reduce", workspace, workspace_bytes, C)) return e;
@@ -676,7 +691,7 @@ extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y,
     return SPC_OK;
   }
   double *partial = reinterpret_cast<double *>(workspace);
-  const BnPlan p = plan_bn(y, dz, dz, C, S);
+  const BnPlan p = plan_bn<T>(y, dz, dz, C, S);
   launch_reduce<1>(p, y, dz, gamma, beta, save_mean, save_invstd, B, C, S, partial, stream);
   bn_finalize_backward_kernel<true><<<ceil_div(C, 128), 128, 0, stream>>>(partial, C, p.splits, dgamma, dbeta,
                                                                           (double)B * S, stats);
@@ -684,31 +699,31 @@ extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y,
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_sync_backward(const float *dz, const float *y, const float *gamma, const float *beta,
-                                         const float *save_mean, const float *save_invstd, int B, int C, int S,
-                                         int world, const double *stats_all, float *dy, void *workspace,
-                                         size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_sync_backward(const T *dz, const T *y, const float *gamma, const float *beta, const float *save_mean,
+                                 const float *save_invstd, int B, int C, int S, int world, const double *stats_all,
+                                 T *dy, void *workspace, size_t workspace_bytes, void *stream_) {
   if (const int e = check_bn("bn_relu_sync_backward", B, 0, C, S, 1, world, {dz, y, dy},
                              {gamma, beta, save_mean, save_invstd, stats_all})) return e;
   if (const int e = check_workspace("bn_relu_sync_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
   bn_sync_combine_backward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, k0, k1);
-  const BnPlan p = plan_bn(y, dz, dy, C, S);
+  const BnPlan p = plan_bn<T>(y, dz, dy, C, S);
   launch_apply<1>(p.vec, y, dz, gamma, beta, save_mean, save_invstd, k1, k0, B, C, S, 1.f, dy, stream);
   SPC_LAUNCH_CHECK("bn_relu_sync_backward");
   return SPC_OK;
 }
 
-// Max-pool variant.  Its statistics phase is spc_bn_relu_sync_stats with S = npoint * nsample.
-extern "C" int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C,
-                                                int npoint, int nsample, int world, const double *stats_all,
-                                                float eps, float momentum, float *running_mean, float *running_var,
-                                                float *pooled, uint8_t *argmax, float *ymax, float *save_mean,
-                                                float *save_invstd, void *stream_) {
+// Max-pool variant.  Its statistics phase is bn_relu_sync_stats with S = npoint * nsample.
+template <class T>
+static int bn_relu_maxpool_sync_forward(const T *y, const float *gamma, const float *beta, int B, int C, int npoint,
+                                        int nsample, int world, const double *stats_all, float eps, float momentum,
+                                        float *running_mean, float *running_var, T *pooled, uint8_t *argmax, T *ymax,
+                                        float *save_mean, float *save_invstd, void *stream_) {
   if (const int e = check_bn("bn_relu_maxpool_sync_forward", B, 0, C, npoint, nsample, world, {y, pooled, argmax, ymax},
                              {gamma, beta, stats_all, save_mean, save_invstd})) return e;
-  if (const int e = check_pool("bn_relu_maxpool_sync_forward", nsample, y, nullptr)) return e;
+  if (const int e = check_pool<T>("bn_relu_maxpool_sync_forward", nsample, y, nullptr)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   bn_sync_finalize_forward_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats_all, world, C, eps, momentum, running_mean,
                                                                         running_var, save_mean, save_invstd);
@@ -717,28 +732,29 @@ extern "C" int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gam
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_maxpool_sync_backward_reduce(const float *dpool, const float *ymax, const float *gamma,
-                                                        const float *beta, const float *save_mean,
-                                                        const float *save_invstd, int B, int C, int npoint,
-                                                        int nsample, float *dgamma, float *dbeta, double *stats,
-                                                        void *stream_) {
+template <class T>
+static int bn_relu_maxpool_sync_backward_reduce(const T *dpool, const T *ymax, const float *gamma, const float *beta,
+                                                const float *save_mean, const float *save_invstd, int B, int C,
+                                                int npoint, int nsample, float *dgamma, float *dbeta, double *stats,
+                                                void *stream_) {
   if (const int e = check_bn("bn_relu_maxpool_sync_backward_reduce", B, 0, C, npoint, nsample, 1, {dpool, ymax},
                              {gamma, beta, save_mean, save_invstd, dgamma, dbeta, stats})) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
-  bn_pool_bwd_reduce_kernel<true><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
-                                                                npoint, dgamma, dbeta, (double)B * npoint * nsample, stats);
+  bn_pool_bwd_reduce_kernel<T, true><<<C, BN_THREADS, 0, stream>>>(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C,
+                                                                   npoint, dgamma, dbeta, (double)B * npoint * nsample, stats);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward_reduce");
   return SPC_OK;
 }
 
-extern "C" int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8_t *argmax, const float *ymax,
-                                                 const float *y, const float *gamma, const float *beta,
-                                                 const float *save_mean, const float *save_invstd, int B, int C,
-                                                 int npoint, int nsample, int world, const double *stats_all,
-                                                 float *dy, void *workspace, size_t workspace_bytes, void *stream_) {
+template <class T>
+static int bn_relu_maxpool_sync_backward(const T *dpool, const uint8_t *argmax, const T *ymax, const T *y,
+                                         const float *gamma, const float *beta, const float *save_mean,
+                                         const float *save_invstd, int B, int C, int npoint, int nsample, int world,
+                                         const double *stats_all, T *dy, void *workspace, size_t workspace_bytes,
+                                         void *stream_) {
   if (const int e = check_bn("bn_relu_maxpool_sync_backward", B, 0, C, npoint, nsample, world,
                              {dpool, argmax, ymax, y, dy}, {gamma, beta, save_mean, save_invstd, stats_all})) return e;
-  if (const int e = check_pool("bn_relu_maxpool_sync_backward", nsample, y, dy)) return e;
+  if (const int e = check_pool<T>("bn_relu_maxpool_sync_backward", nsample, y, dy)) return e;
   if (const int e = check_workspace("bn_relu_maxpool_sync_backward", workspace, workspace_bytes, C)) return e;
   cudaStream_t stream = (cudaStream_t)stream_;
   float *k0 = reinterpret_cast<float *>(workspace), *k1 = k0 + C;
@@ -747,4 +763,180 @@ extern "C" int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8
                   stream);
   SPC_LAUNCH_CHECK("bn_relu_maxpool_sync_backward");
   return SPC_OK;
+}
+
+// ---- C entry points: fp32 storage, and bf16 storage (the void pointers are __nv_bfloat16 tensors) ------------------
+#define BF(p) static_cast<const bf16 *>(p)
+#define BFW(p) static_cast<bf16 *>(p)
+
+extern "C" int spc_bn_relu_train_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
+                                         float eps, float momentum, float *running_mean, float *running_var,
+                                         float *z, float *save_mean, float *save_invstd, void *workspace,
+                                         size_t workspace_bytes, void *stream) {
+  return bn_relu_train_forward(y, gamma, beta, B, C, S, eps, momentum, running_mean, running_var, z, save_mean,
+                               save_invstd, workspace, workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_train_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C, int S,
+                                              float eps, float momentum, float *running_mean, float *running_var,
+                                              void *z, float *save_mean, float *save_invstd, void *workspace,
+                                              size_t workspace_bytes, void *stream) {
+  return bn_relu_train_forward(BF(y), gamma, beta, B, C, S, eps, momentum, running_mean, running_var, BFW(z), save_mean,
+                               save_invstd, workspace, workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_train_backward(const float *dz, const float *y, const float *gamma, const float *beta,
+                                          const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                          float *dy, float *dgamma, float *dbeta, void *workspace,
+                                          size_t workspace_bytes, void *stream) {
+  return bn_relu_train_backward(dz, y, gamma, beta, save_mean, save_invstd, B, C, S, dy, dgamma, dbeta, workspace,
+                                workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_train_backward_bf16(const void *dz, const void *y, const float *gamma, const float *beta,
+                                               const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                               void *dy, float *dgamma, float *dbeta, void *workspace,
+                                               size_t workspace_bytes, void *stream) {
+  return bn_relu_train_backward(BF(dz), BF(y), gamma, beta, save_mean, save_invstd, B, C, S, BFW(dy), dgamma, dbeta,
+                                workspace, workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_maxpool_train_forward(const float *y, const float *gamma, const float *beta, int B, int C,
+                                                 int npoint, int nsample, float eps, float momentum,
+                                                 float *running_mean, float *running_var, float *pooled,
+                                                 uint8_t *argmax, float *ymax, float *save_mean, float *save_invstd,
+                                                 void *workspace, size_t workspace_bytes, void *stream) {
+  return bn_relu_maxpool_train_forward(y, gamma, beta, B, C, npoint, nsample, eps, momentum, running_mean, running_var,
+                                       pooled, argmax, ymax, save_mean, save_invstd, workspace, workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_maxpool_train_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C,
+                                                      int npoint, int nsample, float eps, float momentum,
+                                                      float *running_mean, float *running_var, void *pooled,
+                                                      uint8_t *argmax, void *ymax, float *save_mean, float *save_invstd,
+                                                      void *workspace, size_t workspace_bytes, void *stream) {
+  return bn_relu_maxpool_train_forward(BF(y), gamma, beta, B, C, npoint, nsample, eps, momentum, running_mean,
+                                       running_var, BFW(pooled), argmax, BFW(ymax), save_mean, save_invstd, workspace,
+                                       workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_maxpool_train_backward(const float *dpool, const uint8_t *argmax, const float *ymax,
+                                                  const float *y, const float *gamma, const float *beta,
+                                                  const float *save_mean, const float *save_invstd, int B, int C,
+                                                  int npoint, int nsample, float *dy, float *dgamma, float *dbeta,
+                                                  void *stream) {
+  return bn_relu_maxpool_train_backward(dpool, argmax, ymax, y, gamma, beta, save_mean, save_invstd, B, C, npoint,
+                                        nsample, dy, dgamma, dbeta, stream);
+}
+extern "C" int spc_bn_relu_maxpool_train_backward_bf16(const void *dpool, const uint8_t *argmax, const void *ymax,
+                                                       const void *y, const float *gamma, const float *beta,
+                                                       const float *save_mean, const float *save_invstd, int B, int C,
+                                                       int npoint, int nsample, void *dy, float *dgamma, float *dbeta,
+                                                       void *stream) {
+  return bn_relu_maxpool_train_backward(BF(dpool), argmax, BF(ymax), BF(y), gamma, beta, save_mean, save_invstd, B, C,
+                                        npoint, nsample, BFW(dy), dgamma, dbeta, stream);
+}
+
+extern "C" int spc_bn_relu_sync_stats(const float *y, int B, int C, int S, double *stats, void *workspace,
+                                      size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_stats(y, B, C, S, stats, workspace, workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_sync_stats_bf16(const void *y, int B, int C, int S, double *stats, void *workspace,
+                                           size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_stats(BF(y), B, C, S, stats, workspace, workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C, int S,
+                                        int world, const double *stats_all, float eps, float momentum,
+                                        float *running_mean, float *running_var, float *z, float *save_mean,
+                                        float *save_invstd, void *stream) {
+  return bn_relu_sync_forward(y, gamma, beta, B, C, S, world, stats_all, eps, momentum, running_mean, running_var, z,
+                              save_mean, save_invstd, stream);
+}
+extern "C" int spc_bn_relu_sync_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C, int S,
+                                             int world, const double *stats_all, float eps, float momentum,
+                                             float *running_mean, float *running_var, void *z, float *save_mean,
+                                             float *save_invstd, void *stream) {
+  return bn_relu_sync_forward(BF(y), gamma, beta, B, C, S, world, stats_all, eps, momentum, running_mean, running_var,
+                              BFW(z), save_mean, save_invstd, stream);
+}
+
+extern "C" int spc_bn_relu_sync_backward_reduce(const float *dz, const float *y, const float *gamma, const float *beta,
+                                                const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                                float *dgamma, float *dbeta, double *stats, void *workspace,
+                                                size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_backward_reduce(dz, y, gamma, beta, save_mean, save_invstd, B, C, S, dgamma, dbeta, stats,
+                                      workspace, workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_sync_backward_reduce_bf16(const void *dz, const void *y, const float *gamma,
+                                                     const float *beta, const float *save_mean,
+                                                     const float *save_invstd, int B, int C, int S, float *dgamma,
+                                                     float *dbeta, double *stats, void *workspace,
+                                                     size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_backward_reduce(BF(dz), BF(y), gamma, beta, save_mean, save_invstd, B, C, S, dgamma, dbeta, stats,
+                                      workspace, workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_sync_backward(const float *dz, const float *y, const float *gamma, const float *beta,
+                                         const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                         int world, const double *stats_all, float *dy, void *workspace,
+                                         size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_backward(dz, y, gamma, beta, save_mean, save_invstd, B, C, S, world, stats_all, dy, workspace,
+                               workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_sync_backward_bf16(const void *dz, const void *y, const float *gamma, const float *beta,
+                                              const float *save_mean, const float *save_invstd, int B, int C, int S,
+                                              int world, const double *stats_all, void *dy, void *workspace,
+                                              size_t workspace_bytes, void *stream) {
+  return bn_relu_sync_backward(BF(dz), BF(y), gamma, beta, save_mean, save_invstd, B, C, S, world, stats_all, BFW(dy),
+                               workspace, workspace_bytes, stream);
+}
+
+extern "C" int spc_bn_relu_maxpool_sync_forward(const float *y, const float *gamma, const float *beta, int B, int C,
+                                                int npoint, int nsample, int world, const double *stats_all,
+                                                float eps, float momentum, float *running_mean, float *running_var,
+                                                float *pooled, uint8_t *argmax, float *ymax, float *save_mean,
+                                                float *save_invstd, void *stream) {
+  return bn_relu_maxpool_sync_forward(y, gamma, beta, B, C, npoint, nsample, world, stats_all, eps, momentum,
+                                      running_mean, running_var, pooled, argmax, ymax, save_mean, save_invstd, stream);
+}
+extern "C" int spc_bn_relu_maxpool_sync_forward_bf16(const void *y, const float *gamma, const float *beta, int B, int C,
+                                                     int npoint, int nsample, int world, const double *stats_all,
+                                                     float eps, float momentum, float *running_mean,
+                                                     float *running_var, void *pooled, uint8_t *argmax, void *ymax,
+                                                     float *save_mean, float *save_invstd, void *stream) {
+  return bn_relu_maxpool_sync_forward(BF(y), gamma, beta, B, C, npoint, nsample, world, stats_all, eps, momentum,
+                                      running_mean, running_var, BFW(pooled), argmax, BFW(ymax), save_mean, save_invstd,
+                                      stream);
+}
+
+extern "C" int spc_bn_relu_maxpool_sync_backward_reduce(const float *dpool, const float *ymax, const float *gamma,
+                                                        const float *beta, const float *save_mean,
+                                                        const float *save_invstd, int B, int C, int npoint,
+                                                        int nsample, float *dgamma, float *dbeta, double *stats,
+                                                        void *stream) {
+  return bn_relu_maxpool_sync_backward_reduce(dpool, ymax, gamma, beta, save_mean, save_invstd, B, C, npoint, nsample,
+                                              dgamma, dbeta, stats, stream);
+}
+extern "C" int spc_bn_relu_maxpool_sync_backward_reduce_bf16(const void *dpool, const void *ymax, const float *gamma,
+                                                             const float *beta, const float *save_mean,
+                                                             const float *save_invstd, int B, int C, int npoint,
+                                                             int nsample, float *dgamma, float *dbeta, double *stats,
+                                                             void *stream) {
+  return bn_relu_maxpool_sync_backward_reduce(BF(dpool), BF(ymax), gamma, beta, save_mean, save_invstd, B, C, npoint,
+                                              nsample, dgamma, dbeta, stats, stream);
+}
+
+extern "C" int spc_bn_relu_maxpool_sync_backward(const float *dpool, const uint8_t *argmax, const float *ymax,
+                                                 const float *y, const float *gamma, const float *beta,
+                                                 const float *save_mean, const float *save_invstd, int B, int C,
+                                                 int npoint, int nsample, int world, const double *stats_all,
+                                                 float *dy, void *workspace, size_t workspace_bytes, void *stream) {
+  return bn_relu_maxpool_sync_backward(dpool, argmax, ymax, y, gamma, beta, save_mean, save_invstd, B, C, npoint,
+                                       nsample, world, stats_all, dy, workspace, workspace_bytes, stream);
+}
+extern "C" int spc_bn_relu_maxpool_sync_backward_bf16(const void *dpool, const uint8_t *argmax, const void *ymax,
+                                                      const void *y, const float *gamma, const float *beta,
+                                                      const float *save_mean, const float *save_invstd, int B, int C,
+                                                      int npoint, int nsample, int world, const double *stats_all,
+                                                      void *dy, void *workspace, size_t workspace_bytes, void *stream) {
+  return bn_relu_maxpool_sync_backward(BF(dpool), argmax, BF(ymax), BF(y), gamma, beta, save_mean, save_invstd, B, C,
+                                       npoint, nsample, world, stats_all, BFW(dy), workspace, workspace_bytes, stream);
 }

@@ -20,5 +20,5 @@ int cuda_fail(cudaError_t e, const char *what) {
 }
 }  // namespace spc
 
-extern "C" int spc_abi_version(void) { return 19; }
+extern "C" int spc_abi_version(void) { return 20; }
 extern "C" const char *spc_last_error(void) { return spc::g_err; }

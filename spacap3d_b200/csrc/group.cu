@@ -17,15 +17,13 @@
 // warp are pre-combined (warp-aggregated atomics, __match_any_sync) before a shared-memory
 // atomic, and rows are flushed with plain coalesced stores (or global atomics when the
 // position range had to be split across CTAs to fill the machine).
+// group_points and its backward are instantiated for float and bf16 storage (common.cuh): bf16 rows are grouped as
+// bf16, and the backward reads a bf16 grad_out and accumulates and writes an fp32 gradient (B,C,N), nsample times
+// smaller than grad_out, so the accumulation logic and the partitions are the same for both.
 #include "common.cuh"
 #include "ptx.cuh"
 
 namespace spc {
-
-__device__ __forceinline__ void st_cs_v4(float *p, float a, float b, float c, float d) {
-  asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d)
-               : "memory");
-}
 
 // ----------------------------------------------------------------------------------------------
 // gather_points:  out[b,c,j] = points[b,c,idx[b,j]]      (tiny: C is 3 in SpaCap3D)
@@ -58,24 +56,25 @@ __global__ void gather_points_grad_kernel(const float *__restrict__ grad_out,
 constexpr int GP_THREADS = 512;
 
 // grid = (position chunks, channel tiles, B).  STAGED: rows in smem, else gathers via LDG.
-template <bool STAGED, bool VEC4>
+template <class T, bool STAGED, bool VEC4>
 __global__ void __launch_bounds__(GP_THREADS) group_points_kernel(
-    const float *__restrict__ points, const int32_t *__restrict__ idx, int C, int N, int S, int CT,
-    int chunk, float *__restrict__ out) {
-  extern __shared__ __align__(128) float s_rows[];  // [CT][N]
+    const T *__restrict__ points, const int32_t *__restrict__ idx, int C, int N, int S, int CT,
+    int chunk, T *__restrict__ out) {
+  extern __shared__ __align__(128) float s_smem[];
+  T *s_rows = reinterpret_cast<T *>(s_smem);        // [CT][N]
   __shared__ __align__(8) uint64_t bar;
   const int b = blockIdx.z;
   const int c0 = blockIdx.y * CT;
   const int ct = min(CT, C - c0);
   const int p0 = blockIdx.x * chunk;
   const int p1 = min(S, p0 + chunk);
-  const float *src = points + ((size_t)b * C + c0) * N;
+  const T *src = points + ((size_t)b * C + c0) * N;
   const int32_t *ix = idx + (size_t)b * S;
-  float *dst = out + ((size_t)b * C + c0) * S;
+  T *dst = out + ((size_t)b * C + c0) * S;
   const int tid = threadIdx.x;
 
   if (STAGED) {
-    const size_t bytes = (size_t)ct * N * sizeof(float);
+    const size_t bytes = (size_t)ct * N * sizeof(T);
     const bool bulk_ok = ((reinterpret_cast<uintptr_t>(src) & 15) == 0) && (bytes % 16 == 0);
     if (bulk_ok) {
       if (tid == 0) { mbarrier_init(&bar, 1); fence_mbarrier_init(); }
@@ -93,7 +92,7 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_kernel(
   }
 
   if (VEC4) {
-    // S % 4 == 0 and chunk % 4 == 0: 4 consecutive positions per thread, 16-byte idx load + store.
+    // S % 4 == 0 and chunk % 4 == 0: 4 consecutive positions per thread, 16-byte idx load, 4 * sizeof(T)-byte store.
     // The index loads of UNR iterations are issued together: with one CTA per SM (a 160 KB row)
     // the loop is otherwise bound by the L2 latency of one idx load per thread.
     constexpr int UNR = 4;
@@ -104,13 +103,13 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_kernel(
       for (int u = 0; u < UNR; ++u) i4[u] = __ldg(reinterpret_cast<const int4 *>(ix + t + u * GP_THREADS * 4));
 #pragma unroll 2
       for (int c = 0; c < ct; ++c) {
-        const float *r = STAGED ? s_rows + (size_t)c * N : src + (size_t)c * N;
+        const T *r = STAGED ? s_rows + (size_t)c * N : src + (size_t)c * N;
 #pragma unroll
         for (int u = 0; u < UNR; ++u) {
-          float a0, a1, a2, a3;
+          T a0, a1, a2, a3;
           if (STAGED) { a0 = r[i4[u].x]; a1 = r[i4[u].y]; a2 = r[i4[u].z]; a3 = r[i4[u].w]; }
           else { a0 = __ldg(r + i4[u].x); a1 = __ldg(r + i4[u].y); a2 = __ldg(r + i4[u].z); a3 = __ldg(r + i4[u].w); }
-          st_cs_v4(dst + (size_t)c * S + t + u * GP_THREADS * 4, a0, a1, a2, a3);
+          st_cs4(dst + (size_t)c * S + t + u * GP_THREADS * 4, a0, a1, a2, a3);
         }
       }
     }
@@ -118,15 +117,15 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_kernel(
       const int4 i4 = __ldg(reinterpret_cast<const int4 *>(ix + t));
 #pragma unroll 4
       for (int c = 0; c < ct; ++c) {
-        float a0, a1, a2, a3;
+        T a0, a1, a2, a3;
         if (STAGED) {
-          const float *r = s_rows + (size_t)c * N;
+          const T *r = s_rows + (size_t)c * N;
           a0 = r[i4.x]; a1 = r[i4.y]; a2 = r[i4.z]; a3 = r[i4.w];
         } else {
-          const float *r = src + (size_t)c * N;
+          const T *r = src + (size_t)c * N;
           a0 = __ldg(r + i4.x); a1 = __ldg(r + i4.y); a2 = __ldg(r + i4.z); a3 = __ldg(r + i4.w);
         }
-        st_cs_v4(dst + (size_t)c * S + t, a0, a1, a2, a3);
+        st_cs4(dst + (size_t)c * S + t, a0, a1, a2, a3);
       }
     }
   } else {
@@ -156,9 +155,9 @@ __device__ __forceinline__ void warp_agg_add(float *row, int i, float v, unsigne
   if ((int)lane == __ffs(peers) - 1) atomicAdd(row + i, sum);
 }
 
-template <bool STAGED>
+template <class T, bool STAGED>
 __global__ void __launch_bounds__(GP_THREADS) group_points_grad_kernel(
-    const float *__restrict__ grad_out, const int32_t *__restrict__ idx, int C, int N, int S,
+    const T *__restrict__ grad_out, const int32_t *__restrict__ idx, int C, int N, int S,
     int CT, int chunk, int use_global_atomics, float *__restrict__ grad_points) {
   extern __shared__ __align__(128) float s_rows[];  // [CT][N] accumulators
   const int b = blockIdx.z;
@@ -166,7 +165,7 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_grad_kernel(
   const int ct = min(CT, C - c0);
   const int p0 = blockIdx.x * chunk;
   const int p1 = min(S, p0 + chunk);
-  const float *g = grad_out + ((size_t)b * C + c0) * S;
+  const T *g = grad_out + ((size_t)b * C + c0) * S;
   const int32_t *ix = idx + (size_t)b * S;
   float *dst = grad_points + ((size_t)b * C + c0) * N;
   const int tid = threadIdx.x;
@@ -185,7 +184,7 @@ __global__ void __launch_bounds__(GP_THREADS) group_points_grad_kernel(
     if (!active) continue;
     const unsigned peers = __match_any_sync(act, i);
     for (int c = 0; c < ct; ++c) {
-      const float v = __ldg(g + (size_t)c * S + t);
+      const float v = to_f32(__ldg(g + (size_t)c * S + t));
       warp_agg_add(STAGED ? s_rows + (size_t)c * N : dst + (size_t)c * N, i, v, peers);
     }
   }
@@ -209,9 +208,10 @@ struct GroupPlan {
   size_t smem;
 };
 
-static GroupPlan plan_group(int B, int C, int N, int S, bool backward) {
+// esz: bytes per staged element (the forward stages rows of its storage type, the backward fp32 accumulators)
+static GroupPlan plan_group(int B, int C, int N, int S, bool backward, size_t esz) {
   GroupPlan g;
-  const size_t row = (size_t)N * sizeof(float);
+  const size_t row = (size_t)N * esz;
   const size_t budget = 200 * 1024;
   g.staged = row <= budget && N > 0;
   if (!g.staged) {
@@ -267,15 +267,16 @@ struct GradPlan {
   size_t smem;
 };
 
-static GradPlan plan_group_grad(int C, int N, int S) {
+// esz: bytes per staged grad_out element (rows of the storage type)
+static GradPlan plan_group_grad(int C, int N, int S, size_t esz) {
   GradPlan g;
   g.H = ceil_div(S, GG_PART_MAX);
   g.Sp = ((ceil_div(S, g.H) + 7) / 8) * 8;     // multiples of 8 keep the uint16 lists 16-byte aligned
   g.H = ceil_div(S, g.Sp);
   g.Np = ((N + 1 + 3) / 4) * 4;                // offsets row stride (16-byte aligned rows)
-  int ct = (int)((64 * 1024) / ((size_t)g.Sp * sizeof(float)));
+  int ct = (int)((64 * 1024) / ((size_t)g.Sp * esz));
   g.CT = max(1, min(min(ct, GG_CT_MAX), C));
-  const size_t rows = (size_t)g.CT * g.Sp * sizeof(float);
+  const size_t rows = (size_t)g.CT * g.Sp * esz;
   const size_t lists = (size_t)g.Sp * sizeof(uint16_t) + (size_t)g.Np * sizeof(int);
   g.lists_smem = rows + lists <= 112 * 1024;   // still two CTAs per SM
   g.smem = rows + (g.lists_smem ? lists : 0);
@@ -455,11 +456,12 @@ __global__ void __launch_bounds__(GB_THREADS) gg_build_kernel(const int32_t *__r
   }
 }
 
-template <int CT, bool LISTS_SMEM>
+template <class T, int CT, bool LISTS_SMEM>
 __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
-    const float *__restrict__ grad_out, const int *__restrict__ offsets, const uint16_t *__restrict__ order,
+    const T *__restrict__ grad_out, const int *__restrict__ offsets, const uint16_t *__restrict__ order,
     int C, int N, int S, int Sp, int H, int Np, float *__restrict__ grad_points) {
-  extern __shared__ __align__(128) float s_rows[];   // [CT][Sp] (+ uint16 [Sp] lists + int [Np] offsets)
+  extern __shared__ __align__(128) float s_smem[];
+  T *s_rows = reinterpret_cast<T *>(s_smem);        // [CT][Sp] (+ uint16 [Sp] lists + int [Np] offsets)
   __shared__ __align__(8) uint64_t bar;
   __shared__ int s_long[GG_LONG_CAP];
   __shared__ int s_nlong;
@@ -469,7 +471,7 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
   const int p0 = h * Sp;
   const int len = min(S, p0 + Sp) - p0;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const float *g = grad_out + ((size_t)b * C + c0) * S + p0;
+  const T *g = grad_out + ((size_t)b * C + c0) * S + p0;
   const int *off_g = offsets + ((size_t)b * H + h) * Np;
   const uint16_t *ord_g = order + (size_t)b * S + p0;
   uint16_t *s_ord = reinterpret_cast<uint16_t *>(s_rows + (size_t)CT * Sp);
@@ -482,14 +484,14 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
     if (tid == 0) { mbarrier_init(&bar, 1); fence_mbarrier_init(); }
     __syncthreads();
     if (tid == 0) {
-      unsigned bytes = (unsigned)(ct * len * sizeof(float));
+      unsigned bytes = (unsigned)(ct * len * sizeof(T));
       if (LISTS_SMEM) bytes += (unsigned)(len * sizeof(uint16_t) + Np * sizeof(int));
       mbarrier_arrive_expect_tx(&bar, bytes);
       if (LISTS_SMEM) {       // lists first: they are needed first and come from L2
         bulk_g2s(s_off, off_g, (unsigned)(Np * sizeof(int)), &bar);
         bulk_g2s(s_ord, ord_g, (unsigned)(len * sizeof(uint16_t)), &bar);
       }
-      for (int r = 0; r < ct; ++r) bulk_g2s(s_rows + (size_t)r * Sp, g + (size_t)r * S, (unsigned)(len * sizeof(float)), &bar);
+      for (int r = 0; r < ct; ++r) bulk_g2s(s_rows + (size_t)r * Sp, g + (size_t)r * S, (unsigned)(len * sizeof(T)), &bar);
     }
     mbarrier_wait(&bar, 0);
   } else {
@@ -519,15 +521,15 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
       const int q0 = ord[k], q1 = ord[k + 1], q2 = ord[k + 2], q3 = ord[k + 3];
 #pragma unroll
       for (int r = 0; r < CT; ++r) {
-        const float *row = s_rows + (size_t)r * Sp;
-        acc[r] = ((acc[r] + row[q0]) + row[q1]) + row[q2];
-        acc[r] += row[q3];
+        const T *row = s_rows + (size_t)r * Sp;
+        acc[r] = ((acc[r] + to_f32(row[q0])) + to_f32(row[q1])) + to_f32(row[q2]);
+        acc[r] += to_f32(row[q3]);
       }
     }
     for (; k < o1; ++k) {
       const int q0 = ord[k];
 #pragma unroll
-      for (int r = 0; r < CT; ++r) acc[r] += s_rows[(size_t)r * Sp + q0];
+      for (int r = 0; r < CT; ++r) acc[r] += to_f32(s_rows[(size_t)r * Sp + q0]);
     }
 #pragma unroll
     for (int r = 0; r < CT; ++r) {
@@ -549,7 +551,7 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
     for (int k = o0 + lane; k < o1; k += 32) {
       const int qq = ord[k];
 #pragma unroll
-      for (int r = 0; r < CT; ++r) acc[r] += s_rows[(size_t)r * Sp + qq];
+      for (int r = 0; r < CT; ++r) acc[r] += to_f32(s_rows[(size_t)r * Sp + qq]);
     }
 #pragma unroll
     for (int r = 0; r < CT; ++r)
@@ -567,10 +569,10 @@ __global__ void __launch_bounds__(GG_THREADS) group_points_grad_csr_kernel(
   }
 }
 
-template <int CT, bool LISTS_SMEM>
-static int launch_group_grad_csr(const float *grad_out, const int *offsets, const uint16_t *order, int B, int C,
+template <int CT, bool LISTS_SMEM, class T>
+static int launch_group_grad_csr(const T *grad_out, const int *offsets, const uint16_t *order, int B, int C,
                                  int N, int S, const GradPlan &g, float *grad_points, cudaStream_t stream) {
-  auto kern = group_points_grad_csr_kernel<CT, LISTS_SMEM>;
+  auto kern = group_points_grad_csr_kernel<T, CT, LISTS_SMEM>;
   if (g.smem > 40 * 1024)
     SPC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
   dim3 grid(g.H, ceil_div(C, CT), B);
@@ -625,8 +627,9 @@ __global__ void gl_fill_kernel(const int32_t *__restrict__ idx, int N, int S, in
   if (valid) order[(size_t)b * S + __ldg(offsets + (size_t)b * Np + i) + base + __popc(before)] = t;
 }
 
+template <class T>
 __global__ void __launch_bounds__(GL_THREADS) group_points_grad_gather_kernel(
-    const float *__restrict__ grad_out, const int *__restrict__ offsets, const int32_t *__restrict__ order, int C,
+    const T *__restrict__ grad_out, const int *__restrict__ offsets, const int32_t *__restrict__ order, int C,
     int N, int S, int Np, float *__restrict__ grad_points) {
   __shared__ int s_long[GL_LONG_CAP];
   __shared__ int s_nlong;
@@ -635,7 +638,7 @@ __global__ void __launch_bounds__(GL_THREADS) group_points_grad_gather_kernel(
   const int ct = min(GL_CT, C - c0);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int i = blockIdx.x * GL_THREADS + tid;
-  const float *g = grad_out + ((size_t)b * C + c0) * S;
+  const T *g = grad_out + ((size_t)b * C + c0) * S;
   const int *off = offsets + (size_t)b * Np;
   const int32_t *ord = order + (size_t)b * S;
   float *dst = grad_points + ((size_t)b * C + c0) * N;
@@ -658,8 +661,8 @@ __global__ void __launch_bounds__(GL_THREADS) group_points_grad_gather_kernel(
         float v0[GL_CT], v1[GL_CT];
 #pragma unroll
         for (int r = 0; r < GL_CT; ++r) {
-          v0[r] = r < ct ? __ldg(g + (size_t)r * S + q0) : 0.f;
-          v1[r] = r < ct ? __ldg(g + (size_t)r * S + q1) : 0.f;
+          v0[r] = r < ct ? to_f32(__ldg(g + (size_t)r * S + q0)) : 0.f;
+          v1[r] = r < ct ? to_f32(__ldg(g + (size_t)r * S + q1)) : 0.f;
         }
 #pragma unroll
         for (int r = 0; r < GL_CT; ++r) acc[r] = (acc[r] + v0[r]) + v1[r];
@@ -667,7 +670,7 @@ __global__ void __launch_bounds__(GL_THREADS) group_points_grad_gather_kernel(
       if (k < o1) {
         const int q0 = __ldg(ord + k);
 #pragma unroll
-        for (int r = 0; r < GL_CT; ++r) acc[r] += r < ct ? __ldg(g + (size_t)r * S + q0) : 0.f;
+        for (int r = 0; r < GL_CT; ++r) acc[r] += r < ct ? to_f32(__ldg(g + (size_t)r * S + q0)) : 0.f;
       }
 #pragma unroll
       for (int r = 0; r < GL_CT; ++r)
@@ -686,7 +689,7 @@ __global__ void __launch_bounds__(GL_THREADS) group_points_grad_gather_kernel(
     for (int k = o0 + lane; k < o1; k += 32) {
       const int qq = __ldg(ord + k);
 #pragma unroll
-      for (int r = 0; r < GL_CT; ++r) acc[r] += r < ct ? __ldg(g + (size_t)r * S + qq) : 0.f;
+      for (int r = 0; r < GL_CT; ++r) acc[r] += r < ct ? to_f32(__ldg(g + (size_t)r * S + qq)) : 0.f;
     }
 #pragma unroll
     for (int r = 0; r < GL_CT; ++r)
@@ -737,8 +740,9 @@ extern "C" int spc_gather_points_grad(const float *grad_out, const int32_t *idx,
   return SPC_OK;
 }
 
-extern "C" int spc_group_points(const float *points, const int32_t *idx, int B, int C, int N,
-                                int npoint, int nsample, float *out, void *stream_) {
+template <class T>
+static int group_points(const T *points, const int32_t *idx, int B, int C, int N, int npoint, int nsample, T *out,
+                        void *stream_) {
   SPC_CHECK_ARG(B >= 0 && C >= 0 && N >= 0 && npoint >= 0 && nsample >= 0, "group_points: bad sizes");
   const long long S64 = (long long)npoint * nsample;
   SPC_CHECK_ARG(S64 < (1LL << 31), "group_points: npoint*nsample overflows int32");
@@ -747,7 +751,7 @@ extern "C" int spc_group_points(const float *points, const int32_t *idx, int B, 
   SPC_CHECK_ARG(points && idx && out, "group_points: null pointer");
   SPC_CHECK_ARG(B <= 65535, "group_points: B too large");
   cudaStream_t stream = (cudaStream_t)stream_;
-  const GroupPlan g = plan_group(B, C, N, S, false);
+  const GroupPlan g = plan_group(B, C, N, S, false, sizeof(T));
   const bool vec4 = (S % 4 == 0) && ((reinterpret_cast<uintptr_t>(idx) & 15) == 0) &&
                     ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
   dim3 grid(g.nchunks, ceil_div(C, g.CT), B);
@@ -755,20 +759,21 @@ extern "C" int spc_group_points(const float *points, const int32_t *idx, int B, 
 #define GP_LAUNCH(ST, V4)                                                                       \
   do {                                                                                          \
     if (g.smem > 40 * 1024)                                                                     \
-      SPC_CUDA(cudaFuncSetAttribute(group_points_kernel<ST, V4>,                                \
+      SPC_CUDA(cudaFuncSetAttribute(group_points_kernel<T, ST, V4>,                             \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem)); \
-    group_points_kernel<ST, V4><<<grid, GP_THREADS, g.smem, stream>>>(points, idx, C, N, S,     \
-                                                                      g.CT, g.chunk, out);      \
+    group_points_kernel<T, ST, V4><<<grid, GP_THREADS, g.smem, stream>>>(points, idx, C, N, S,  \
+                                                                         g.CT, g.chunk, out);   \
   } while (0)
   if (g.staged) { if (vec4) GP_LAUNCH(true, true); else GP_LAUNCH(true, false); }
   else { if (vec4) GP_LAUNCH(false, true); else GP_LAUNCH(false, false); }
+#undef GP_LAUNCH
   SPC_LAUNCH_CHECK("group_points_kernel");
   return SPC_OK;
 }
 
-extern "C" int spc_group_points_grad(const float *grad_out, const int32_t *idx, int B, int C,
-                                     int N, int npoint, int nsample, float *grad_points,
-                                     void *stream_) {
+template <class T>
+static int group_points_grad(const T *grad_out, const int32_t *idx, int B, int C, int N, int npoint, int nsample,
+                             float *grad_points, void *stream_) {
   SPC_CHECK_ARG(B >= 0 && C >= 0 && N >= 0 && npoint >= 0 && nsample >= 0, "group_points_grad: bad sizes");
   const long long S64 = (long long)npoint * nsample;
   SPC_CHECK_ARG(S64 < (1LL << 31), "group_points_grad: npoint*nsample overflows int32");
@@ -781,7 +786,7 @@ extern "C" int spc_group_points_grad(const float *grad_out, const int32_t *idx, 
     SPC_CUDA(cudaMemsetAsync(grad_points, 0, (size_t)B * C * N * sizeof(float), stream));
     return SPC_OK;
   }
-  const GroupPlan g = plan_group(B, C, N, S, true);
+  const GroupPlan g = plan_group(B, C, N, S, true, sizeof(float));
   const int global_atomics = (!g.staged || g.nchunks > 1) ? 1 : 0;
   if (global_atomics)
     SPC_CUDA(cudaMemsetAsync(grad_points, 0, (size_t)B * C * N * sizeof(float), stream));
@@ -789,12 +794,12 @@ extern "C" int spc_group_points_grad(const float *grad_out, const int32_t *idx, 
   SPC_CHECK_ARG(grid.y <= 65535, "group_points_grad: too many channel tiles");
   if (g.staged) {
     if (g.smem > 40 * 1024)
-      SPC_CUDA(cudaFuncSetAttribute(group_points_grad_kernel<true>,
+      SPC_CUDA(cudaFuncSetAttribute(group_points_grad_kernel<T, true>,
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
-    group_points_grad_kernel<true><<<grid, GP_THREADS, g.smem, stream>>>(
+    group_points_grad_kernel<T, true><<<grid, GP_THREADS, g.smem, stream>>>(
         grad_out, idx, C, N, S, g.CT, g.chunk, global_atomics, grad_points);
   } else {
-    group_points_grad_kernel<false><<<grid, GP_THREADS, 0, stream>>>(
+    group_points_grad_kernel<T, false><<<grid, GP_THREADS, 0, stream>>>(
         grad_out, idx, C, N, S, g.CT, g.chunk, 1, grad_points);
   }
   SPC_LAUNCH_CHECK("group_points_grad_kernel");
@@ -806,14 +811,14 @@ extern "C" size_t spc_group_points_grad_workspace_bytes(int B, int N, int npoint
   const long long S = (long long)npoint * nsample;
   if (S >= (1LL << 31)) return 0;
   if (N > GB_MAX_N) return gl_workspace_bytes(B, N, S);
-  const GradPlan g = plan_group_grad(1, N, (int)S);
+  const GradPlan g = plan_group_grad(1, N, (int)S, sizeof(float));   // H and Np do not depend on the element size
   // offsets (B,H,Np) int32  +  order (B,S) uint16, both starting 16-byte aligned
   return (size_t)B * g.H * (size_t)g.Np * sizeof(int) + (((size_t)B * (size_t)S * sizeof(uint16_t) + 15) & ~(size_t)15);
 }
 
-extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *idx, int B, int C, int N, int npoint,
-                                        int nsample, float *grad_points, void *workspace, size_t workspace_bytes,
-                                        void *stream_) {
+template <class T>
+static int group_points_grad_ex(const T *grad_out, const int32_t *idx, int B, int C, int N, int npoint, int nsample,
+                                float *grad_points, void *workspace, size_t workspace_bytes, void *stream_) {
   SPC_CHECK_ARG(B >= 0 && C >= 0 && N >= 0 && npoint >= 0 && nsample >= 0, "group_points_grad: bad sizes");
   const long long S64 = (long long)npoint * nsample;
   SPC_CHECK_ARG(S64 < (1LL << 31), "group_points_grad: npoint*nsample overflows int32");
@@ -823,7 +828,7 @@ extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *id
   // every input level with features); with fewer the atomic kernel is faster.
   if (!workspace || need == 0 || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 15) || C < 4 ||
       (N <= GB_MAX_N && (long long)N > 512LL * C) || B == 0 || B > 65535)
-    return spc_group_points_grad(grad_out, idx, B, C, N, npoint, nsample, grad_points, stream_);
+    return group_points_grad(grad_out, idx, B, C, N, npoint, nsample, grad_points, stream_);
   SPC_CHECK_ARG(grad_points && grad_out && idx, "group_points_grad: null pointer");
   cudaStream_t stream = (cudaStream_t)stream_;
   if (N > GB_MAX_N) {
@@ -843,7 +848,7 @@ extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *id
     SPC_LAUNCH_CHECK("group_points_grad_gather_kernel");
     return SPC_OK;
   }
-  const GradPlan g = plan_group_grad(C, N, S);
+  const GradPlan g = plan_group_grad(C, N, S, sizeof(T));
   SPC_CHECK_ARG(ceil_div(C, g.CT) <= 65535 && g.H <= 65535, "group_points_grad: grid too large");
   int *offsets = reinterpret_cast<int *>(workspace);
   const size_t off_bytes = (size_t)B * g.H * (size_t)g.Np * sizeof(int);
@@ -865,4 +870,38 @@ extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *id
                           : launch_group_grad_csr<4, false>(grad_out, offsets, order, B, C, N, S, g, grad_points, stream);
   }
 #undef GG_CASE
+}
+
+// ---- C entry points: fp32 storage, and bf16 storage (points / out / grad_out are __nv_bfloat16 tensors) ------------
+extern "C" int spc_group_points(const float *points, const int32_t *idx, int B, int C, int N,
+                                int npoint, int nsample, float *out, void *stream) {
+  return group_points(points, idx, B, C, N, npoint, nsample, out, stream);
+}
+extern "C" int spc_group_points_bf16(const void *points, const int32_t *idx, int B, int C, int N,
+                                     int npoint, int nsample, void *out, void *stream) {
+  return group_points(static_cast<const bf16 *>(points), idx, B, C, N, npoint, nsample, static_cast<bf16 *>(out),
+                      stream);
+}
+
+extern "C" int spc_group_points_grad(const float *grad_out, const int32_t *idx, int B, int C,
+                                     int N, int npoint, int nsample, float *grad_points,
+                                     void *stream) {
+  return group_points_grad(grad_out, idx, B, C, N, npoint, nsample, grad_points, stream);
+}
+extern "C" int spc_group_points_grad_bf16(const void *grad_out, const int32_t *idx, int B, int C,
+                                          int N, int npoint, int nsample, float *grad_points,
+                                          void *stream) {
+  return group_points_grad(static_cast<const bf16 *>(grad_out), idx, B, C, N, npoint, nsample, grad_points, stream);
+}
+
+extern "C" int spc_group_points_grad_ex(const float *grad_out, const int32_t *idx, int B, int C, int N, int npoint,
+                                        int nsample, float *grad_points, void *workspace, size_t workspace_bytes,
+                                        void *stream) {
+  return group_points_grad_ex(grad_out, idx, B, C, N, npoint, nsample, grad_points, workspace, workspace_bytes, stream);
+}
+extern "C" int spc_group_points_grad_ex_bf16(const void *grad_out, const int32_t *idx, int B, int C, int N, int npoint,
+                                             int nsample, float *grad_points, void *workspace, size_t workspace_bytes,
+                                             void *stream) {
+  return group_points_grad_ex(static_cast<const bf16 *>(grad_out), idx, B, C, N, npoint, nsample, grad_points,
+                              workspace, workspace_bytes, stream);
 }

@@ -6,6 +6,9 @@
 // wide grid with on-chip reuse: `known` is staged once per CTA in shared memory for three_nn;
 // three_interpolate keeps (idx, weight) of a point in registers and sweeps channels with
 // coalesced stores, the small feature rows being served by L1.
+// three_interpolate and its backward are instantiated for float and bf16 storage of the features (common.cuh): the
+// forward reads bf16 rows and writes bf16, the backward reads a bf16 grad_out and writes an fp32 gradient.  idx and
+// weight stay fp32 / int32, and the arithmetic is fp32 either way.
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -77,8 +80,9 @@ __global__ void __launch_bounds__(NN_THREADS) three_nn_kernel(const float *__res
 constexpr int TI_THREADS = 256;
 
 // one bulk-TMA copy global -> shared (bytes % 16 == 0, 16-byte aligned) or a plain copy; all threads call it
-__device__ __forceinline__ void ti_stage(float *dst, const float *src, size_t count, uint64_t *bar, int tid, int nthr) {
-  const size_t bytes = count * sizeof(float);
+template <class T>
+__device__ __forceinline__ void ti_stage(T *dst, const T *src, size_t count, uint64_t *bar, int tid, int nthr) {
+  const size_t bytes = count * sizeof(T);
   if (((reinterpret_cast<uintptr_t>(src) & 15) == 0) && bytes % 16 == 0 && bytes < (1u << 20)) {
     if (tid == 0) {
       mbarrier_init(bar, 1);
@@ -97,16 +101,17 @@ __device__ __forceinline__ void ti_stage(float *dst, const float *src, size_t co
 }
 
 // points (B,C,m), idx/weight (B,n,3) -> out (B,C,n).   grid = (ceil(n/1024), ceil(C/CT), B)
-template <bool STAGED>
+template <class T, bool STAGED>
 __global__ void __launch_bounds__(TI_THREADS) three_interpolate_kernel(
-    const float *__restrict__ points, const int32_t *__restrict__ idx,
-    const float *__restrict__ weight, int C, int m, int n, int CT, float *__restrict__ out) {
-  extern __shared__ __align__(128) float s_rows[];   // [CT][m]
+    const T *__restrict__ points, const int32_t *__restrict__ idx,
+    const float *__restrict__ weight, int C, int m, int n, int CT, T *__restrict__ out) {
+  extern __shared__ __align__(128) float s_smem[];
+  T *s_rows = reinterpret_cast<T *>(s_smem);        // [CT][m]
   __shared__ __align__(8) uint64_t bar;
   const int b = blockIdx.z;
   const int c0 = blockIdx.y * CT;
   const int ct = min(CT, C - c0);
-  const float *src = points + ((size_t)b * C + c0) * m;
+  const T *src = points + ((size_t)b * C + c0) * m;
   if (STAGED) ti_stage(s_rows, src, (size_t)ct * m, &bar, threadIdx.x, TI_THREADS);
   const int j0 = (blockIdx.x * TI_THREADS + threadIdx.x) * 4;
   if (j0 >= n) return;
@@ -132,28 +137,29 @@ __global__ void __launch_bounds__(TI_THREADS) three_interpolate_kernel(
   }
   const bool vec = j0 + 4 <= n && n % 4 == 0;
   for (int c = 0; c < ct; ++c) {
-    const float *row = STAGED ? s_rows + (size_t)c * m : src + (size_t)c * m;
+    const T *row = STAGED ? s_rows + (size_t)c * m : src + (size_t)c * m;
     float v[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      const float p1 = STAGED ? row[a[3 * q]] : __ldg(row + a[3 * q]);
-      const float p2 = STAGED ? row[a[3 * q + 1]] : __ldg(row + a[3 * q + 1]);
-      const float p3 = STAGED ? row[a[3 * q + 2]] : __ldg(row + a[3 * q + 2]);
+      const float p1 = to_f32(STAGED ? row[a[3 * q]] : __ldg(row + a[3 * q]));
+      const float p2 = to_f32(STAGED ? row[a[3 * q + 1]] : __ldg(row + a[3 * q + 1]));
+      const float p3 = to_f32(STAGED ? row[a[3 * q + 2]] : __ldg(row + a[3 * q + 2]));
       v[q] = __fmaf_rn(p3, ww[3 * q + 2], __fmaf_rn(p1, ww[3 * q], __fmul_rn(p2, ww[3 * q + 1])));
     }
-    float *o = out + ((size_t)b * C + c0 + c) * n + j0;
-    if (vec) asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]) : "memory");
+    T *o = out + ((size_t)b * C + c0 + c) * n + j0;
+    if (vec) st_cs4(o, from_f32<T>(v[0]), from_f32<T>(v[1]), from_f32<T>(v[2]), from_f32<T>(v[3]));
     else
 #pragma unroll
-      for (int q = 0; q < 4; ++q) if (j0 + q < n) o[q] = v[q];
+      for (int q = 0; q < 4; ++q) if (j0 + q < n) o[q] = from_f32<T>(v[q]);
   }
 }
 
 // grad_out (B,C,n) -> grad_points (B,C,m): a CTA owns TI_CT whole output rows (all n positions), accumulates them
 // in shared memory and stores them once.
 constexpr int TI_CT = 8;
+template <class T>
 __global__ void __launch_bounds__(TI_THREADS) three_interpolate_grad_kernel(
-    const float *__restrict__ grad_out, const int32_t *__restrict__ idx,
+    const T *__restrict__ grad_out, const int32_t *__restrict__ idx,
     const float *__restrict__ weight, int C, int n, int m, float *__restrict__ grad_points) {
   extern __shared__ float s_acc[];  // [TI_CT][m]
   const int b = blockIdx.y;
@@ -167,7 +173,7 @@ __global__ void __launch_bounds__(TI_THREADS) three_interpolate_grad_kernel(
     const int a1 = __ldg(ix), a2 = __ldg(ix + 1), a3 = __ldg(ix + 2);
     const float w1 = __ldg(w), w2 = __ldg(w + 1), w3 = __ldg(w + 2);
     for (int c = 0; c < ct; ++c) {
-      const float g = __ldg(grad_out + ((size_t)b * C + c0 + c) * n + j);
+      const float g = to_f32(__ldg(grad_out + ((size_t)b * C + c0 + c) * n + j));
       float *row = s_acc + (size_t)c * m;
       atomicAdd(row + a1, g * w1);
       atomicAdd(row + a2, g * w2);
@@ -180,7 +186,8 @@ __global__ void __launch_bounds__(TI_THREADS) three_interpolate_grad_kernel(
 }
 
 // fallback for rows that do not fit in shared memory: global atomics into a zeroed buffer
-__global__ void three_interpolate_grad_global_kernel(const float *__restrict__ grad_out,
+template <class T>
+__global__ void three_interpolate_grad_global_kernel(const T *__restrict__ grad_out,
                                                      const int32_t *__restrict__ idx,
                                                      const float *__restrict__ weight, int C,
                                                      int n, int m,
@@ -193,7 +200,7 @@ __global__ void three_interpolate_grad_global_kernel(const float *__restrict__ g
   const int a1 = __ldg(ix), a2 = __ldg(ix + 1), a3 = __ldg(ix + 2);
   const float w1 = __ldg(w), w2 = __ldg(w + 1), w3 = __ldg(w + 2);
   for (int c = blockIdx.y; c < C; c += gridDim.y) {
-    const float g = __ldg(grad_out + ((size_t)b * C + c) * n + j);
+    const float g = to_f32(__ldg(grad_out + ((size_t)b * C + c) * n + j));
     float *row = grad_points + ((size_t)b * C + c) * m;
     atomicAdd(row + a1, g * w1);
     atomicAdd(row + a2, g * w2);
@@ -217,15 +224,17 @@ extern "C" int spc_three_nn(const float *unknown, const float *known, int B, int
   return SPC_OK;
 }
 
-extern "C" int spc_three_interpolate(const float *points, const int32_t *idx, const float *weight,
-                                     int B, int C, int m, int n, float *out, void *stream_) {
+template <class T>
+static int three_interpolate(const T *points, const int32_t *idx, const float *weight, int B, int C, int m, int n,
+                             T *out, void *stream_) {
   SPC_CHECK_ARG(B >= 0 && C >= 0 && m >= 0 && n >= 0, "three_interpolate: bad sizes");
   if (B == 0 || C == 0 || n == 0) return SPC_OK;
   SPC_CHECK_ARG(points && idx && weight && out, "three_interpolate: null pointer");
   SPC_CHECK_ARG(B <= 65535, "three_interpolate: B too large");
   cudaStream_t stream = (cudaStream_t)stream_;
-  // rows staged per CTA: as many as fit in ~64 KB (re-reading idx / weight once per channel tile costs
-  // 24 B per point and tile against 4*CT B of output), but enough CTAs to fill the machine
+  // rows staged per CTA: as many fp32 rows as fit in ~64 KB (re-reading idx / weight once per channel tile costs
+  // 24 B per point and tile against 4*CT B of output), but enough CTAs to fill the machine; bf16 rows take the same
+  // tiling in half the shared memory
   int CT = m > 0 ? (int)((64 * 1024) / ((size_t)m * sizeof(float))) : 0;
   if (CT > 32) CT = 32;
   if (CT > C) CT = C;
@@ -233,23 +242,24 @@ extern "C" int spc_three_interpolate(const float *points, const int32_t *idx, co
   while (CT > 4 && (long long)xchunks * ceil_div(C, CT) * B < 2 * kNumSMs) CT /= 2;
   if (CT >= 1) {
     SPC_CHECK_ARG(ceil_div(C, CT) <= 65535, "three_interpolate: C too large");
-    const size_t smem = (size_t)CT * m * sizeof(float);
-    SPC_CUDA(cudaFuncSetAttribute(three_interpolate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = (size_t)CT * m * sizeof(T);
+    SPC_CUDA(cudaFuncSetAttribute(three_interpolate_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid(xchunks, ceil_div(C, CT), B);
-    three_interpolate_kernel<true><<<grid, TI_THREADS, smem, stream>>>(points, idx, weight, C, m, n, CT, out);
+    three_interpolate_kernel<T, true><<<grid, TI_THREADS, smem, stream>>>(points, idx, weight, C, m, n, CT, out);
   } else {                                         // a single row exceeds the budget: read-only-cache gathers
     CT = 8;
     SPC_CHECK_ARG(ceil_div(C, CT) <= 65535, "three_interpolate: C too large");
     dim3 grid(xchunks, ceil_div(C, CT), B);
-    three_interpolate_kernel<false><<<grid, TI_THREADS, 0, stream>>>(points, idx, weight, C, m, n, CT, out);
+    three_interpolate_kernel<T, false><<<grid, TI_THREADS, 0, stream>>>(points, idx, weight, C, m, n, CT, out);
   }
   SPC_LAUNCH_CHECK("three_interpolate_kernel");
   return SPC_OK;
 }
 
-extern "C" int spc_three_interpolate_grad(const float *grad_out, const int32_t *idx,
-                                          const float *weight, int B, int C, int n, int m,
-                                          float *grad_points, void *stream_) {
+// the accumulators are fp32 rows for either storage type of grad_out
+template <class T>
+static int three_interpolate_grad(const T *grad_out, const int32_t *idx, const float *weight, int B, int C, int n,
+                                  int m, float *grad_points, void *stream_) {
   SPC_CHECK_ARG(B >= 0 && C >= 0 && m >= 0 && n >= 0, "three_interpolate_grad: bad sizes");
   if (B == 0 || C == 0 || m == 0) return SPC_OK;
   SPC_CHECK_ARG(grad_points && (n == 0 || (grad_out && idx && weight)), "three_interpolate_grad: null pointer");
@@ -258,7 +268,7 @@ extern "C" int spc_three_interpolate_grad(const float *grad_out, const int32_t *
   const size_t smem = (size_t)TI_CT * m * sizeof(float);
   if (smem <= 96 * 1024) {
     if (smem > 40 * 1024)
-      SPC_CUDA(cudaFuncSetAttribute(three_interpolate_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      SPC_CUDA(cudaFuncSetAttribute(three_interpolate_grad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     three_interpolate_grad_kernel<<<dim3(ceil_div(C, TI_CT), B), TI_THREADS, smem, stream>>>(grad_out, idx, weight, C, n, m,
                                                                                          grad_points);
     SPC_LAUNCH_CHECK("three_interpolate_grad_kernel");
@@ -270,4 +280,26 @@ extern "C" int spc_three_interpolate_grad(const float *grad_out, const int32_t *
   three_interpolate_grad_global_kernel<<<grid, 256, 0, stream>>>(grad_out, idx, weight, C, n, m, grad_points);
   SPC_LAUNCH_CHECK("three_interpolate_grad_global_kernel");
   return SPC_OK;
+}
+
+// ---- C entry points: fp32 storage, and bf16 storage (points / out / grad_out are __nv_bfloat16 tensors) ------------
+extern "C" int spc_three_interpolate(const float *points, const int32_t *idx, const float *weight,
+                                     int B, int C, int m, int n, float *out, void *stream) {
+  return three_interpolate(points, idx, weight, B, C, m, n, out, stream);
+}
+extern "C" int spc_three_interpolate_bf16(const void *points, const int32_t *idx, const float *weight,
+                                          int B, int C, int m, int n, void *out, void *stream) {
+  return three_interpolate(static_cast<const bf16 *>(points), idx, weight, B, C, m, n, static_cast<bf16 *>(out),
+                           stream);
+}
+
+extern "C" int spc_three_interpolate_grad(const float *grad_out, const int32_t *idx,
+                                          const float *weight, int B, int C, int n, int m,
+                                          float *grad_points, void *stream) {
+  return three_interpolate_grad(grad_out, idx, weight, B, C, n, m, grad_points, stream);
+}
+extern "C" int spc_three_interpolate_grad_bf16(const void *grad_out, const int32_t *idx,
+                                               const float *weight, int B, int C, int n, int m,
+                                               float *grad_points, void *stream) {
+  return three_interpolate_grad(static_cast<const bf16 *>(grad_out), idx, weight, B, C, n, m, grad_points, stream);
 }

@@ -51,7 +51,14 @@ def _sample_centres(xyz, npoint, inds=None):
 
 
 INLINE_MAX_FEATURES = 13   # raw feature channels the fused kernel evaluates in-line (layer 0)
-PAD_TRAINING_CHANNELS = True   # training: pad 3+C grouped channels to a multiple of 4 (aligned conv GEMMs)
+PAD_TRAINING_CHANNELS = True   # training: pad 3+C grouped channels to a multiple of 4 (aligned conv GEMMs; 8 in bf16)
+
+
+def _autocast_bf16():
+    """torch.bfloat16 when the convolutions that follow will run in bf16 under CUDA autocast, else None."""
+    if torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16:
+        return torch.bfloat16
+    return None
 
 
 def attach_pm(t, pm, pm_lo=None):
@@ -314,13 +321,18 @@ class PointnetSAModuleVotes(nn.Module):
         if features is not None and not features.is_contiguous():
             features = features.contiguous()      # (a caller may hand in a channel-major VIEW of a point-major cloud)
         # training on the GPU: zero-pad the grouped tensor to a multiple of 4 channels (aligned GEMM rows, see
-        # QueryAndGroup.forward); the first SharedMLP block pads its weight to match -- same values either way
-        pad = 4 if (self.training and xyz.is_cuda and features is not None and len(self.mlp_module) > 0
-                    and isinstance(self.grouper, pointnet2_utils.QueryAndGroup) and PAD_TRAINING_CHANNELS) else 1
-        if pad > 1:
-            grouped_features, grouped_xyz = self.grouper(xyz, new_xyz, features, pad_channels_to=pad)
-        else:
-            grouped_features, grouped_xyz = self.grouper(xyz, new_xyz, features)
+        # QueryAndGroup.forward); the first SharedMLP block pads its weight to match -- same values either way.
+        # Under bf16 autocast the grouped tensor is built in bf16 (the conv's input dtype) and padded to a multiple
+        # of 8 channels, 16-byte rows of bf16.
+        train_gpu = (self.training and xyz.is_cuda and features is not None and len(self.mlp_module) > 0
+                     and isinstance(self.grouper, pointnet2_utils.QueryAndGroup))
+        group_kw = {}
+        amp = _autocast_bf16() if train_gpu else None
+        if amp is not None:
+            group_kw["dtype"] = amp
+        if train_gpu and PAD_TRAINING_CHANNELS:
+            group_kw["pad_channels_to"] = 8 if amp is not None else 4
+        grouped_features, grouped_xyz = self.grouper(xyz, new_xyz, features, **group_kw)
         if (self.pooling == 'max' and self.training and grouped_features.is_cuda and len(self.mlp_module) > 0
                 and pt_utils.FUSED_BN_RELU_TRAINING):
             # training: the last block's BatchNorm + ReLU + max-pool run as one kernel pair (csrc/bn_relu.cu)

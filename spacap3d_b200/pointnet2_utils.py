@@ -146,12 +146,15 @@ class QueryAndGroup(nn.Module):
         if self.ret_unique_cnt:
             assert self.sample_uniformly
 
-    def forward(self, xyz, new_xyz, features=None, pad_channels_to=1):
+    def forward(self, xyz, new_xyz, features=None, pad_channels_to=1, dtype=None):
         """xyz (B,N,3), new_xyz (B,npoint,3), features (B,C,N) -> (B,3+C,npoint,nsample).
         pad_channels_to = 4 (an extension the SA module uses in training) appends all-zero channels so that the
         channel count is a multiple of 4: 3 + 128 or 3 + 256 input channels make every row of the 1x1-conv GEMMs
         that follow 4 bytes short of 16-byte alignment, which sends cuDNN / cuBLAS to their slow `align1` kernels
-        (14 % of a training step); the consumer pads its weight with matching zero columns."""
+        (14 % of a training step); the consumer pads its weight with matching zero columns.
+        dtype = torch.bfloat16 (the SA module under bf16 autocast) groups the features cast to bf16 and casts the
+        relative xyz before the concatenation: bit for bit the conv input autocast would produce, without an fp32
+        copy of the grouped tensor (torch.cat promotes mixed inputs to fp32).  The returned grouped_xyz stays fp32."""
         if self.sample_uniformly:
             # the reference prints and exit(1)s here (:337-339); raise instead of killing the process
             raise NotImplementedError("sample_uniformly is a dead path in the reference")
@@ -161,12 +164,13 @@ class QueryAndGroup(nn.Module):
         if self.normalize_xyz:
             grouped_xyz /= self.radius
         if features is not None:
-            grouped_features = grouping_operation(features, idx)
+            grouped_features = grouping_operation(features if dtype is None else features.to(dtype), idx)
             if self.use_xyz:
-                parts = [grouped_xyz, grouped_features]
+                xyz_part = grouped_xyz if dtype is None else grouped_xyz.to(dtype)
+                parts = [xyz_part, grouped_features]
                 extra = -(3 + grouped_features.shape[1]) % max(int(pad_channels_to), 1)
                 if extra:
-                    parts.append(grouped_xyz.new_zeros((grouped_xyz.shape[0], extra) + tuple(grouped_xyz.shape[2:])))
+                    parts.append(xyz_part.new_zeros((xyz_part.shape[0], extra) + tuple(xyz_part.shape[2:])))
                 new_features = torch.cat(parts, dim=1)
             else:
                 new_features = grouped_features

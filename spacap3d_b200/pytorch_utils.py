@@ -15,7 +15,12 @@ import torch.nn.functional as F
 # instead of cuDNN batch-norm + a separate ReLU pass.  Same parameters, buffers and results (fp32, within
 # summation-order rounding); set to False to get the plain module sequence.  A BatchNorm converted to
 # nn.SyncBatchNorm runs the synced variants of the same kernels when torch's SyncBatchNorm would synchronise.
+# Under torch.autocast(dtype=torch.bfloat16) the convolution returns bf16 and the kernels' bf16 twins run: bf16
+# activations, fp32 arithmetic and fp32 BatchNorm parameters and statistics, as torch's own bf16 sequence.
 FUSED_BN_RELU_TRAINING = True
+
+# storage dtypes of a conv output the fused kernels take; anything else (fp16 autocast, fp64) runs torch's modules
+_FUSED_DTYPES = (torch.float32, torch.bfloat16)
 
 
 class _BnReluTrain(torch.autograd.Function):
@@ -172,11 +177,13 @@ class _ConvBase(nn.Sequential):
         self._conv_name, self._bn_name = name + "conv", name + "bn"   # names, not modules: no second registration
 
     def _fused_training_ok(self, x):
-        if not (self._fusable and FUSED_BN_RELU_TRAINING and self.training and x.is_cuda
-                and x.dtype == torch.float32 and torch.is_grad_enabled()):
+        """Everything but the conv output's dtype, which forward() checks once the conv has run (autocast decides
+        it).  The BatchNorm's parameters must be fp32: a model cast wholesale with .bfloat16() keeps torch's."""
+        if not (self._fusable and FUSED_BN_RELU_TRAINING and self.training and x.is_cuda and torch.is_grad_enabled()):
             return False
         bn = getattr(self, self._bn_name)[0]
-        return bn.training and bn.affine and bn.track_running_stats and bn.momentum is not None
+        return (bn.training and bn.affine and bn.track_running_stats and bn.momentum is not None
+                and bn.weight.dtype == torch.float32 and bn.running_mean.dtype == torch.float32)
 
     def forward(self, x, max_pool_last_dim=False):
         """max_pool_last_dim=True additionally takes the max over the last axis (the SA module's
@@ -195,6 +202,12 @@ class _ConvBase(nn.Sequential):
             # the kernels take any batch, so whether they run depends only on the module, C and nsample, never on this
             # rank's share of the batch: with SyncBatchNorm all ranks issue the same collectives
             y = run_conv(x).contiguous()
+            if y.dtype not in _FUSED_DTYPES:
+                out = y
+                for name, mod in self.named_children():      # conv -> bn -> activation; the conv has run
+                    if name != self._conv_name:
+                        out = mod(out)
+                return _max_pool_last(out) if max_pool_last_dim else out
             args = (y, bn.weight, bn.bias, bn.running_mean, bn.running_var, float(bn.momentum), float(bn.eps),
                     _sync_group(bn))
             if max_pool_last_dim and y.dim() == 4 and y.shape[3] in (16, 32, 64):

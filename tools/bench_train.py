@@ -17,7 +17,14 @@ extension (oracle/_ref) driving the same modules on rank 0.  One JSON line per c
 in the backward of each block, torch's SyncBatchNorm for the voting and proposal heads) or `torch` (the converted
 model with the fused kernels switched off: torch's SyncBatchNorm everywhere).  Each line records the GPU's name and
 power limit.
+
+`--amp` runs the step without autocast (`off`) or under torch.autocast("cuda", dtype=torch.bfloat16) (`bf16`: bf16
+activations through the bf16 twins of the grouping, interpolation and fused BatchNorm kernels); `--amp off,bf16`
+times both for every cloud size, alternating them `--repeats` times, eager and graphed (captured with
+cache_enabled=False, so no cast of a weight is cached across replays).  Each line also records the peak memory of the
+eager steps (torch.cuda.max_memory_allocated).
 """
+import contextlib
 import argparse
 import json
 import os
@@ -71,6 +78,13 @@ def step(model, pc, world):
     return loss
 
 
+def amp_context(amp):
+    """The autocast region of one step: nothing for `off`, bf16 autocast for `bf16`."""
+    if amp == "bf16":
+        return torch.autocast("cuda", dtype=torch.bfloat16, cache_enabled=False)
+    return contextlib.nullcontext()
+
+
 def time_steps(fn, iters, warmup=2):
     for _ in range(warmup):
         fn()
@@ -84,6 +98,64 @@ def time_steps(fn, iters, warmup=2):
     return float(np.median([a.elapsed_time(b) for a, b in ev]))
 
 
+def measure(args, amp, n, scale, pc, dev, rank, world, ref, info, pytorch_utils, max_over_ranks):
+    """One JSON record: eager (and graphed, on one GPU) ms per step of a fresh model in autocast mode `amp`."""
+    model = build_model(scale, dev, args.sync_bn)
+
+    def ours():
+        model.zero_grad(set_to_none=True)
+        with amp_context(amp):
+            step(model, pc, world)
+
+    torch.cuda.synchronize()
+    torch.cuda.empty_cache()
+    torch.cuda.reset_peak_memory_stats(dev)
+    ms = time_steps(ours, args.iters)
+    peak = torch.cuda.max_memory_allocated(dev)
+    ms = max_over_ranks(ms, device=dev) if world > 1 else ms
+    rec = {"config": "fwd+bwd, %d scenes/GPU x %d pts, SA npoint x%d" % (args.scenes, n, scale), "n_gpus": world,
+           "ms_per_step": round(ms, 3), "scenes_per_s": round(world * args.scenes / ms * 1e3, 2),
+           "sync_bn": args.sync_bn, "amp": amp,
+           "peak_mem_gb": round(peak / 1e9, 3), **info}
+    if world == 1 and not args.no_graph:
+        # the step has no host synchronisation (box decode stays on the device), so forward + backward can be
+        # captured once and replayed: removes the ~3 ms/step of Python/launch overhead of ~600 small launches
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            ours()
+        torch.cuda.current_stream().wait_stream(side)
+        model.zero_grad(set_to_none=True)
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph), amp_context(amp):
+            step(model, pc, 1)
+        gms = time_steps(graph.replay, args.iters)
+        rec["graphed_ms_per_step"] = round(gms, 3)
+        rec["graphed_scenes_per_s"] = round(args.scenes / gms * 1e3, 2)
+        del graph
+    if ref is not None:
+        import bench
+
+        def theirs():      # reference extension + the plain cuDNN BatchNorm / ReLU / max_pool2d sequence
+            model.zero_grad(set_to_none=True)
+            pytorch_utils.FUSED_BN_RELU_TRAINING = False
+            try:
+                with bench.swapped_ops(ref, host_decode=False), amp_context(amp):
+                    step(model, pc, 1)
+            finally:
+                pytorch_utils.FUSED_BN_RELU_TRAINING = args.sync_bn != "torch"
+
+        try:
+            rms = time_steps(theirs, max(2, args.iters // 2), warmup=1)
+            rec["reference_ext_ms_per_step"] = round(rms, 3)
+            rec["speedup_vs_reference_ext"] = round(rms / ms, 2)
+        except Exception as e:   # the reference FPS kernel has a fixed 512-thread block; very large N still works, but be safe
+            rec["reference_ext_error"] = str(e)[:200]
+    del model
+    torch.cuda.empty_cache()
+    return rec
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--points", default="40000,80000,120000,200000")
@@ -93,7 +165,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--sync-bn", choices=("off", "fused", "torch"), default="off",
                     help="BatchNorm statistics per rank (off) or across ranks with the fused kernels or torch's")
+    ap.add_argument("--amp", default="off",
+                    help="comma-separated autocast modes to time, alternated: off, bf16 (e.g. off,bf16)")
+    ap.add_argument("--repeats", type=int, default=1, help="rounds of the --amp modes per cloud size")
     args = ap.parse_args()
+    amps = args.amp.split(",")
+    assert all(a in ("off", "bf16") for a in amps), args.amp
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     torch.cuda.set_device(local)
@@ -112,56 +189,13 @@ def main():
         ref = load_ref()
     for n in [int(x) for x in args.points.split(",")]:
         scale = max(1, round(n / 40000))
-        model = build_model(scale, dev, args.sync_bn)
         pc = torch.from_numpy(np.stack([make_scene(5000 + rank * 100 + i, n) for i in range(args.scenes)], 0)).to(dev)
-
-        def ours():
-            model.zero_grad(set_to_none=True)
-            step(model, pc, world)
-
-        ms = time_steps(ours, args.iters)
-        ms = max_over_ranks(ms, device=dev) if world > 1 else ms
-        rec = {"config": "fwd+bwd, %d scenes/GPU x %d pts, SA npoint x%d" % (args.scenes, n, scale), "n_gpus": world,
-               "ms_per_step": round(ms, 3), "scenes_per_s": round(world * args.scenes / ms * 1e3, 2),
-               "sync_bn": args.sync_bn, **info}
-        if world == 1 and not args.no_graph:
-            # the step has no host synchronisation (box decode stays on the device), so forward + backward can be
-            # captured once and replayed: removes the ~3 ms/step of Python/launch overhead of ~600 small launches
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                ours()
-            torch.cuda.current_stream().wait_stream(side)
-            model.zero_grad(set_to_none=True)
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                step(model, pc, 1)
-            gms = time_steps(graph.replay, args.iters)
-            rec["graphed_ms_per_step"] = round(gms, 3)
-            rec["graphed_scenes_per_s"] = round(args.scenes / gms * 1e3, 2)
-            del graph
-        if ref is not None:
-            import bench
-
-            def theirs():      # reference extension + the plain cuDNN BatchNorm / ReLU / max_pool2d sequence
-                model.zero_grad(set_to_none=True)
-                pytorch_utils.FUSED_BN_RELU_TRAINING = False
-                try:
-                    with bench.swapped_ops(ref, host_decode=False):
-                        step(model, pc, 1)
-                finally:
-                    pytorch_utils.FUSED_BN_RELU_TRAINING = args.sync_bn != "torch"
-
-            try:
-                rms = time_steps(theirs, max(2, args.iters // 2), warmup=1)
-                rec["reference_ext_ms_per_step"] = round(rms, 3)
-                rec["speedup_vs_reference_ext"] = round(rms / ms, 2)
-            except Exception as e:   # the reference FPS kernel has a fixed 512-thread block; very large N still works, but be safe
-                rec["reference_ext_error"] = str(e)[:200]
-        if rank == 0:
-            print(json.dumps(rec), flush=True)
-        del model, pc
-        torch.cuda.empty_cache()
+        for _ in range(args.repeats):
+            for amp in amps:
+                rec = measure(args, amp, n, scale, pc, dev, rank, world, ref, info, pytorch_utils, max_over_ranks)
+                if rank == 0:
+                    print(json.dumps(rec), flush=True)
+        del pc
     if world > 1:
         torch.distributed.destroy_process_group()
 
